@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- frames/s of the heatmap -> 3D keypoint path on N B200s (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A step is one pass of the hot path (K1 peaks, K3/K4 grouping + 3D lift; for N > 1 the grouping kernel also
@@ -127,6 +127,24 @@ def parity_mismatches(got, want):
     return n, int(bad.sum())
 
 
+DUMP_BYTES = 60_000_000
+
+
+def dump_outputs(directory, tables, budget=DUMP_BYTES):
+    """Writes decode tables (NumPy, as DecodeTables.numpy() returns them) as DIR/<table>.npy, float32 tables as they are and
+    the integer tables and flags as float64 (exact), so that two builds can be compared output for output. When all frames
+    would take more than `budget` bytes, a fixed seeded sample of frames is written; frame_index.npy lists the frames."""
+    import numpy as np
+    n = tables['n_objects'].shape[0]
+    per_frame = sum(int(np.prod(v.shape[1:])) * (4 if v.dtype == np.float32 else 8) for v in tables.values())
+    keep = min(n, budget // max(per_frame, 1))
+    frames = np.arange(n) if keep == n else np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+    os.makedirs(directory, exist_ok=True)
+    np.save(os.path.join(directory, 'frame_index.npy'), frames.astype(np.float64))
+    for name, value in tables.items():
+        np.save(os.path.join(directory, f'{name}.npy'), value[frames].astype(np.float32 if value.dtype == np.float32 else np.float64))
+
+
 def make_inputs(workload, device, seed):
     import torch
     from object_keypoints_b200 import synthetic
@@ -189,8 +207,10 @@ def run_reference(args):
     times = []
     for _ in range(args.steps):
         t0 = time.perf_counter()
-        c_oracle.decode(heat, depth, centers, w['cfg'], camera, threads=cores)
+        out = c_oracle.decode(heat, depth, centers, w['cfg'], camera, threads=cores)
         times.append(time.perf_counter() - t0)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, out)
     ms = 1e3 * sum(times) / len(times)
     value = sample / (ms / 1e3)
     line = {
@@ -436,6 +456,8 @@ def run_ours(args):
     # K1, behind it (overflow fix-up, grouping + record stores, launch gaps)
     lead_ms = sum(phase_events[i][0].elapsed_time(k1_events[i][0]) for i in k1_events) / len(k1_events)
     tail_ms = sum(k1_events[i][1].elapsed_time(phase_events[i][1]) for i in k1_events) / len(k1_events)
+    if args.dump_outputs and rank == 0:                 # the tables of the last timed step, before anything else reuses them
+        dump_outputs(args.dump_outputs, tables.numpy())
 
     # ---- sustained behaviour: ~1 s of back-to-back steps (the K timed steps above last ~10 ms), clocks sampled throughout ----
     sustained = None
@@ -716,7 +738,12 @@ def main():
                     help="N > 1: gather the records to rank 0 (north_star) or to every rank")
     ap.add_argument('--transport', default='auto', choices=['auto', 'peer', 'nccl'],
                     help="N > 1: how the keypoint records are gathered (sharding.RecordExchange)")
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help="write the tables of the last timed step (rank 0's when N > 1) to DIR/<table>.npy as float32 / float64, "
+                         "at most 60 MB (a fixed seeded sample of frames beyond that)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.frames:
         WORKLOADS[args.workload] = dict(WORKLOADS[args.workload], frames=args.frames)
     if args.impl == 'reference':

@@ -4,12 +4,15 @@ Run in the build container only (needs /root/reference, OpenCV and scikit-learn)
 
     python -m oracle.make_goldens
 
-Every fixture stores the inputs together with what the reference returned for them, converted
-to the fixed-capacity record tables of include/okp.h so tests can compare arrays one to one.
+Every fixture stores the inputs (or, when the seeded generator made them, the recipe and digests
+to rebuild them) together with what the reference returned for them, converted to the
+fixed-capacity record tables of include/okp.h so tests can compare arrays one to one.
 The GPU box has no reference; its tests read these files.
 """
 import contextlib
+import hashlib
 import io
+import json
 import os
 import sys
 
@@ -24,6 +27,14 @@ from object_keypoints_b200 import synthetic                  # noqa: E402
 
 GOLDEN = os.path.join(ROOT, 'tests', 'golden')
 K_PEAKS, O_OBJECTS, V_VOTES = 32, 16, 16
+
+# inputs of the decode fixtures: synthetic.py batches, stored in the fixture as this recipe (JSON)
+VALVE_64 = {'generator': 'make_batch',
+            'args': {'n_frames': 48, 'keypoint_config': [1, 3], 'size': [64, 64], 'seed': 1001, 'objects': [1, 2]}}
+CUPS_64 = {'generator': 'make_batch',
+           'args': {'n_frames': 64, 'keypoint_config': [1, 1, 1], 'size': [64, 64], 'seed': 1002, 'objects': [1, 4]}}
+VALVE_GRID_180x320 = {'generator': 'make_grid_batch',
+                      'args': {'n_frames': 6, 'keypoint_config': [1, 3], 'size': [180, 320], 'seed': 1003}}
 
 
 def reference_camera(camera_utils, size):
@@ -156,13 +167,22 @@ def clean_frames(batch, cfg, cam_dict, wanted):
     return np.array(keep)
 
 
-def decode_case(ref, camera_utils, name, cfg, size, batch, wanted, seed):
+def generated(recipe):
+    """recipe: {'generator': name of a synthetic.py batch function, 'args': its keyword arguments}."""
+    return getattr(synthetic, recipe['generator'])(**recipe['args'])
+
+
+def decode_case(ref, camera_utils, name, recipe, batch, wanted, seed):
+    """Stores the generator recipe, the frames kept and the SHA-256 of each input instead of the noise-like maps
+    (tests/helpers.py rebuilds and checks them), so that the fixture stays a small file."""
+    cfg, size = recipe['args']['keypoint_config'], recipe['args']['size']
     camera = reference_camera(camera_utils, size)
     cam_dict = np_oracle.camera_dict(camera)
     keep = clean_frames(batch, cfg, cam_dict, wanted)
-    heat, depth, centers = batch.heat[keep], batch.depth[keep], batch.centers[keep]
-    tables = reference_tables(ref, camera, heat, depth, centers, cfg, seed)
-    save(name, heat=heat, depth=depth, centers=centers, keypoint_config=np.array(cfg, np.int32),
+    inputs = {'heat': batch.heat[keep], 'depth': batch.depth[keep], 'centers': batch.centers[keep]}
+    tables = reference_tables(ref, camera, inputs['heat'], inputs['depth'], inputs['centers'], cfg, seed)
+    digests = {'sha256_' + k: np.array(hashlib.sha256(np.ascontiguousarray(v).tobytes()).hexdigest()) for k, v in inputs.items()}
+    save(name, input_recipe=np.array(json.dumps(recipe)), **digests, keypoint_config=np.array(cfg, np.int32),
          source_frames=keep, **camera_arrays(camera), **{'ref_' + k: v for k, v in tables.items()})
     return tables
 
@@ -650,14 +670,14 @@ def main():
         return
 
     # 1-2: model-resolution clean sets (bit-exact parity)
-    valve = synthetic.make_batch(48, [1, 3], (64, 64), seed=1001, objects=(1, 2))
-    decode_case(ref, camera_utils, 'valve_64.npz', [1, 3], (64, 64), valve, 24, seed=11)
-    cups = synthetic.make_batch(64, [1, 1, 1], (64, 64), seed=1002, objects=(1, 4))
-    decode_case(ref, camera_utils, 'cups_64.npz', [1, 1, 1], (64, 64), cups, 24, seed=12)
+    valve = generated(VALVE_64)
+    decode_case(ref, camera_utils, 'valve_64.npz', VALVE_64, valve, 24, seed=11)
+    cups = generated(CUPS_64)
+    decode_case(ref, camera_utils, 'cups_64.npz', CUPS_64, cups, 24, seed=12)
 
     # 3: 180x320, eight valves on a grid (config 3 frames)
-    grid = synthetic.make_grid_batch(6, [1, 3], (180, 320), seed=1003)
-    decode_case(ref, camera_utils, 'valve_grid_180x320.npz', [1, 3], (180, 320), grid, 2, seed=13)
+    grid = generated(VALVE_GRID_180x320)
+    decode_case(ref, camera_utils, 'valve_grid_180x320.npz', VALVE_GRID_180x320, grid, 2, seed=13)
 
     # 4: knife edges -- compared with set / flag semantics
     names, cfg, heat, depth, centers = adversarial_frames()

@@ -1,19 +1,44 @@
 """Shared helpers for the parity tests: golden fixtures and table comparison."""
+import hashlib
+import json
 import os
 import types
 
 import numpy as np
 
 GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden')
+INPUTS = ('heat', 'depth', 'centers')
 
 # tolerances stated by BASELINE.json's north_star
 TOL_PIXELS = 1e-3          # 2D sub-pixel positions, px
 TOL_METRES_REL = 1e-4      # 3D points, relative
 
 
+def sha256(array):
+    return hashlib.sha256(np.ascontiguousarray(array).tobytes()).hexdigest()
+
+
 def load_golden(name):
     data = np.load(os.path.join(GOLDEN, name), allow_pickle=False)
-    return {k: data[k] for k in data.files}
+    g = {k: data[k] for k in data.files}
+    if 'input_recipe' in g:
+        g.update(rebuild_inputs(g))
+    return g
+
+
+def rebuild_inputs(g):
+    """Fixtures whose inputs came from the seeded generator store the generator call (input_recipe, JSON), the frames
+    kept (source_frames) and the SHA-256 of each input array instead of the maps themselves: the maps are noise-like
+    and would not fit a small file. They are rebuilt here and must hash to the stored digests, so the reference
+    tables are always compared on exactly the inputs the reference saw."""
+    from object_keypoints_b200 import synthetic
+    recipe = json.loads(str(g['input_recipe']))
+    batch = getattr(synthetic, recipe['generator'])(**recipe['args'])
+    inputs = {k: getattr(batch, k)[g['source_frames']] for k in INPUTS}
+    for k in INPUTS:
+        assert sha256(inputs[k]) == str(g['sha256_' + k]), \
+            f"synthetic.{recipe['generator']}{recipe['args']} no longer reproduces the fixture's {k}"
+    return inputs
 
 
 def golden_camera(g, prefix='cam_'):

@@ -5,7 +5,7 @@ import os
 import numpy as np
 
 from object_keypoints_b200 import camera_utils, linalg, synthetic
-from helpers import load_golden
+from helpers import GOLDEN, INPUTS, load_golden, sha256
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 CALIBRATION = os.path.join(ROOT, 'config', 'calibration.yaml')
@@ -87,10 +87,11 @@ def test_synthetic_generator_is_deterministic_and_separated():
         if len(scene.centers) > 1:
             d = np.linalg.norm(scene.centers[0] - scene.centers[1])
             assert d >= 22.0
-    # the golden fixture was produced by this very generator
-    g = load_golden('valve_64.npz')
+    # the golden fixture was produced by this very generator (it keeps the SHA-256 of the maps it was made from)
+    g = np.load(os.path.join(GOLDEN, 'valve_64.npz'))
     again = synthetic.make_batch(48, [1, 3], (64, 64), seed=1001, objects=(1, 2))
-    np.testing.assert_array_equal(again.heat[g['source_frames']], g['heat'])
+    for k in INPUTS:
+        assert sha256(getattr(again, k)[g['source_frames']]) == str(g['sha256_' + k]), k
 
 
 def test_decode_tables_are_views_into_one_allocation():
@@ -165,3 +166,27 @@ def test_bench_parity_rule_sees_a_single_wrong_value():
         flat[2, column] = np.nextafter(flat[2, column], np.float32(np.inf)) if change is None else \
             flat[2, column] + np.asarray(change, dtype=flat.dtype)
         assert bench.parity_mismatches(got, want) == (6, 1), key
+
+
+def test_bench_dump_is_exact_float_and_bounded(tmp_path):
+    """bench.py --dump-outputs: every table as float32 / float64 holding exactly the decoded values, and beyond the byte
+    budget the same seeded sample of frames on every run."""
+    import os
+    import sys
+    sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
+    import bench
+    from oracle import c_oracle
+    cfg, size = [1, 3], (64, 64)
+    batch = synthetic.make_batch(6, cfg, size, seed=4, objects=(1, 2))
+    want = c_oracle.decode(batch.heat, batch.depth, batch.centers, cfg, synthetic.default_camera(size))
+    bench.dump_outputs(str(tmp_path / 'all'), want)
+    for key, value in want.items():
+        got = np.load(tmp_path / 'all' / f'{key}.npy')
+        assert got.dtype in (np.float32, np.float64) and got.shape == value.shape, key
+        assert np.array_equal(got.astype(value.dtype), value, equal_nan=value.dtype.kind == 'f'), key
+    per_frame = sum(v[0].size * (4 if v.dtype == np.float32 else 8) for v in want.values())
+    for run in ('a', 'b'):
+        bench.dump_outputs(str(tmp_path / run), want, budget=3 * per_frame)
+    frames = np.load(tmp_path / 'a' / 'frame_index.npy')
+    assert len(frames) == 3 and np.array_equal(frames, np.load(tmp_path / 'b' / 'frame_index.npy'))
+    np.testing.assert_array_equal(np.load(tmp_path / 'a' / 'kp_point.npy'), want['kp_point'][frames.astype(int)])
