@@ -31,13 +31,9 @@ class OkpError(RuntimeError):
         super().__init__(f"{where}: {_abi.ERRORS.get(code, code)} ({strerror(code)})")
 
 
-def build(verbose=False, tuning=False, output=None):
-    """Compile csrc/okp_api.cu for sm_100a into libokp.so (nvcc cross-compiles without a GPU).
-    tuning=True adds -DOKP_TUNING_KNOBS: the OKP_* environment variables of tools/sweep_k1.py override the launch-plan
-    constants (the shipped library reads no environment). output: write the library there instead of libokp.so (the sweep
-    tools build libokp_tuning.so beside the shipped one and point LIBRARY_PATH at it before the first lib() call)."""
+def build(verbose=False):
+    """Compile csrc/okp_api.cu for sm_100a into libokp.so (nvcc cross-compiles without a GPU)."""
     import subprocess
-    target = LIBRARY_PATH if output is None else output
     src = os.path.join(_HERE, 'csrc', 'okp_api.cu')
     # the host side of the sparse transfer is plain C++ (OpenMP; its AVX2 loop is a run-time-dispatched target function,
     # so no -mavx2 here and the file also builds on aarch64 hosts): g++ compiles it, nvcc links it in
@@ -48,17 +44,15 @@ def build(verbose=False, tuning=False, output=None):
     if host.returncode != 0:
         raise RuntimeError("g++ failed:\n" + host.stdout + host.stderr)
     cmd = ['nvcc', '-gencode', 'arch=compute_100a,code=sm_100a', '-O3', '-lineinfo', '-fmad=false',
-           '-std=c++17', '-Xcompiler', '-fPIC', '-shared', '-cudart', 'static', '-o', target, src, host_obj, '-lgomp']
-    if tuning:
-        cmd.insert(1, '-DOKP_TUNING_KNOBS')
+           '-std=c++17', '-Xcompiler', '-fPIC', '-shared', '-cudart', 'static', '-o', LIBRARY_PATH, src, host_obj, '-lgomp']
     if verbose:
         cmd.insert(1, '-Xptxas')
         cmd.insert(2, '-v')
     result = subprocess.run(cmd, capture_output=True, text=True)
     if result.returncode != 0:
         raise RuntimeError("nvcc failed:\n" + result.stdout + result.stderr)
-    with open(target + '.stamp', 'w') as handle:
-        handle.write(_source_digest() + ('\ntuning' if tuning else '') + '\n')
+    with open(STAMP_PATH, 'w') as handle:
+        handle.write(_source_digest() + '\n')
     return result.stdout + result.stderr
 
 
@@ -83,7 +77,7 @@ def needs_build():
     if not os.path.exists(LIBRARY_PATH) or not os.path.exists(STAMP_PATH):
         return True
     with open(STAMP_PATH) as handle:
-        return handle.read().split('\n')[0].strip() != _source_digest()
+        return handle.read().strip() != _source_digest()
 
 
 def lib():
@@ -93,7 +87,7 @@ def lib():
     if not os.path.exists(LIBRARY_PATH):
         raise ImportError(f"{LIBRARY_PATH} is missing: build it with `python -c 'import __graft_entry__ as g; g.build()'` "
                           "(there is no CPU fallback for the decode path)")
-    if LIBRARY_PATH.endswith('libokp.so') and needs_build():
+    if needs_build():
         import warnings
         warnings.warn(f"{LIBRARY_PATH} is older than its sources (csrc/, include/okp.h): rebuild it with "
                       "`python -c 'import __graft_entry__ as g; g.build()'`", RuntimeWarning, stacklevel=2)

@@ -8,9 +8,6 @@
 #include "okp_peaks.cuh"
 #include "okp_peaks_strip.cuh"
 #include "okp_peaks_stream.cuh"
-#ifdef OKP_TUNING_KNOBS
-#include "okp_peaks_tile.cuh"      // experimental sparse tile form of K1: tuning build only (profiles/r02e_tile_kernel.md)
-#endif
 #include "okp_geometry.cuh"
 #include "okp_group.cuh"
 #include "okp_dlt.cuh"
@@ -25,9 +22,8 @@ namespace {
 constexpr int kSmCount = 148;            // B200: 2 dies x 74 SMs
 
 struct PeakPlan {
-    bool strip;                          // tuned TMA kernel (tile or stream) + overflow path, else generic tile kernel + merge
-    bool tile;                           // the sparse tile kernel (okp_peaks_tile.cuh) covers the call, else the stream kernel
-    OkpStripPlan sp;
+    bool strip;                          // the stream kernel (plan sp) + overflow path, else generic tile kernel + merge
+    OkpStreamPlan sp;                    // peaks only (sp.F = 0)
     OkpTileGeometry geo;                 // generic tiles (also the strip kernel's overflow path)
     size_t smem_bytes;
     int grid;
@@ -36,18 +32,12 @@ struct PeakPlan {
 
 inline int round_up(int v, int m) { return (v + m - 1) / m * m; }
 
-PeakPlan plan_peaks(int maps, int H, int W, int K, int esize, const OkpDecodeParams* prm) {
+PeakPlan plan_peaks(int maps, int C, int H, int W, int K, int esize, const OkpDecodeParams* prm) {
     PeakPlan p;
     memset(&p, 0, sizeof(p));
-    // the tuned TMA kernels implement the reference's configuration only (5x5 window on the 5x5 box sum)
+    // the stream kernel implements the reference's configuration only (5x5 window on the 5x5 box sum)
     const bool reference_mode = prm->nms_size == 5 && prm->box_sum == 1;
-    p.tile = false;
-#ifdef OKP_TUNING_KNOBS
-    OkpTilePlan probe;
-    p.tile = reference_mode && okp_env_int("OKP_PEAKS_TILE", 0, 1, 0) != 0 &&
-             okp_tile_plan(maps, 1, H, W, K, esize, prm->threshold, 0, prm->lean_tables, &probe);
-#endif
-    p.strip = p.tile || (reference_mode && okp_strip_plan(maps, H, W, K, esize, &p.sp));
+    p.strip = reference_mode && okp_stream_plan(maps, C, H, W, K, esize, 0, prm->lean_tables, &p.sp);
     p.geo.H = H; p.geo.W = W; p.geo.maps = maps;
     p.geo.radius = prm->nms_size / 2; p.geo.box_sum = prm->box_sum ? 1 : 0;
     p.geo.TW = W <= 64 ? round_up(W, 8) : 64;
@@ -89,8 +79,8 @@ inline int overflow_grid(int maps) { return maps < OKP_OVERFLOW_CTAS ? maps : OK
 inline int overflow_maps_per_cta(int maps) { return (maps + overflow_grid(maps) - 1) / overflow_grid(maps); }
 
 // tile lists: one per (map, tile) for the generic kernels, one per (overflow CTA, tile) for the strip path
-size_t workspace_for(const PeakPlan& p, int maps, int K, bool strip) {
-    const size_t tiles = strip ? (size_t)overflow_grid(maps) * p.tiles_per_map : (size_t)maps * p.tiles_per_map;
+size_t workspace_for(const PeakPlan& p, int maps, int K) {
+    const size_t tiles = p.strip ? (size_t)overflow_grid(maps) * p.tiles_per_map : (size_t)maps * p.tiles_per_map;
     // + alignment slack in front, + the launch's group counter (okp_peaks_stream.cuh) behind the lists
     return align_up(tiles * sizeof(int32_t), 256) + align_up(tiles * K * sizeof(OkpPeakRecord), 256) + 256 + 256;
 }
@@ -120,8 +110,8 @@ size_t okp_decode_workspace_bytes(int N, int C, int H, int W, const OkpDecodePar
     // enough for either element type (their launch plans can differ: bf16 rows need W % 8 == 0 for TMA)
     size_t need = 0;
     for (int esize = 2; esize <= 4; esize += 2) {
-        const PeakPlan p = plan_peaks(N * C, H, W, params->max_peaks, esize, params);
-        const size_t bytes = workspace_for(p, N * C, params->max_peaks, p.strip);
+        const PeakPlan p = plan_peaks(N * C, C, H, W, params->max_peaks, esize, params);
+        const size_t bytes = workspace_for(p, N * C, params->max_peaks);
         if (bytes > need) need = bytes;
     }
     return need;
@@ -134,7 +124,6 @@ namespace {
 // Everything the peak entry checks before it launches; fills the plan and the workspace carving.
 struct PeakCall {
     PeakPlan plan;
-    bool strip;
     int32_t* tile_count;
     OkpPeakRecord* tile_peaks;
     int* group_counter;                  // one int the stream kernel's CTAs claim their groups from
@@ -152,13 +141,12 @@ int prepare_peaks(const T* heat_dev, int N, int C, int H, int W, const OkpDecode
         return OKP_E_UNSUPPORTED;
     const int K = params->max_peaks;
     const int maps = N * C;
-    call->plan = plan_peaks(maps, H, W, K, (int)sizeof(T), params);
-    call->strip = call->plan.strip;
+    call->plan = plan_peaks(maps, C, H, W, K, (int)sizeof(T), params);
     // TMA needs a 16-byte aligned base. The generic kernels would take the map, but with a workspace orders of magnitude
     // larger than okp_decode_workspace_bytes() advertises for this shape: refuse instead of failing later
-    if (call->strip && ((uintptr_t)heat_dev & 15u) != 0) return OKP_E_UNSUPPORTED;
-    if (workspace_bytes < workspace_for(call->plan, maps, K, call->strip)) return OKP_E_WORKSPACE;
-    const size_t tiles = call->strip ? (size_t)overflow_grid(maps) * call->plan.tiles_per_map : (size_t)maps * call->plan.tiles_per_map;
+    if (call->plan.strip && ((uintptr_t)heat_dev & 15u) != 0) return OKP_E_UNSUPPORTED;
+    if (workspace_bytes < workspace_for(call->plan, maps, K)) return OKP_E_WORKSPACE;
+    const size_t tiles = call->plan.strip ? (size_t)overflow_grid(maps) * call->plan.tiles_per_map : (size_t)maps * call->plan.tiles_per_map;
     uintptr_t base = align_up((uintptr_t)workspace_dev, 256);
     call->tile_count = (int32_t*)base;
     call->tile_peaks = (OkpPeakRecord*)(base + align_up(tiles * sizeof(int32_t), 256));
@@ -178,6 +166,35 @@ int launch_overflow(const T* heat_dev, const PeakCall& call, int maps, const Okp
     return OKP_OK;
 }
 
+// The peak extraction's launches for a prepared call: the stream kernel + overflow fix-up, or the generic kernels + merge.
+template <typename T>
+int launch_peaks(const T* heat_dev, const PeakCall& call, int maps, int C, int W, const OkpDecodeParams* params,
+                 const OkpDecodeTables* tables, cudaStream_t s, void* event_before = nullptr, void* event_after = nullptr) {
+    const int K = params->max_peaks;
+    const PeakPlan& p = call.plan;
+    if (p.strip) {
+        int rc = okp_stream_launch<T>(heat_dev, p.sp, params->threshold, *tables, nullptr, call.group_counter, s,
+                                      (cudaEvent_t)event_before, (cudaEvent_t)event_after);
+        if (rc != OKP_OK) return rc;
+        rc = launch_overflow<T>(heat_dev, call, maps, params, tables, s);
+        if (rc != OKP_OK) return rc;
+    } else {
+        auto kernel = okp_peaks_generic_kernel<256, T>;
+        OKP_CUDA_CHECK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p.smem_bytes));
+        kernel<<<p.grid, 256, p.smem_bytes, s>>>(heat_dev, p.geo, params->threshold, K, call.tile_count, call.tile_peaks);
+        OKP_CUDA_CHECK(cudaGetLastError());
+        const int warps_per_block = 4;
+        okp_merge_peaks_kernel<<<(maps + warps_per_block - 1) / warps_per_block, warps_per_block * 32, 0, s>>>(
+            call.tile_count, call.tile_peaks, maps, p.tiles_per_map, W, K, C, *tables);
+        OKP_CUDA_CHECK(cudaGetLastError());
+    }
+    if (params->top_k > 0) {
+        okp_topk_kernel<<<(maps + 3) / 4, 128, 0, s>>>(maps, K, params->top_k, *tables);
+        OKP_CUDA_CHECK(cudaGetLastError());
+    }
+    return OKP_OK;
+}
+
 template <typename T>
 int extract_peaks(const T* heat_dev, int N, int C, int H, int W, const OkpDecodeParams* params,
                   const OkpDecodeTables* tables, void* workspace_dev, size_t workspace_bytes, void* stream,
@@ -190,49 +207,7 @@ int extract_peaks(const T* heat_dev, int N, int C, int H, int W, const OkpDecode
     PeakCall call;
     rc = prepare_peaks<T>(heat_dev, N, C, H, W, params, tables, workspace_dev, workspace_bytes, &call);
     if (rc != OKP_OK) return rc;
-    cudaStream_t s = (cudaStream_t)stream;
-    const int K = params->max_peaks;
-    const int maps = N * C;
-    const PeakPlan& p = call.plan;
-
-    if (call.strip) {
-#ifdef OKP_TUNING_KNOBS
-        if (p.tile) {
-            OkpTilePlan tile_plan;
-            if (!okp_tile_plan(maps, C, H, W, K, (int)sizeof(T), params->threshold, 0, params->lean_tables, &tile_plan)) return OKP_E_UNSUPPORTED;
-            rc = okp_tile_launch<T>(heat_dev, tile_plan, params->threshold, *tables, nullptr, s);
-        } else
-#endif
-        {
-            OkpStreamPlan stream_plan;
-            if (!okp_stream_plan(maps, C, H, W, K, (int)sizeof(T), 0, params->lean_tables, &stream_plan)) return OKP_E_UNSUPPORTED;
-            rc = okp_stream_launch<T>(heat_dev, stream_plan, params->threshold, *tables, nullptr, call.group_counter, s,
-                                      (cudaEvent_t)event_before, (cudaEvent_t)event_after);
-        }
-        if (rc != OKP_OK) return rc;
-        rc = launch_overflow<T>(heat_dev, call, maps, params, tables, s);
-        if (rc != OKP_OK) return rc;
-        if (params->top_k > 0) {
-            okp_topk_kernel<<<(maps + 3) / 4, 128, 0, s>>>(maps, K, params->top_k, *tables);
-            OKP_CUDA_CHECK(cudaGetLastError());
-        }
-        return OKP_OK;
-    }
-    {
-        auto kernel = okp_peaks_generic_kernel<256, T>;
-        OKP_CUDA_CHECK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p.smem_bytes));
-        kernel<<<p.grid, 256, p.smem_bytes, s>>>(heat_dev, p.geo, params->threshold, K, call.tile_count, call.tile_peaks);
-        OKP_CUDA_CHECK(cudaGetLastError());
-    }
-    const int warps_per_block = 4;
-    okp_merge_peaks_kernel<<<(maps + warps_per_block - 1) / warps_per_block, warps_per_block * 32, 0, s>>>(
-        call.tile_count, call.tile_peaks, maps, p.tiles_per_map, W, K, C, *tables);
-    OKP_CUDA_CHECK(cudaGetLastError());
-    if (params->top_k > 0) {
-        okp_topk_kernel<<<(maps + 3) / 4, 128, 0, s>>>(maps, K, params->top_k, *tables);
-        OKP_CUDA_CHECK(cudaGetLastError());
-    }
-    return OKP_OK;
+    return launch_peaks<T>(heat_dev, call, N * C, C, W, params, tables, (cudaStream_t)stream, event_before, event_after);
 }
 
 int convert_sink(const OkpRecordSink* sink, int O, int C, int P, OkpRecordSinks* out) {
@@ -305,8 +280,7 @@ int launch_group_lanes(const OkpGroupArgs& a, int only_pending, const OkpDecodeT
 // Small frames hold few peaks (a 64x64 valve frame: ~10): half a warp per frame, two frames per warp (okp_group.cuh).
 template <typename T>
 int launch_group(const OkpGroupArgs& a, int only_pending, const OkpDecodeTables* tables, cudaStream_t s) {
-    const bool small = (long long)a.H * a.W <= 96LL * 96LL && 2 * (size_t)a.frame_smem_bytes <= 48 * 1024 &&
-                       okp_env_int("OKP_GROUP_LANES", 16, 32, 16) == 16;
+    const bool small = (long long)a.H * a.W <= 96LL * 96LL && 2 * (size_t)a.frame_smem_bytes <= 48 * 1024;
     return small ? launch_group_lanes<T, 16>(a, only_pending, tables, s) : launch_group_lanes<T, 32>(a, only_pending, tables, s);
 }
 
@@ -344,35 +318,21 @@ int decode(const T* heat_dev, const T* depth_dev, const T* centers_dev, int N, i
     rc = prepare_peaks<T>(heat_dev, N, C, H, W, params, tables, workspace_dev, workspace_bytes, &call);
     if (rc != OKP_OK) return rc;
     cudaStream_t s = (cudaStream_t)stream;
-    OkpStreamPlan stream_plan;
-#ifdef OKP_TUNING_KNOBS
-    OkpTilePlan tile_plan;
-#endif
     // One fused pass (grouping in the peak kernel's epilogue warps) or two launches (peaks, then one warp per frame): the
     // grouping is a chain of latencies (gathers from HBM, float64 Newton + tan), and a launch of its own overlaps thousands
     // of them where the fused form has two epilogue warps per SM. Measured (profiles/r02c_fused_vs_split.txt): the split
-    // form is faster at every size, so it is the default; OkpDecodeParams.single_pass asks for the fused one.
-    bool fused = params->single_pass != 0 && call.strip && params->top_k == 0;
-    if (fused) {
-#ifdef OKP_TUNING_KNOBS
-        if (call.plan.tile)
-            fused = okp_tile_plan(N * C, C, H, W, params->max_peaks, (int)sizeof(T), params->threshold, a.frame_smem_bytes,
-                                  params->lean_tables, &tile_plan) && tile_plan.sp.F > 0;
-        else
-#endif
-            fused = okp_stream_plan(N * C, C, H, W, params->max_peaks, (int)sizeof(T), a.frame_smem_bytes, params->lean_tables,
-                                    &stream_plan) && stream_plan.F > 0;
-    }
+    // form is faster at every size, so it is the default; OkpDecodeParams.single_pass asks for the fused one, whose groups
+    // are whole frames with their grouping scratch: a plan of its own.
+    OkpStreamPlan fused_plan;
+    const bool fused = params->single_pass != 0 && call.plan.strip && params->top_k == 0 &&
+                       okp_stream_plan(N * C, C, H, W, params->max_peaks, (int)sizeof(T), a.frame_smem_bytes, params->lean_tables,
+                                       &fused_plan) && fused_plan.F > 0;
     if (!fused) {
-        rc = extract_peaks<T>(heat_dev, N, C, H, W, params, tables, workspace_dev, workspace_bytes, stream);
+        rc = launch_peaks<T>(heat_dev, call, N * C, C, W, params, tables, s);
         if (rc != OKP_OK) return rc;
         return launch_group<T>(a, 0, tables, s);
     }
-#ifdef OKP_TUNING_KNOBS
-    if (call.plan.tile) rc = okp_tile_launch<T>(heat_dev, tile_plan, params->threshold, *tables, &a, s);
-    else
-#endif
-        rc = okp_stream_launch<T>(heat_dev, stream_plan, params->threshold, *tables, &a, call.group_counter, s);
+    rc = okp_stream_launch<T>(heat_dev, fused_plan, params->threshold, *tables, &a, call.group_counter, s);
     if (rc != OKP_OK) return rc;
     // fix-up launches: maps that overflowed the fast path are redone exactly, then their frames are grouped. With no such
     // map each is one read of peak_count / n_objects

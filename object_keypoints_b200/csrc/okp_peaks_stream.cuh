@@ -29,7 +29,7 @@
 #include "okp_group.cuh"
 
 struct OkpStreamPlan {
-    OkpStripPlan s;               // geometry, M, NS, stage layout (smem offsets below replace s.off_*)
+    OkpStripPlan s;               // geometry, M, NS, stage layout
     int groups;                   // ceil(maps / M)
     int EW;                       // epilogue warps
     int off_pending[2], off_count[2];   // candidate lists and [n_pending[M], redo[M]] per buffer
@@ -38,7 +38,6 @@ struct OkpStreamPlan {
     int C;                        // maps per frame
     int F;                        // fused: frames per group (M = F * C); 0 = peaks only
     int lean;                     // OkpDecodeParams.lean_tables
-    int edge_only;                // 1: every batch runs the border-checked step variant (small maps: one variant in the i-cache)
     int smem_bytes;
     int threads;                  // compute warps + producer warp + epilogue warps
 };
@@ -47,15 +46,14 @@ __device__ __forceinline__ void okp_named_barrier(int id, int threads) {
     asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(threads) : "memory");
 }
 
-// The epilogue warps' loop (shared by the stream kernel above and the tile kernel of okp_peaks_tile.cuh): one finished
-// candidate buffer at a time -- exact box sums from L2, undecided neighbours, raster ranks, table rows and, fused, the
-// frame's grouping and 3D lift. et: thread index among the sp.EW epilogue warps. claimed: the CTA's groups are the ones its
-// producer lane claimed from the launch's counter (ids in the ring behind the mbarriers, -1 = no more), else group
-// blockIdx.x + it * gridDim.x for it < my_groups.
+// The epilogue warps' loop of the stream kernel below: one finished candidate buffer at a time -- exact box sums from L2,
+// undecided neighbours, raster ranks, table rows and, fused, the frame's grouping and 3D lift. et: thread index among the
+// sp.EW epilogue warps. The CTA's groups are the ones its producer lane claimed from the launch's counter (ids in the ring
+// behind the mbarriers, -1 = no more).
 template <typename T, bool FUSED>
 __device__ __forceinline__ void okp_stream_epilogue(unsigned char* smem, const OkpStreamPlan& sp, const T* __restrict__ heat,
                                                     const float threshold, const OkpDecodeTables& t, const OkpGroupArgs& ga,
-                                                    const int et, const int my_groups, const bool claimed) {
+                                                    const int et) {
     const OkpStripPlan& p = sp.s;
     const int H = p.H, W = p.W;
     OkpStripPeak* peaks = reinterpret_cast<OkpStripPeak*>(smem + sp.off_peaks);                // [M][PK]
@@ -66,12 +64,12 @@ __device__ __forceinline__ void okp_stream_epilogue(unsigned char* smem, const O
     int* pend = cand_start + p.M + 1;                                                          // [M] fused: frame f is left to the fix-up launches
     uint64_t* cand_full = reinterpret_cast<uint64_t*>(smem + sp.off_mbar) + 2 * OKP_STRIP_MAX_NS;
     uint64_t* cand_free = cand_full + 2;
-    const volatile int* group_ring = reinterpret_cast<const volatile int*>(cand_free + 2);    // [8] claimed group ids (claimed)
+    const volatile int* group_ring = reinterpret_cast<const volatile int*>(cand_free + 2);    // [8] claimed group ids
     const int ethreads = sp.EW * 32;
-    for (int it = 0; claimed || it < my_groups; ++it) {
+    for (int it = 0;; ++it) {
         const int buf = it & 1;
         okp_mbar_wait(cand_full + buf, (uint32_t)((it >> 1) & 1), 400);
-        const int group = claimed ? group_ring[it & 7] : blockIdx.x + it * gridDim.x;
+        const int group = group_ring[it & 7];
         if (group < 0) break;                                                                  // the end marker
         const int first_map = group * p.M;
         OkpStripCandidate* pending = reinterpret_cast<OkpStripCandidate*>(smem + sp.off_pending[buf]);
@@ -402,7 +400,7 @@ okp_peaks_stream_kernel(const __grid_constant__ CUtensorMap tmap, const T* __res
                 if (b > 0) okp_mbar_wait(full + stage, full_parity);
                 const unsigned char* raw = smem + (size_t)stage * p.stage_bytes + thread_raw;
                 const int y0 = b * RB - 4;
-                if (!sp.edge_only && b >= 2 && y0 + 4 < H)
+                if (b >= 2 && y0 + 4 < H)
                     okp_strip_batch<false, T>(raw, row_pitch, pr, hp, sv, sign, y0, L);
                 else
                     okp_strip_batch<true, T>(raw, row_pitch, pr, hp, sv, sign, y0, L);
@@ -416,48 +414,70 @@ okp_peaks_stream_kernel(const __grid_constant__ CUtensorMap tmap, const T* __res
         }
     } else {
         // ------------------------------- epilogue warps: one finished candidate buffer at a time ---------
-        okp_stream_epilogue<T, FUSED>(smem, sp, heat, threshold, t, ga, tid - (compute_warps + 1) * 32, 0, true);
+        okp_stream_epilogue<T, FUSED>(smem, sp, heat, threshold, t, ga, tid - (compute_warps + 1) * 32);
     }
 }
 
-// C: maps per frame. group_frame_bytes > 0 asks for the fused form: groups of whole frames plus one grouping scratch
-// (group_frame_bytes each) per frame of a group; returns with sp.F == 0 when not even one frame fits a group (the caller
-// then runs the peak kernel and okp_group_kernel separately).
+// The stream kernel's plan for `maps` maps of H x W elements of esize bytes (4: float32, 2: bfloat16), K table rows per map,
+// C maps per frame; false when the kernel does not cover the shape (the caller runs the generic kernels). group_frame_bytes
+// > 0 asks for the fused form: groups of whole frames plus one grouping scratch (group_frame_bytes each) per frame of a
+// group; false when not even one frame fits a group (the caller then runs the peak kernel and okp_group_kernel separately).
 static inline bool okp_stream_plan(int maps, int C, int H, int W, int K, int esize, int group_frame_bytes, int lean,
                                    OkpStreamPlan* out) {
+    const int align = 16 / esize;                         // elements per 16 bytes: TMA box starts and row pitches
+    if (maps < 1 || H < 1 || W < 4 || (W % 4) != 0 || (W % align) != 0 || W > 500) return false;
     OkpStreamPlan sp;
     memset(&sp, 0, sizeof(sp));
-    if (!okp_strip_plan(maps, H, W, K, esize, &sp.s)) return false;
     OkpStripPlan& p = sp.s;
+    p.H = H; p.W = W; p.maps = maps; p.K = K; p.esize = esize;
+    p.strips = W / 4 + 1;
+    p.lead[0] = align - 4;                                // box 0 starts at column -4 - lead[0] = -align
+    if (4 * p.strips + 4 + p.lead[0] <= 256) {
+        p.halves = 1; p.half_strips = p.strips;
+    } else {
+        p.halves = 2; p.half_strips = (p.strips + 1) / 2;
+        p.lead[1] = (4 * p.half_strips - 4) % align;      // box 1 starts at the aligned column below 4 * half_strips - 4
+    }
+    // columns 4s-4 .. 4s+3 of the box's strips behind the lead, rounded up to whole 16-byte units
+    p.BW = okp_round_up_int(4 * p.half_strips + 4 + (p.lead[0] > p.lead[1] ? p.lead[0] : p.lead[1]), align);
+    if (p.BW > 256) return false;                         // a TMA box holds at most 256 elements per dimension
+    p.nb = (H + 6 + OKP_STRIP_RB - 1) / OKP_STRIP_RB;
+    p.PK = 2 * K;
+    // maps per group, first estimate: as many as the shared-memory budget (110 KB: two CTAs per SM) and 256 compute threads
+    // allow, counted with four stages (small maps too) and one candidate buffer; the layout loop below settles it. 256
+    // compute threads + the producer warp + one epilogue warp = 320 threads: two CTAs per SM at 96 registers. (288 let a
+    // 64x64 bfloat16 plan -- more maps fit its shared-memory budget -- grow to 352 threads, i.e. ONE CTA per SM: 719 us
+    // against the float32 plan's 454 us for the same pixels, profiles/r02f_bench_k1.txt)
+    const int budget = 110 * 1024;
+    const int per_map = 4 * OKP_STRIP_RB * p.BW * p.halves * esize +
+                        p.PK * (int)(sizeof(OkpStripCandidate) + sizeof(OkpStripPeak)) + 64 * 4 + 12;
+    int M = (budget - 1024) / per_map;
+    if (M > 256 / p.strips) M = 256 / p.strips;
+    if (M > maps) M = maps;
+    if (M < 1) {
+        M = 1;
+        if (per_map + 1024 > 224 * 1024 || p.strips > OKP_STRIP_MAX_THREADS - 32) return false;
+    }
     // small maps (64x64: 14 row batches per group): 224 compute threads leave room for a second epilogue warp inside 320
     // threads, and three stages stream as well as four (r02h / r02i sweeps: 464 -> 440 us float32, 566 -> 505 us bfloat16)
     const bool small_map = p.nb <= 20;
-    if (small_map) {
-        if (okp_env_int("OKP_STRIP_STAGES", 0, OKP_STRIP_MAX_NS, 0) == 0) p.NS = 3;
-        const int cap = okp_env_int("OKP_STRIP_THREADS", 0, OKP_STRIP_MAX_THREADS - 32, 0) == 0 ? 224 : OKP_STRIP_MAX_THREADS;
-        if (p.M * p.strips > cap && cap / p.strips >= 1) p.M = cap / p.strips;      // resized below
-    }
+    p.NS = small_map ? 3 : 4;
+    if (small_map && M * p.strips > 224) M = 224 / p.strips;
     sp.C = C;
     sp.lean = lean;
     const bool fused = group_frame_bytes > 0;
-    if (fused && p.M < C) return false;
-    auto resize = [&](int M) {
-        p.M = M;
+    if (fused && M < C) return false;
+    auto resize = [&](int m) {
+        p.M = m;
         p.threads = p.M * p.strips;
         p.IC = p.M * 64;
         p.half_bytes = p.M * OKP_STRIP_RB * p.BW * esize;
         p.half_stride = okp_round_up_int(p.half_bytes, 128);
         p.stage_bytes = p.halves * p.half_stride;
     };
-    resize(fused ? p.M / C * C : p.M);
-    // every batch on the border-checked variant of the row step (one variant instead of two in the instruction cache): helped
-    // small bfloat16 maps with the static group assignment (r02i: 505 -> 487 us), not with claimed groups (r02u: 448 -> 454 us)
-    // and never float32 (440 -> 472 us): off, kept as a knob of the tuning build
-    sp.edge_only = okp_env_int("OKP_STREAM_EDGE_ONLY", 0, 1, 0);
-    sp.EW = okp_env_int("OKP_STREAM_EPILOGUE_WARPS", 0, 4, 0);    // 0: decided below, once M is known
+    resize(fused ? M / C * C : M);
     // the second candidate buffer costs PK * 8 bytes per map: give it back from the per-CTA budget by re-planning M
-    const int budget = okp_env_int("OKP_STRIP_SMEM_KB", 16, 224, 110) * 1024;
-    const int compute_limit = OKP_STRIP_MAX_THREADS - 32 - (sp.EW ? sp.EW : 2) * 32;
+    const int compute_limit = OKP_STRIP_MAX_THREADS - 32 - 2 * 32;   // beside the producer warp and up to two epilogue warps
     for (;;) {
         int off = p.NS * p.stage_bytes;
         for (int b = 0; b < 2; ++b) { sp.off_pending[b] = off; off += p.M * p.PK * (int)sizeof(OkpStripCandidate); }
@@ -479,7 +499,7 @@ static inline bool okp_stream_plan(int maps, int C, int H, int W, int K, int esi
     // two epilogue warps where they fit beside the compute warps in 320 threads (two CTAs per SM at 96 registers), else
     // one: small maps (64x64: 14 row batches per group) finish a group every few microseconds and one warp cannot keep
     // up (profiles/r01m_k1_64x64_ncu.md)
-    if (sp.EW == 0) sp.EW = (p.threads + 31) / 32 * 32 + 32 + 64 <= 320 ? 2 : 1;
+    sp.EW = (p.threads + 31) / 32 * 32 + 32 + 64 <= 320 ? 2 : 1;
     sp.groups = (maps + p.M - 1) / p.M;
     sp.threads = (p.threads + 31) / 32 * 32 + 32 + sp.EW * 32;
     *out = sp;

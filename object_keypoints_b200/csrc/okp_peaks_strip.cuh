@@ -41,7 +41,6 @@
 // that hand-over.
 #pragma once
 #include <cuda.h>
-#include <stdlib.h>
 
 #include "okp_common.cuh"
 #include "okp_peaks.cuh"
@@ -71,9 +70,6 @@ struct OkpStripPlan {
     int half_bytes;               // bytes of one TMA box: M * RB * BW * esize
     int half_stride;              // half_bytes rounded up to 128 (TMA destinations are 128-byte aligned)
     int stage_bytes;              // halves * half_stride
-    int off_pending, off_peaks, off_items, off_count, off_mbar;
-    int smem_bytes;
-    int grid;
 };
 
 struct OkpStripPeak { int32_t key; float score, cx, cy, conf; };   // key < 0: not a peak
@@ -287,79 +283,9 @@ __device__ __forceinline__ void okp_strip_batch(const unsigned char* raw, int ro
 }
 
 // ---------------------------------------------------------------------------------------------
-// host side: plan + tensor map + launch
+// host side: tensor map encoder (the plan and the launch are in okp_peaks_stream.cuh)
 // ---------------------------------------------------------------------------------------------
 static inline int okp_round_up_int(int v, int m) { return (v + m - 1) / m * m; }
-
-// Launch-plan constants. The library keeps no global state and reads no environment: the values below are the shipped
-// ones. A build with -DOKP_TUNING_KNOBS (python -c "from object_keypoints_b200 import _lib; _lib.build(tuning=True)";
-// tools/sweep_k1.py) lets OKP_* environment variables override them for parameter sweeps.
-static inline int okp_env_int(const char* name, int lo, int hi, int fallback) {
-#ifdef OKP_TUNING_KNOBS
-    const char* e = getenv(name);
-    if (!e) return fallback;
-    const int v = atoi(e);
-    return v >= lo && v <= hi ? v : fallback;
-#else
-    (void)name; (void)lo; (void)hi;
-    return fallback;
-#endif
-}
-
-static inline bool okp_strip_plan(int maps, int H, int W, int K, int esize, OkpStripPlan* out) {
-    const int align = 16 / esize;                         // elements per 16 bytes: TMA box starts and row pitches
-    if (maps < 1 || H < 1 || W < 4 || (W % 4) != 0 || (W % align) != 0 || W > 500) return false;
-    OkpStripPlan p;
-    memset(&p, 0, sizeof(p));
-    p.H = H; p.W = W; p.maps = maps; p.K = K; p.esize = esize;
-    p.strips = W / 4 + 1;
-    p.lead[0] = align - 4;                                // box 0 starts at column -4 - lead[0] = -align
-    if (4 * p.strips + 4 + p.lead[0] <= 256) {
-        p.halves = 1; p.half_strips = p.strips;
-    } else {
-        p.halves = 2; p.half_strips = (p.strips + 1) / 2;
-        p.lead[1] = (4 * p.half_strips - 4) % align;      // box 1 starts at the aligned column below 4 * half_strips - 4
-    }
-    // columns 4s-4 .. 4s+3 of the box's strips behind the lead, rounded up to whole 16-byte units
-    p.BW = okp_round_up_int(4 * p.half_strips + 4 + (p.lead[0] > p.lead[1] ? p.lead[0] : p.lead[1]), align);
-    if (p.BW > 256) return false;                         // a TMA box holds at most 256 elements per dimension
-    p.nb = (H + 6 + OKP_STRIP_RB - 1) / OKP_STRIP_RB;
-    p.NS = okp_env_int("OKP_STRIP_STAGES", 2, OKP_STRIP_MAX_NS, 4);
-    p.PK = 2 * K;
-    const int items_per_map = 64;
-    const int per_map = p.NS * OKP_STRIP_RB * p.BW * p.halves * esize +
-                        p.PK * (int)(sizeof(OkpStripCandidate) + sizeof(OkpStripPeak)) + items_per_map * 4 + 12;
-    const int budget = okp_env_int("OKP_STRIP_SMEM_KB", 16, 224, 110) * 1024;   // default: two CTAs per SM
-    // 256 compute threads + the producer warp + one epilogue warp = 320 threads: two CTAs per SM at 96 registers. (288 let a
-    // 64x64 bfloat16 plan -- more maps fit its shared-memory budget -- grow to 352 threads, i.e. ONE CTA per SM: 719 us
-    // against the float32 plan's 454 us for the same pixels, profiles/r02f_bench_k1.txt)
-    const int max_threads = okp_env_int("OKP_STRIP_THREADS", 32, OKP_STRIP_MAX_THREADS - 32, 256);
-    int M = (budget - 1024) / per_map;
-    if (M > max_threads / p.strips) M = max_threads / p.strips;
-    if (M > maps) M = maps;
-    if (M > 256) M = 256;
-    if (M < 1) {
-        M = 1;
-        if (per_map + 1024 > 224 * 1024 || p.strips > OKP_STRIP_MAX_THREADS - 32) return false;
-    }
-    p.M = M;
-    p.threads = M * p.strips;
-    p.IC = M * items_per_map;
-    p.half_bytes = M * OKP_STRIP_RB * p.BW * esize;
-    p.half_stride = okp_round_up_int(p.half_bytes, 128);
-    p.stage_bytes = p.halves * p.half_stride;
-    int off = p.NS * p.stage_bytes;
-    p.off_pending = off; off += M * p.PK * (int)sizeof(OkpStripCandidate);
-    p.off_peaks = off; off += M * p.PK * (int)sizeof(OkpStripPeak);
-    p.off_items = off; off += p.IC * 4;
-    p.off_count = off; off += (3 * M + 1) * 4;
-    off = okp_round_up_int(off, 8);
-    p.off_mbar = off; off += 2 * OKP_STRIP_MAX_NS * 8;
-    p.smem_bytes = off;
-    p.grid = (maps + M - 1) / M;
-    *out = p;
-    return true;
-}
 
 typedef CUresult (*OkpEncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
                                      const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,

@@ -3,9 +3,7 @@ usage: python tools/bench_k1.py [180x320|64x64] [frames] [reps] [f32|bf16] [lean
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
-from object_keypoints_b200 import KeypointDecoder, synthetic, _lib
-if os.environ.get('OKP_TUNING_LIBRARY'):                 # knob sweeps: the -DOKP_TUNING_KNOBS build (tools/gpu_r2b.sh)
-    _lib.LIBRARY_PATH = os.environ['OKP_TUNING_LIBRARY']
+from object_keypoints_b200 import KeypointDecoder, synthetic
 
 shape = sys.argv[1] if len(sys.argv) > 1 else '180x320'
 frames = int(sys.argv[2]) if len(sys.argv) > 2 else 2048
@@ -43,7 +41,7 @@ ev[1].record()
 torch.cuda.synchronize()
 fused = ev[0].elapsed_time(ev[1]) / reps
 gb = frames * 3 * H * W * heat.element_size() / 1e9
-print(f"{shape} {dtype} frames={frames} env={ {k: v for k, v in os.environ.items() if k.startswith('OKP_')} } "
+print(f"{shape} {dtype} frames={frames} "
       f"K1 {k1 * 1e3:.1f} us = {gb / (k1 / 1e3):.0f} GB/s ({gb / (k1 / 1e3) / 6547.2:.3f} of measured HBM peak); group {k3 * 1e3:.1f} us; "
       f"decode_batch {' '.join(flags)} {fused * 1e3:.1f} us = {gb / (fused / 1e3) / 6547.2:.3f}; "
       f"objects/frame {float(tables['n_objects'].float().mean()):.2f}")
