@@ -50,7 +50,7 @@ enum {
 #define OKP_FLAG_NO_CENTERS 32u       /* empty centre map: frame has no objects (pipeline.py:105-106) */
 #define OKP_FLAG_ARGMAX_RESOLVED 64u  /* > cfg[t] detections, cfg[t] == 1: most confident kept (pipeline.py:139-142) */
 #define OKP_FLAG_GENERIC_PATH 128u    /* not a property of the data: this call's shape / mode is outside the tuned TMA kernel
-                                         (W % 4 != 0, W > 500, bfloat16 with W % 8 != 0, nms_size 3, box_sum 0) and ran
+                                         (W % 4 != 0, W > 500, 16-bit maps with W % 8 != 0, nms_size 3, box_sum 0) and ran
                                          on the exact generic tile kernels, about 3x slower per pixel -- same results */
 
 #define OKP_MAX_MAPS 16               /* C = 1 + number of keypoint types */
@@ -196,6 +196,23 @@ int okp_decode_bf16(const void* heat_dev, const void* depth_dev, const void* cen
                     const OkpDecodeTables* tables, void* workspace_dev, size_t workspace_bytes,
                     void* stream);
 
+/* float16 forms of the same entries, for heads that write float16 (torch.autocast on CUDA, model.half(), a half-precision
+ * TorchScript export). All three maps are float16 [same shapes as the _f32 forms]; every float16 value, subnormals
+ * included, is exactly a float32 value, and every sum, comparison and centroid is computed in float32 exactly as in the
+ * _f32 forms, so the tables equal those of the _f32 entry run on the up-cast maps bit for bit. The TMA path needs
+ * W % 8 == 0; other widths take the generic kernels. */
+int okp_extract_peaks_f16(const void* heat_dev, int N, int C, int H, int W,
+                          const OkpDecodeParams* params, const OkpDecodeTables* tables,
+                          void* workspace_dev, size_t workspace_bytes, void* stream);
+int okp_group_objects_f16(const void* depth_dev, const void* centers_dev, int N, int C, int H, int W,
+                          const int32_t* keypoint_config, const OkpCamera* camera,
+                          const OkpDecodeParams* params, const OkpDecodeTables* tables, void* stream);
+int okp_decode_f16(const void* heat_dev, const void* depth_dev, const void* centers_dev,
+                   int N, int C, int H, int W, const int32_t* keypoint_config,
+                   const OkpCamera* camera, const OkpDecodeParams* params,
+                   const OkpDecodeTables* tables, void* workspace_dev, size_t workspace_bytes,
+                   void* stream);
+
 /* okp_decode_* that also EMITS one compact record per frame -- what ObjectKeypointPipeline.__call__ returns per
  * frame (pipeline.py:195-199): object count, kept-keypoint counts, camera-frame 3D points -- into every sink buffer
  * while it decodes. This is the multi-GPU exchange of SURVEY section 8e (the reference is single-GPU, batch 1:
@@ -223,6 +240,11 @@ int okp_decode_emit_bf16(const void* heat_dev, const void* depth_dev, const void
                          const OkpCamera* camera, const OkpDecodeParams* params,
                          const OkpDecodeTables* tables, void* workspace_dev, size_t workspace_bytes,
                          const OkpRecordSink* sink, void* stream);
+int okp_decode_emit_f16(const void* heat_dev, const void* depth_dev, const void* centers_dev,
+                        int N, int C, int H, int W, const int32_t* keypoint_config,
+                        const OkpCamera* camera, const OkpDecodeParams* params,
+                        const OkpDecodeTables* tables, void* workspace_dev, size_t workspace_bytes,
+                        const OkpRecordSink* sink, void* stream);
 /* okp_group_objects_* with the record sink of okp_decode_emit_*: the second half of the two-launch decode for callers
  * that run the halves themselves (e.g. to put an event between them; ObjectExtraction + DetectionToPoint,
  * pipeline.py:104-171,189-199). sink may be NULL. */
@@ -234,6 +256,10 @@ int okp_group_objects_emit_bf16(const void* depth_dev, const void* centers_dev, 
                                 const int32_t* keypoint_config, const OkpCamera* camera,
                                 const OkpDecodeParams* params, const OkpDecodeTables* tables,
                                 const OkpRecordSink* sink, void* stream);
+int okp_group_objects_emit_f16(const void* depth_dev, const void* centers_dev, int N, int C, int H, int W,
+                               const int32_t* keypoint_config, const OkpCamera* camera,
+                               const OkpDecodeParams* params, const OkpDecodeTables* tables,
+                               const OkpRecordSink* sink, void* stream);
 
 /* Replaces FisheyeCamera.undistort (camera_utils.py:75-81, cv2.fisheye.undistortPoints with
  * P = K). xy_dev/out_dev: [n,2] float64. round_to_f32 != 0 reproduces OpenCV's float32 output

@@ -22,6 +22,7 @@ EXPORTS = [
     'okp_rasterise_targets_f32', 'okp_host_pack_scratch_bytes', 'okp_host_pack_tiles_f32', 'okp_scatter_tiles_f32',
     'okp_record_bytes', 'okp_decode_emit_f32', 'okp_decode_emit_bf16', 'okp_triangulate_tracks_f64', 'okp_associate_pairs_f64',
     'okp_group_objects_emit_f32', 'okp_group_objects_emit_bf16', 'okp_extract_peaks_events_f32',
+    'okp_extract_peaks_f16', 'okp_group_objects_f16', 'okp_decode_f16', 'okp_decode_emit_f16', 'okp_group_objects_emit_f16',
 ]
 
 
@@ -111,7 +112,7 @@ def lib():
     L.okp_decode_f32.restype = i32
     L.okp_decode_f32.argtypes = [vp, vp, vp, i32, i32, i32, i32, P(ctypes.c_int32), P(_abi.OkpCamera),
                                  P(_abi.OkpDecodeParams), P(_abi.OkpDecodeTables), vp, sz, vp]
-    for suffix in ('f32', 'bf16'):
+    for suffix in ('f32', 'bf16', 'f16'):
         extract, group, decode = (getattr(L, f'okp_{stem}_{suffix}') for stem in ('extract_peaks', 'group_objects', 'decode'))
         extract.restype = group.restype = decode.restype = i32
         extract.argtypes = L.okp_extract_peaks_f32.argtypes
@@ -119,7 +120,7 @@ def lib():
         decode.argtypes = L.okp_decode_f32.argtypes
     L.okp_record_bytes.restype = i32
     L.okp_record_bytes.argtypes = [i32, i32, P(ctypes.c_int32)]
-    for suffix in ('f32', 'bf16'):
+    for suffix in ('f32', 'bf16', 'f16'):
         emit = getattr(L, f'okp_decode_emit_{suffix}')
         emit.restype = i32
         emit.argtypes = L.okp_decode_f32.argtypes[:-1] + [P(_abi.OkpRecordSink), vp]

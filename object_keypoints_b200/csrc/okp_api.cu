@@ -107,7 +107,8 @@ const char* okp_strerror(int code) {
 size_t okp_decode_workspace_bytes(int N, int C, int H, int W, const OkpDecodeParams* params) {
     if (check_params(params) != OKP_OK || check_shape(N, C, H, W) != OKP_OK) return 0;
     if (N == 0) return 256;
-    // enough for either element type (their launch plans can differ: bf16 rows need W % 8 == 0 for TMA)
+    // enough for every element type (their launch plans can differ: 16-bit rows need W % 8 == 0 for TMA; bf16 and f16
+    // share one plan)
     size_t need = 0;
     for (int esize = 2; esize <= 4; esize += 2) {
         const PeakPlan p = plan_peaks(N * C, C, H, W, params->max_peaks, esize, params);
@@ -362,6 +363,11 @@ int okp_extract_peaks_bf16(const void* heat_dev, int N, int C, int H, int W, con
                                         workspace_bytes, stream);
 }
 
+int okp_extract_peaks_f16(const void* heat_dev, int N, int C, int H, int W, const OkpDecodeParams* params,
+                          const OkpDecodeTables* tables, void* workspace_dev, size_t workspace_bytes, void* stream) {
+    return extract_peaks<__half>((const __half*)heat_dev, N, C, H, W, params, tables, workspace_dev, workspace_bytes, stream);
+}
+
 int okp_group_objects_f32(const float* depth_dev, const float* centers_dev, int N, int C, int H, int W,
                           const int32_t* keypoint_config, const OkpCamera* camera, const OkpDecodeParams* params,
                           const OkpDecodeTables* tables, void* stream) {
@@ -373,6 +379,13 @@ int okp_group_objects_bf16(const void* depth_dev, const void* centers_dev, int N
                            const OkpDecodeTables* tables, void* stream) {
     return group_objects<__nv_bfloat16>((const __nv_bfloat16*)depth_dev, (const __nv_bfloat16*)centers_dev, N, C, H, W,
                                         keypoint_config, camera, params, tables, nullptr, stream);
+}
+
+int okp_group_objects_f16(const void* depth_dev, const void* centers_dev, int N, int C, int H, int W,
+                          const int32_t* keypoint_config, const OkpCamera* camera, const OkpDecodeParams* params,
+                          const OkpDecodeTables* tables, void* stream) {
+    return group_objects<__half>((const __half*)depth_dev, (const __half*)centers_dev, N, C, H, W, keypoint_config, camera,
+                                 params, tables, nullptr, stream);
 }
 
 int okp_host_alias(const void* host_ptr, void** dev_ptr_out) {
@@ -401,6 +414,13 @@ int okp_decode_bf16(const void* heat_dev, const void* depth_dev, const void* cen
                                  N, C, H, W, keypoint_config, camera, params, tables, workspace_dev, workspace_bytes, nullptr, stream);
 }
 
+int okp_decode_f16(const void* heat_dev, const void* depth_dev, const void* centers_dev, int N, int C, int H, int W,
+                   const int32_t* keypoint_config, const OkpCamera* camera, const OkpDecodeParams* params,
+                   const OkpDecodeTables* tables, void* workspace_dev, size_t workspace_bytes, void* stream) {
+    return decode<__half>((const __half*)heat_dev, (const __half*)depth_dev, (const __half*)centers_dev, N, C, H, W,
+                          keypoint_config, camera, params, tables, workspace_dev, workspace_bytes, nullptr, stream);
+}
+
 int okp_record_bytes(int O, int C, const int32_t* keypoint_config) {
     if (O < 1 || O > OKP_MAX_OBJECTS || C < 1 || C > OKP_MAX_MAPS || (C > 1 && !keypoint_config)) return 0;
     int P = 1;
@@ -427,6 +447,14 @@ int okp_decode_emit_bf16(const void* heat_dev, const void* depth_dev, const void
                                  N, C, H, W, keypoint_config, camera, params, tables, workspace_dev, workspace_bytes, sink, stream);
 }
 
+int okp_decode_emit_f16(const void* heat_dev, const void* depth_dev, const void* centers_dev, int N, int C, int H, int W,
+                        const int32_t* keypoint_config, const OkpCamera* camera, const OkpDecodeParams* params,
+                        const OkpDecodeTables* tables, void* workspace_dev, size_t workspace_bytes,
+                        const OkpRecordSink* sink, void* stream) {
+    return decode<__half>((const __half*)heat_dev, (const __half*)depth_dev, (const __half*)centers_dev, N, C, H, W,
+                          keypoint_config, camera, params, tables, workspace_dev, workspace_bytes, sink, stream);
+}
+
 int okp_group_objects_emit_f32(const float* depth_dev, const float* centers_dev, int N, int C, int H, int W,
                                const int32_t* keypoint_config, const OkpCamera* camera, const OkpDecodeParams* params,
                                const OkpDecodeTables* tables, const OkpRecordSink* sink, void* stream) {
@@ -438,6 +466,13 @@ int okp_group_objects_emit_bf16(const void* depth_dev, const void* centers_dev, 
                                 const OkpDecodeTables* tables, const OkpRecordSink* sink, void* stream) {
     return group_objects<__nv_bfloat16>((const __nv_bfloat16*)depth_dev, (const __nv_bfloat16*)centers_dev, N, C, H, W,
                                         keypoint_config, camera, params, tables, sink, stream);
+}
+
+int okp_group_objects_emit_f16(const void* depth_dev, const void* centers_dev, int N, int C, int H, int W,
+                               const int32_t* keypoint_config, const OkpCamera* camera, const OkpDecodeParams* params,
+                               const OkpDecodeTables* tables, const OkpRecordSink* sink, void* stream) {
+    return group_objects<__half>((const __half*)depth_dev, (const __half*)centers_dev, N, C, H, W, keypoint_config, camera,
+                                 params, tables, sink, stream);
 }
 
 int okp_fisheye_undistort_f64(const double* xy_dev, int n, const OkpCamera* camera, int round_to_f32,

@@ -5,6 +5,7 @@
 // separately, exactly like the reference's NumPy / torch-CPU arithmetic.
 #pragma once
 #include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <math.h>
 #include <stdint.h>
@@ -34,13 +35,16 @@ __device__ __forceinline__ int okp_max(int a, int b) { return a > b ? a : b; }
 __device__ __forceinline__ int okp_clamp(int v, int lo, int hi) { return v < lo ? lo : (v > hi ? hi : v); }
 
 // Map element types. float32 is the reference's type; bfloat16 is what a bf16 network head writes
-// (BASELINE config 5). bf16 -> f32 is exact, so every kernel computes on the very float32 values the
-// oracle sees when it is handed the up-cast map: the parity contract does not change with the type.
+// (BASELINE config 5); float16 is what torch.autocast on CUDA, model.half() or a half-precision TorchScript
+// export writes. bf16 -> f32 and f16 -> f32 are exact (every float16, subnormals included, is a float32
+// value), so every kernel computes on the very float32 values the oracle sees when it is handed the up-cast
+// map: the parity contract does not change with the type.
 template <typename T> __device__ __forceinline__ float okp_ld(const T* p);
 template <> __device__ __forceinline__ float okp_ld<float>(const float* p) { return __ldg(p); }
 template <> __device__ __forceinline__ float okp_ld<__nv_bfloat16>(const __nv_bfloat16* p) {
     return __uint_as_float((uint32_t)__ldg(reinterpret_cast<const unsigned short*>(p)) << 16);
 }
+template <> __device__ __forceinline__ float okp_ld<__half>(const __half* p) { return __half2float(__ldg(p)); }
 
 // Programmatic dependent launch (sm_90+): a kernel launched with okp_launch_dependent() may be scheduled while the kernel
 // in front of it on the stream drains -- its launch latency (2-4 us between dependent kernels on a B200) overlaps the

@@ -418,7 +418,7 @@ okp_peaks_stream_kernel(const __grid_constant__ CUtensorMap tmap, const T* __res
     }
 }
 
-// The stream kernel's plan for `maps` maps of H x W elements of esize bytes (4: float32, 2: bfloat16), K table rows per map,
+// The stream kernel's plan for `maps` maps of H x W elements of esize bytes (4: float32, 2: bfloat16 or float16), K table rows per map,
 // C maps per frame; false when the kernel does not cover the shape (the caller runs the generic kernels). group_frame_bytes
 // > 0 asks for the fused form: groups of whole frames plus one grouping scratch (group_frame_bytes each) per frame of a
 // group; false when not even one frame fits a group (the caller then runs the peak kernel and okp_group_kernel separately).
@@ -506,6 +506,11 @@ static inline bool okp_stream_plan(int maps, int C, int H, int W, int K, int esi
     return true;
 }
 
+template <typename T> static inline CUtensorMapDataType okp_tensor_map_type();
+template <> inline CUtensorMapDataType okp_tensor_map_type<float>() { return CU_TENSOR_MAP_DATA_TYPE_FLOAT32; }
+template <> inline CUtensorMapDataType okp_tensor_map_type<__nv_bfloat16>() { return CU_TENSOR_MAP_DATA_TYPE_BFLOAT16; }
+template <> inline CUtensorMapDataType okp_tensor_map_type<__half>() { return CU_TENSOR_MAP_DATA_TYPE_FLOAT16; }
+
 // ga: grouping arguments (fused form, sp.F > 0) or NULL (peaks only).
 template <typename T>
 static inline int okp_stream_launch(const T* heat, const OkpStreamPlan& sp, float threshold,
@@ -520,7 +525,7 @@ static inline int okp_stream_launch(const T* heat, const OkpStreamPlan& sp, floa
     const cuuint64_t strides[2] = {(cuuint64_t)p.W * sizeof(T), (cuuint64_t)p.W * p.H * sizeof(T)};
     const cuuint32_t box[3] = {(cuuint32_t)p.BW, (cuuint32_t)OKP_STRIP_RB, (cuuint32_t)p.M};
     const cuuint32_t elem[3] = {1, 1, 1};
-    const CUtensorMapDataType dtype = sizeof(T) == 4 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
+    const CUtensorMapDataType dtype = okp_tensor_map_type<T>();
     const CUresult r = encode(&tmap, dtype, 3, (void*)heat, dims, strides, box, elem, CU_TENSOR_MAP_INTERLEAVE_NONE,
                               CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (r != CUDA_SUCCESS) return OKP_E_CUDA;

@@ -57,9 +57,9 @@ struct OkpStripPlan {
     int half_strips;              // strips served by TMA box 0 (all of them when halves == 1)
     int halves;                   // 1 or 2 TMA boxes per row (box width <= 256 elements)
     int BW;                       // box width in elements
-    int esize;                    // bytes per map element: 4 (float32) or 2 (bfloat16)
+    int esize;                    // bytes per map element: 4 (float32) or 2 (bfloat16, float16)
     int lead[2];                  // elements between a box's first column and its first strip's column 4s-4
-                                  // (the box start must be 16-byte aligned: 0 for float32, 0 or 4 for bfloat16)
+                                  // (the box start must be 16-byte aligned: 0 for float32, 0 or 4 for 16-bit maps)
     int M;                        // maps per CTA
     int NS;                       // TMA stages
     int nb;                       // batches
@@ -262,6 +262,14 @@ template <> __device__ __forceinline__ void okp_strip_window<__nv_bfloat16>(cons
     lo.z = __uint_as_float(a.y << 16); lo.w = __uint_as_float(a.y & 0xFFFF0000u);
     hi.x = __uint_as_float(b.x << 16); hi.y = __uint_as_float(b.x & 0xFFFF0000u);
     hi.z = __uint_as_float(b.y << 16); hi.w = __uint_as_float(b.y & 0xFFFF0000u);
+}
+// float16 maps: the same two LDS.64; each __half22float2 is two HADD2.F32 (exact, subnormals included).
+template <> __device__ __forceinline__ void okp_strip_window<__half>(const unsigned char* row, float4& lo, float4& hi) {
+    const uint2 a = reinterpret_cast<const uint2*>(row)[0], b = reinterpret_cast<const uint2*>(row)[1];
+    const float2 a0 = __half22float2(*reinterpret_cast<const __half2*>(&a.x)), a1 = __half22float2(*reinterpret_cast<const __half2*>(&a.y));
+    const float2 b0 = __half22float2(*reinterpret_cast<const __half2*>(&b.x)), b1 = __half22float2(*reinterpret_cast<const __half2*>(&b.y));
+    lo = make_float4(a0.x, a0.y, a1.x, a1.y);
+    hi = make_float4(b0.x, b0.y, b1.x, b1.y);
 }
 
 // One batch of RB rows: the five unrolled steps, rows fetched one step ahead of their use (two register

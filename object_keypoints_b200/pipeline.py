@@ -67,13 +67,18 @@ def _aligned(x):
     return x.clone() if x.data_ptr() % 16 else x
 
 
+# element type of a map -> suffix of the okp_* entries that read it in place
+_MAP_KINDS = {torch.float32: 'f32', torch.bfloat16: 'bf16', torch.float16: 'f16'}
+
+
 def _as_device_map(x, device):
-    """Like _as_device_f32, but a bfloat16 tensor (a bf16 network head's output) stays bfloat16:
-    the okp_*_bf16 entries read it in place. -> (tensor, 'f32' | 'bf16')."""
-    if isinstance(x, torch.Tensor) and x.dtype == torch.bfloat16:
+    """Like _as_device_f32, but a bfloat16 or float16 tensor (the output of a bf16 or half-precision network head)
+    keeps its type: the okp_*_bf16 / okp_*_f16 entries read it in place, on the device or after a copy of the 16-bit
+    bytes from the host. -> (tensor, 'f32' | 'bf16' | 'f16')."""
+    if isinstance(x, torch.Tensor) and x.dtype in (torch.bfloat16, torch.float16):
         if x.device != device:
             x = x.to(device, non_blocking=True)
-        return _aligned(x.contiguous()), 'bf16'
+        return _aligned(x.contiguous()), _MAP_KINDS[x.dtype]
     return _as_device_f32(x, device), 'f32'
 
 
@@ -173,8 +178,10 @@ class KeypointDecoder:
         return int(self._lib.okp_record_bytes(self.params.max_objects, self.C, self._cfg_array))
 
     def decode_batch(self, heat, depth, centers, tables=None, stream=None, records=None, peaks_done=None):
-        """heat [N,C,H,W], depth [N,C,H,W], centers [N,C-1,2,H,W] (float32 or bfloat16; CUDA tensors
-        are used in place, host arrays are copied) -> DecodeTables on the device. No synchronisation.
+        """heat [N,C,H,W], depth [N,C,H,W], centers [N,C-1,2,H,W] (float32, bfloat16 or float16; CUDA tensors
+        are used in place, host arrays are copied, 16-bit tensors keep their type) -> DecodeTables on the device. No
+        synchronisation. Heatmaps of one type with depth / centre maps of another take two C calls (peaks, then
+        grouping); depth and centre maps of different types are both up-cast to float32.
         records: an ``_abi.OkpRecordSink`` (sharding.RecordExchange.begin()): the kernel also writes every frame's
         compact record into the sink's buffers while it decodes (the multi-GPU gather).
         peaks_done: a ``torch.cuda.Event`` recorded between the peak kernel (+ its overflow fix-up) and the grouping
@@ -201,7 +208,7 @@ class KeypointDecoder:
                 ctypes.byref(self.params), ctypes.byref(tables.struct), ws.data_ptr(), ws.numel(),
                 ctypes.byref(records) if records is not None else None, _stream_handle(stream))
             _lib.check(rc, f'okp_decode_emit_{heat_kind}')
-        else:                                                # e.g. bf16 heatmaps with float32 depth / centre maps
+        else:                                                # e.g. 16-bit heatmaps with float32 depth / centre maps
             pair = peaks_done if isinstance(peaks_done, (tuple, list)) else None
             if pair is not None and heat_kind == 'f32':
                 for event in pair:
@@ -230,7 +237,8 @@ class KeypointDecoder:
 
     def _host_alias(self, tensor):
         """Device-side address of a pinned CPU tensor (okp_host_alias), or None if it has to be copied."""
-        if tensor.device.type != 'cpu' or tensor.dtype != torch.float32 or not tensor.is_contiguous() or not tensor.is_pinned():
+        if (tensor.device.type != 'cpu' or tensor.dtype not in _MAP_KINDS or not tensor.is_contiguous() or
+                not tensor.is_pinned()):
             return None
         alias = ctypes.c_void_p()
         if self._lib.okp_host_alias(ctypes.c_void_p(tensor.data_ptr()), ctypes.byref(alias)) != 0 or not alias.value:
@@ -261,10 +269,14 @@ class KeypointDecoder:
 
     def _check_host_inputs(self, heat, depth, centers):
         """Shapes / dtypes of decode_host_batch's inputs: the host pass and the in-place gathers work on raw pointers, so a
-        wrong shape would be an out-of-bounds read, not an exception."""
+        wrong shape or element type would be an out-of-bounds read, not an exception. All three maps share one dtype:
+        float32, bfloat16 or float16."""
         for name, tensor in (('heat', heat), ('depth', depth), ('centers', centers)):
-            if not isinstance(tensor, torch.Tensor) or tensor.device.type != 'cpu' or tensor.dtype != torch.float32:
-                raise ValueError(f"{name} must be a float32 CPU tensor")
+            if not isinstance(tensor, torch.Tensor) or tensor.device.type != 'cpu' or tensor.dtype not in _MAP_KINDS:
+                raise ValueError(f"{name} must be a float32, bfloat16 or float16 CPU tensor")
+        if not heat.dtype == depth.dtype == centers.dtype:
+            raise ValueError(f"heat, depth and centers must share one dtype, got {heat.dtype}, {depth.dtype} and "
+                             f"{centers.dtype}")
         self._check(heat)
         N = int(heat.shape[0])
         if tuple(depth.shape) != tuple(heat.shape):
@@ -281,7 +293,9 @@ class KeypointDecoder:
     def decode_host_batch(self, heat, depth, centers, chunk_frames=128, sparse='auto', out=None):
         """End-to-end form for HOST inputs, the shape the reference's caller has (CPU tensors out of
         InferenceComponent, pipeline.py:24-28). The batch is cut into chunks that are pipelined: while chunk i is
-        decoded, chunk i+1 crosses PCIe and chunk i+2 is prepared on the host.
+        decoded, chunk i+1 crosses PCIe and chunk i+2 is prepared on the host. The three maps are float32, bfloat16
+        or float16 CPU tensors of one dtype; 16-bit maps cross the bus as they are (half the bytes of float32) and are
+        decoded by the okp_*_bf16 / okp_*_f16 entries.
 
         Heatmaps: with ``sparse='auto'`` a host pass (okp_host_pack_tiles_f32, OpenMP + AVX2, in a worker thread)
         marks the 4x16-pixel tiles within reach of a value above threshold / 25 and only those cross the bus; the
@@ -293,7 +307,8 @@ class KeypointDecoder:
         (dense maps) is copied densely too; ``sparse=False`` disables the host pass, ``sparse='only'`` the side-by-side
         dense copies. Depth and centre maps are only gathered from (3 values per spoke peak): when they live in
         pinned host memory the kernels read them in place over PCIe; pageable tensors are copied like dense
-        heatmaps. The object tables of every chunk are copied back into pinned host tensors.
+        heatmaps. The host pass is float32-only: 16-bit heatmaps always take the dense copy. The object tables of
+        every chunk are copied back into pinned host tensors.
         Returns a dict of CPU tensors (synchronised): freshly allocated for every call, or ``out`` (a dict from an earlier
         call or from ``host_result``) filled in place."""
         self._check_host_inputs(heat, depth, centers)
@@ -304,20 +319,21 @@ class KeypointDecoder:
         centers_alias = self._host_alias(centers)
         in_place = depth_alias is not None and centers_alias is not None
         use_sparse = self._sparse_ok(heat, sparse)
-        key = ('host', chunk, in_place, use_sparse)
+        dtype, kind = heat.dtype, _MAP_KINDS[heat.dtype]
+        key = ('host', chunk, in_place, use_sparse, dtype)
         tiles_per_map = ((self.H + 3) // 4) * ((self.W + 15) // 16)
         capacity = max(1, int(self.SPARSE_CAPACITY * chunk * self.C * tiles_per_map))
         if key not in self._tables:
             staging = []
             for slot_index in range(5 if use_sparse else 2):       # sparse: three packing slots, two dense-copy slots
                 slot = {
-                    'heat': torch.empty((chunk, self.C, self.H, self.W), dtype=torch.float32, device=self.device),
+                    'heat': torch.empty((chunk, self.C, self.H, self.W), dtype=dtype, device=self.device),
                     'tables': DecodeTables(chunk, self.C, self.cfg, self.params, self.device),
                     'ready': torch.cuda.Event(), 'done': torch.cuda.Event(), 'copied': torch.cuda.Event(),
                 }
                 if not in_place:
-                    slot['depth'] = torch.empty((chunk, self.C, self.H, self.W), dtype=torch.float32, device=self.device)
-                    slot['centers'] = torch.empty((chunk, self.C - 1, 2, self.H, self.W), dtype=torch.float32, device=self.device)
+                    slot['depth'] = torch.empty((chunk, self.C, self.H, self.W), dtype=dtype, device=self.device)
+                    slot['centers'] = torch.empty((chunk, self.C - 1, 2, self.H, self.W), dtype=dtype, device=self.device)
                 if use_sparse and slot_index < 3:
                     maps = chunk * self.C
                     slot['packed_host'] = torch.empty((capacity, 64), dtype=torch.float32).pin_memory()
@@ -343,8 +359,8 @@ class KeypointDecoder:
                     raise ValueError(f"out['{name}'] must be a pinned CPU tensor with {N} rows (see host_result)")
         compute = torch.cuda.current_stream()
         self._workspace_for(chunk)
-        depth_frame = self.C * self.H * self.W * 4
-        centers_frame = (self.C - 1) * 2 * self.H * self.W * 4
+        depth_frame = self.C * self.H * self.W * heat.element_size()            # bytes of one frame's heat or depth maps
+        centers_frame = (self.C - 1) * 2 * self.H * self.W * heat.element_size()
         cam = ctypes.byref(self._camera) if self._camera is not None else None
         self.host_bytes_copied = 0
         self.host_chunks_sparse = 0
@@ -401,11 +417,11 @@ class KeypointDecoder:
             tables = slot['tables'] if n == chunk else self.tables(n)
             if in_place:
                 ws = self._workspace_for(n)
-                rc = self._lib.okp_decode_f32(slot['heat'].data_ptr(), depth_alias + f0 * depth_frame,
-                                              centers_alias + f0 * centers_frame, n, self.C, self.H, self.W,
-                                              self._cfg_array, cam, ctypes.byref(self.params), ctypes.byref(tables.struct),
-                                              ws.data_ptr(), ws.numel(), _stream_handle(compute))
-                _lib.check(rc, 'okp_decode_f32')
+                rc = getattr(self._lib, f'okp_decode_{kind}')(
+                    slot['heat'].data_ptr(), depth_alias + f0 * depth_frame, centers_alias + f0 * centers_frame, n, self.C,
+                    self.H, self.W, self._cfg_array, cam, ctypes.byref(self.params), ctypes.byref(tables.struct),
+                    ws.data_ptr(), ws.numel(), _stream_handle(compute))
+                _lib.check(rc, f'okp_decode_{kind}')
             else:
                 self.decode_batch(slot['heat'][:n], slot['depth'][:n], slot['centers'][:n], tables=tables)
             for name in self.HOST_RESULT_TABLES:
