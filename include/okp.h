@@ -261,6 +261,41 @@ int okp_group_objects_emit_f16(const void* depth_dev, const void* centers_dev, i
                                const OkpDecodeParams* params, const OkpDecodeTables* tables,
                                const OkpRecordSink* sink, void* stream);
 
+/* Per-frame cameras: okp_decode_emit_* / okp_group_objects_emit_* for a batch whose frames come from more than one camera
+ * (the two views of a stereo rig, sequences with different calibrations or different crops). Frame n is undistorted,
+ * clipped (clip_x / clip_y) and unprojected with cameras_dev[n]; everything else is the single-camera entry's
+ * arithmetic, so the rows of frame n equal that entry's rows for the same frame run with camera = &cameras_dev[n].
+ * cameras_dev: DEVICE array [N] of OkpCamera (144 bytes each), 16-byte aligned, read by the grouping kernel (one load
+ * per frame). It is a device pointer because a caller reuses one table for every batch of the same layout; the indices
+ * behind it are the caller's to check. sink may be NULL. N = 0 returns OKP_OK, as for every entry. With N > 0, refused on
+ * the host, before any CUDA call: NULL cameras_dev or NULL depth_dev (OKP_E_NULL), cameras_dev not 16-byte aligned or
+ * OkpDecodeParams.single_pass set (OKP_E_UNSUPPORTED: only the two-launch form has a per-frame camera). */
+int okp_decode_cameras_f32(const float* heat_dev, const float* depth_dev, const float* centers_dev,
+                           int N, int C, int H, int W, const int32_t* keypoint_config,
+                           const OkpCamera* cameras_dev /* DEVICE [N]: frame n is lifted with cameras_dev[n] */,
+                           const OkpDecodeParams* params, const OkpDecodeTables* tables, void* workspace_dev,
+                           size_t workspace_bytes, const OkpRecordSink* sink, void* stream);
+int okp_decode_cameras_bf16(const void* heat_dev, const void* depth_dev, const void* centers_dev,
+                            int N, int C, int H, int W, const int32_t* keypoint_config, const OkpCamera* cameras_dev,
+                            const OkpDecodeParams* params, const OkpDecodeTables* tables, void* workspace_dev,
+                            size_t workspace_bytes, const OkpRecordSink* sink, void* stream);
+int okp_decode_cameras_f16(const void* heat_dev, const void* depth_dev, const void* centers_dev,
+                           int N, int C, int H, int W, const int32_t* keypoint_config, const OkpCamera* cameras_dev,
+                           const OkpDecodeParams* params, const OkpDecodeTables* tables, void* workspace_dev,
+                           size_t workspace_bytes, const OkpRecordSink* sink, void* stream);
+int okp_group_objects_cameras_f32(const float* depth_dev, const float* centers_dev, int N, int C, int H, int W,
+                                  const int32_t* keypoint_config, const OkpCamera* cameras_dev,
+                                  const OkpDecodeParams* params, const OkpDecodeTables* tables,
+                                  const OkpRecordSink* sink, void* stream);
+int okp_group_objects_cameras_bf16(const void* depth_dev, const void* centers_dev, int N, int C, int H, int W,
+                                   const int32_t* keypoint_config, const OkpCamera* cameras_dev,
+                                   const OkpDecodeParams* params, const OkpDecodeTables* tables,
+                                   const OkpRecordSink* sink, void* stream);
+int okp_group_objects_cameras_f16(const void* depth_dev, const void* centers_dev, int N, int C, int H, int W,
+                                  const int32_t* keypoint_config, const OkpCamera* cameras_dev,
+                                  const OkpDecodeParams* params, const OkpDecodeTables* tables,
+                                  const OkpRecordSink* sink, void* stream);
+
 /* Replaces FisheyeCamera.undistort (camera_utils.py:75-81, cv2.fisheye.undistortPoints with
  * P = K). xy_dev/out_dev: [n,2] float64. round_to_f32 != 0 reproduces OpenCV's float32 output
  * for float32 input (the value is rounded to float32, stored as float64). */

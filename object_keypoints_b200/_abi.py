@@ -117,6 +117,25 @@ def pack_camera(camera):
     return out
 
 
+def pack_camera_table(cameras, camera_index):
+    """Per-frame camera table of okp_decode_cameras_* / okp_group_objects_cameras_*: a short sequence of camera objects
+    (as pack_camera takes them) and camera_index [N], the camera of every frame -> ctypes array of N OkpCamera whose row n
+    is pack_camera(cameras[camera_index[n]]). The library reads the rows as they are, so every index is checked here:
+    ValueError for an index that is not an integer, negative or out of range, or an index array that is not 1-D."""
+    index = np.asarray(camera_index)
+    if index.ndim != 1:
+        raise ValueError(f"camera_index must be one index per frame (1-D), got shape {index.shape}")
+    if index.size and index.dtype.kind not in 'iu':
+        raise ValueError(f"camera_index must hold integers, got {index.dtype}")
+    packed = [pack_camera(camera) for camera in cameras]
+    if index.size and (index.min() < 0 or index.max() >= len(packed)):
+        raise ValueError(f"camera_index out of range: values in [{index.min()}, {index.max()}] for {len(packed)} cameras")
+    table = (OkpCamera * index.size)()
+    for n, c in enumerate(index.tolist()):
+        table[n] = packed[c]
+    return table
+
+
 def check_keypoint_config(keypoint_config):
     """Accepts the parsed JSON dict {'keypoint_config': [...]} (what the reference passes,
     pipeline.py:36,95) or the bare list; returns the list of ints."""

@@ -23,6 +23,8 @@ EXPORTS = [
     'okp_record_bytes', 'okp_decode_emit_f32', 'okp_decode_emit_bf16', 'okp_triangulate_tracks_f64', 'okp_associate_pairs_f64',
     'okp_group_objects_emit_f32', 'okp_group_objects_emit_bf16', 'okp_extract_peaks_events_f32',
     'okp_extract_peaks_f16', 'okp_group_objects_f16', 'okp_decode_f16', 'okp_decode_emit_f16', 'okp_group_objects_emit_f16',
+    'okp_decode_cameras_f32', 'okp_decode_cameras_bf16', 'okp_decode_cameras_f16',
+    'okp_group_objects_cameras_f32', 'okp_group_objects_cameras_bf16', 'okp_group_objects_cameras_f16',
 ]
 
 
@@ -127,6 +129,13 @@ def lib():
         group_emit = getattr(L, f'okp_group_objects_emit_{suffix}')
         group_emit.restype = i32
         group_emit.argtypes = L.okp_group_objects_f32.argtypes[:-1] + [P(_abi.OkpRecordSink), vp]
+        # the _cameras forms: the emit entries with a DEVICE camera table [N] in place of the host camera
+        cameras = getattr(L, f'okp_decode_cameras_{suffix}')
+        cameras.restype = i32
+        cameras.argtypes = emit.argtypes[:8] + [vp] + emit.argtypes[9:]
+        group_cameras = getattr(L, f'okp_group_objects_cameras_{suffix}')
+        group_cameras.restype = i32
+        group_cameras.argtypes = group_emit.argtypes[:7] + [vp] + group_emit.argtypes[8:]
     L.okp_host_alias.restype = i32
     L.okp_host_alias.argtypes = [vp, P(vp)]
     L.okp_fisheye_undistort_f64.restype = i32

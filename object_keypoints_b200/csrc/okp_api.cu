@@ -230,11 +230,12 @@ int convert_sink(const OkpRecordSink* sink, int O, int C, int P, OkpRecordSinks*
 }
 
 // Checks and packs what the grouping needs (okp_group.cuh); *warps = frames per CTA of the stand-alone kernel.
+// cameras_dev != NULL: the per-frame-camera form (okp_group_cameras_kernel), whose scratch also holds the frame's camera.
 int make_group_args(const void* depth_dev, const void* centers_dev, int N, int C, int H, int W,
-                    const int32_t* keypoint_config, const OkpCamera* camera, const OkpDecodeParams* params,
-                    const OkpDecodeTables* tables, const OkpRecordSink* sink, OkpGroupArgs* a) {
+                    const int32_t* keypoint_config, const OkpCamera* camera, const OkpCamera* cameras_dev,
+                    const OkpDecodeParams* params, const OkpDecodeTables* tables, const OkpRecordSink* sink, OkpGroupArgs* a) {
     if (!tables || (C > 1 && (!centers_dev || !keypoint_config))) return OKP_E_NULL;
-    if (camera && !depth_dev) return OKP_E_NULL;
+    if ((camera || cameras_dev) && !depth_dev) return OKP_E_NULL;
     const void* const* fields = (const void* const*)tables;
     for (size_t i = 0; i < sizeof(OkpDecodeTables) / sizeof(void*); ++i)
         if (!fields[i]) return OKP_E_NULL;
@@ -255,56 +256,77 @@ int make_group_args(const void* depth_dev, const void* centers_dev, int N, int C
     a->prm = *params;
     a->depth = depth_dev; a->centers = centers_dev;
     a->N = N; a->C = C; a->H = H; a->W = W; a->S = S; a->P = P;
-    a->have_camera = camera != nullptr;
+    a->have_camera = camera != nullptr || cameras_dev != nullptr;
     const int K = params->max_peaks, O = params->max_objects;
-    const size_t per_frame = okp_group_smem_bytes(C, K, O);
+    const size_t per_frame = okp_group_smem_bytes(C, K, O, cameras_dev != nullptr);
     if (per_frame > 200 * 1024) return OKP_E_CAPACITY;
     a->frame_smem_bytes = (int)per_frame;
     return convert_sink(sink, O, C, P, &a->sinks);
 }
 
 template <typename T, int LANES>
-int launch_group_lanes(const OkpGroupArgs& a, int only_pending, const OkpDecodeTables* tables, cudaStream_t s) {
+int launch_group_lanes(const OkpGroupArgs& a, int only_pending, const OkpDecodeTables* tables, const OkpCamera* cameras_dev,
+                       cudaStream_t s) {
     const int most = 128 / LANES;                                          // frames per CTA: LANES lanes each
     int frames = (int)((size_t)(48 * 1024) / a.frame_smem_bytes);
     if (frames > most) frames = most;
     if (LANES == 16) frames &= ~1;                                         // whole warps (the caller checked that two frames fit)
     if (frames < 1) frames = 1;
     const size_t smem = (size_t)a.frame_smem_bytes * frames;
+    const dim3 grid((a.N + frames - 1) / frames), block(frames * LANES);
+    if (cameras_dev) {
+        auto kernel = okp_group_cameras_kernel<T, LANES>;
+        if (smem > 48 * 1024) OKP_CUDA_CHECK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        OKP_CUDA_CHECK(okp_launch_dependent(kernel, grid, block, smem, s, a, *tables, cameras_dev));
+        return OKP_OK;
+    }
     auto kernel = okp_group_kernel<T, LANES>;
     if (smem > 48 * 1024) OKP_CUDA_CHECK(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    const int threads = frames * LANES;
-    OKP_CUDA_CHECK(okp_launch_dependent(kernel, dim3((a.N + frames - 1) / frames), dim3(threads), smem, s, a, only_pending, *tables));
+    OKP_CUDA_CHECK(okp_launch_dependent(kernel, grid, block, smem, s, a, only_pending, *tables));
     return OKP_OK;
 }
 
 // Small frames hold few peaks (a 64x64 valve frame: ~10): half a warp per frame, two frames per warp (okp_group.cuh).
 template <typename T>
-int launch_group(const OkpGroupArgs& a, int only_pending, const OkpDecodeTables* tables, cudaStream_t s) {
+int launch_group(const OkpGroupArgs& a, int only_pending, const OkpDecodeTables* tables, const OkpCamera* cameras_dev,
+                 cudaStream_t s) {
     const bool small = (long long)a.H * a.W <= 96LL * 96LL && 2 * (size_t)a.frame_smem_bytes <= 48 * 1024;
-    return small ? launch_group_lanes<T, 16>(a, only_pending, tables, s) : launch_group_lanes<T, 32>(a, only_pending, tables, s);
+    return small ? launch_group_lanes<T, 16>(a, only_pending, tables, cameras_dev, s)
+                 : launch_group_lanes<T, 32>(a, only_pending, tables, cameras_dev, s);
 }
 
+// What the okp_*_cameras_* entries refuse on top of the checks of their single-camera twins. N <= 0 is left to those
+// checks: like every entry, a call with no frames returns OKP_OK (an empty table may be NULL) and N < 0 is OKP_E_SHAPE.
+int check_cameras(int N, const void* depth_dev, const OkpCamera* cameras_dev, const OkpDecodeParams* params) {
+    if (N <= 0) return OKP_OK;
+    if (!params || !cameras_dev || !depth_dev) return OKP_E_NULL;
+    if ((uintptr_t)cameras_dev & 15u) return OKP_E_UNSUPPORTED;       // each lane copies one 16-byte word of the camera
+    if (params->single_pass) return OKP_E_UNSUPPORTED;                // the fused single pass has no per-frame-camera form
+    return OKP_OK;
+}
+
+// cameras_dev: NULL for the single-camera entries (camera, which may be NULL too, is the call's camera), else the
+// per-frame camera table of okp_group_objects_cameras_* (camera NULL).
 template <typename T>
 int group_objects(const T* depth_dev, const T* centers_dev, int N, int C, int H, int W,
-                  const int32_t* keypoint_config, const OkpCamera* camera, const OkpDecodeParams* params,
-                  const OkpDecodeTables* tables, const OkpRecordSink* sink, void* stream) {
+                  const int32_t* keypoint_config, const OkpCamera* camera, const OkpCamera* cameras_dev,
+                  const OkpDecodeParams* params, const OkpDecodeTables* tables, const OkpRecordSink* sink, void* stream) {
     int rc = check_params(params);
     if (rc != OKP_OK) return rc;
     rc = check_shape(N, C, H, W);
     if (rc != OKP_OK) return rc;
     if (N == 0) return OKP_OK;
     OkpGroupArgs a;
-    rc = make_group_args(depth_dev, centers_dev, N, C, H, W, keypoint_config, camera, params, tables, sink, &a);
+    rc = make_group_args(depth_dev, centers_dev, N, C, H, W, keypoint_config, camera, cameras_dev, params, tables, sink, &a);
     if (rc != OKP_OK) return rc;
-    return launch_group<T>(a, 0, tables, (cudaStream_t)stream);
+    return launch_group<T>(a, 0, tables, cameras_dev, (cudaStream_t)stream);
 }
 
 // ObjectKeypointPipeline.__call__ for a batch (perception/pipeline.py:182-200): the fused streaming pass where the
 // shape and the mode allow it, else peak extraction followed by grouping.
 template <typename T>
 int decode(const T* heat_dev, const T* depth_dev, const T* centers_dev, int N, int C, int H, int W,
-           const int32_t* keypoint_config, const OkpCamera* camera, const OkpDecodeParams* params,
+           const int32_t* keypoint_config, const OkpCamera* camera, const OkpCamera* cameras_dev, const OkpDecodeParams* params,
            const OkpDecodeTables* tables, void* workspace_dev, size_t workspace_bytes, const OkpRecordSink* sink,
            void* stream) {
     int rc = check_params(params);
@@ -313,7 +335,7 @@ int decode(const T* heat_dev, const T* depth_dev, const T* centers_dev, int N, i
     if (rc != OKP_OK) return rc;
     if (N == 0) return OKP_OK;
     OkpGroupArgs a;
-    rc = make_group_args(depth_dev, centers_dev, N, C, H, W, keypoint_config, camera, params, tables, sink, &a);
+    rc = make_group_args(depth_dev, centers_dev, N, C, H, W, keypoint_config, camera, cameras_dev, params, tables, sink, &a);
     if (rc != OKP_OK) return rc;
     PeakCall call;
     rc = prepare_peaks<T>(heat_dev, N, C, H, W, params, tables, workspace_dev, workspace_bytes, &call);
@@ -325,13 +347,13 @@ int decode(const T* heat_dev, const T* depth_dev, const T* centers_dev, int N, i
     // form is faster at every size, so it is the default; OkpDecodeParams.single_pass asks for the fused one, whose groups
     // are whole frames with their grouping scratch: a plan of its own.
     OkpStreamPlan fused_plan;
-    const bool fused = params->single_pass != 0 && call.plan.strip && params->top_k == 0 &&
+    const bool fused = params->single_pass != 0 && !cameras_dev && call.plan.strip && params->top_k == 0 &&
                        okp_stream_plan(N * C, C, H, W, params->max_peaks, (int)sizeof(T), a.frame_smem_bytes, params->lean_tables,
                                        &fused_plan) && fused_plan.F > 0;
     if (!fused) {
         rc = launch_peaks<T>(heat_dev, call, N * C, C, W, params, tables, s);
         if (rc != OKP_OK) return rc;
-        return launch_group<T>(a, 0, tables, s);
+        return launch_group<T>(a, 0, tables, cameras_dev, s);
     }
     rc = okp_stream_launch<T>(heat_dev, fused_plan, params->threshold, *tables, &a, call.group_counter, s);
     if (rc != OKP_OK) return rc;
@@ -339,7 +361,7 @@ int decode(const T* heat_dev, const T* depth_dev, const T* centers_dev, int N, i
     // map each is one read of peak_count / n_objects
     rc = launch_overflow<T>(heat_dev, call, N * C, params, tables, s);
     if (rc != OKP_OK) return rc;
-    return launch_group<T>(a, 1, tables, s);
+    return launch_group<T>(a, 1, tables, nullptr, s);
 }
 
 }  // namespace
@@ -371,20 +393,20 @@ int okp_extract_peaks_f16(const void* heat_dev, int N, int C, int H, int W, cons
 int okp_group_objects_f32(const float* depth_dev, const float* centers_dev, int N, int C, int H, int W,
                           const int32_t* keypoint_config, const OkpCamera* camera, const OkpDecodeParams* params,
                           const OkpDecodeTables* tables, void* stream) {
-    return group_objects<float>(depth_dev, centers_dev, N, C, H, W, keypoint_config, camera, params, tables, nullptr, stream);
+    return group_objects<float>(depth_dev, centers_dev, N, C, H, W, keypoint_config, camera, nullptr, params, tables, nullptr, stream);
 }
 
 int okp_group_objects_bf16(const void* depth_dev, const void* centers_dev, int N, int C, int H, int W,
                            const int32_t* keypoint_config, const OkpCamera* camera, const OkpDecodeParams* params,
                            const OkpDecodeTables* tables, void* stream) {
     return group_objects<__nv_bfloat16>((const __nv_bfloat16*)depth_dev, (const __nv_bfloat16*)centers_dev, N, C, H, W,
-                                        keypoint_config, camera, params, tables, nullptr, stream);
+                                        keypoint_config, camera, nullptr, params, tables, nullptr, stream);
 }
 
 int okp_group_objects_f16(const void* depth_dev, const void* centers_dev, int N, int C, int H, int W,
                           const int32_t* keypoint_config, const OkpCamera* camera, const OkpDecodeParams* params,
                           const OkpDecodeTables* tables, void* stream) {
-    return group_objects<__half>((const __half*)depth_dev, (const __half*)centers_dev, N, C, H, W, keypoint_config, camera,
+    return group_objects<__half>((const __half*)depth_dev, (const __half*)centers_dev, N, C, H, W, keypoint_config, camera, nullptr,
                                  params, tables, nullptr, stream);
 }
 
@@ -403,7 +425,7 @@ int okp_host_alias(const void* host_ptr, void** dev_ptr_out) {
 int okp_decode_f32(const float* heat_dev, const float* depth_dev, const float* centers_dev, int N, int C, int H, int W,
                    const int32_t* keypoint_config, const OkpCamera* camera, const OkpDecodeParams* params,
                    const OkpDecodeTables* tables, void* workspace_dev, size_t workspace_bytes, void* stream) {
-    return decode<float>(heat_dev, depth_dev, centers_dev, N, C, H, W, keypoint_config, camera, params, tables, workspace_dev,
+    return decode<float>(heat_dev, depth_dev, centers_dev, N, C, H, W, keypoint_config, camera, nullptr, params, tables, workspace_dev,
                          workspace_bytes, nullptr, stream);
 }
 
@@ -411,14 +433,14 @@ int okp_decode_bf16(const void* heat_dev, const void* depth_dev, const void* cen
                     const int32_t* keypoint_config, const OkpCamera* camera, const OkpDecodeParams* params,
                     const OkpDecodeTables* tables, void* workspace_dev, size_t workspace_bytes, void* stream) {
     return decode<__nv_bfloat16>((const __nv_bfloat16*)heat_dev, (const __nv_bfloat16*)depth_dev, (const __nv_bfloat16*)centers_dev,
-                                 N, C, H, W, keypoint_config, camera, params, tables, workspace_dev, workspace_bytes, nullptr, stream);
+                                 N, C, H, W, keypoint_config, camera, nullptr, params, tables, workspace_dev, workspace_bytes, nullptr, stream);
 }
 
 int okp_decode_f16(const void* heat_dev, const void* depth_dev, const void* centers_dev, int N, int C, int H, int W,
                    const int32_t* keypoint_config, const OkpCamera* camera, const OkpDecodeParams* params,
                    const OkpDecodeTables* tables, void* workspace_dev, size_t workspace_bytes, void* stream) {
     return decode<__half>((const __half*)heat_dev, (const __half*)depth_dev, (const __half*)centers_dev, N, C, H, W,
-                          keypoint_config, camera, params, tables, workspace_dev, workspace_bytes, nullptr, stream);
+                          keypoint_config, camera, nullptr, params, tables, workspace_dev, workspace_bytes, nullptr, stream);
 }
 
 int okp_record_bytes(int O, int C, const int32_t* keypoint_config) {
@@ -435,7 +457,7 @@ int okp_decode_emit_f32(const float* heat_dev, const float* depth_dev, const flo
                         const int32_t* keypoint_config, const OkpCamera* camera, const OkpDecodeParams* params,
                         const OkpDecodeTables* tables, void* workspace_dev, size_t workspace_bytes,
                         const OkpRecordSink* sink, void* stream) {
-    return decode<float>(heat_dev, depth_dev, centers_dev, N, C, H, W, keypoint_config, camera, params, tables, workspace_dev,
+    return decode<float>(heat_dev, depth_dev, centers_dev, N, C, H, W, keypoint_config, camera, nullptr, params, tables, workspace_dev,
                          workspace_bytes, sink, stream);
 }
 
@@ -444,7 +466,7 @@ int okp_decode_emit_bf16(const void* heat_dev, const void* depth_dev, const void
                          const OkpDecodeTables* tables, void* workspace_dev, size_t workspace_bytes,
                          const OkpRecordSink* sink, void* stream) {
     return decode<__nv_bfloat16>((const __nv_bfloat16*)heat_dev, (const __nv_bfloat16*)depth_dev, (const __nv_bfloat16*)centers_dev,
-                                 N, C, H, W, keypoint_config, camera, params, tables, workspace_dev, workspace_bytes, sink, stream);
+                                 N, C, H, W, keypoint_config, camera, nullptr, params, tables, workspace_dev, workspace_bytes, sink, stream);
 }
 
 int okp_decode_emit_f16(const void* heat_dev, const void* depth_dev, const void* centers_dev, int N, int C, int H, int W,
@@ -452,27 +474,85 @@ int okp_decode_emit_f16(const void* heat_dev, const void* depth_dev, const void*
                         const OkpDecodeTables* tables, void* workspace_dev, size_t workspace_bytes,
                         const OkpRecordSink* sink, void* stream) {
     return decode<__half>((const __half*)heat_dev, (const __half*)depth_dev, (const __half*)centers_dev, N, C, H, W,
-                          keypoint_config, camera, params, tables, workspace_dev, workspace_bytes, sink, stream);
+                          keypoint_config, camera, nullptr, params, tables, workspace_dev, workspace_bytes, sink, stream);
 }
 
 int okp_group_objects_emit_f32(const float* depth_dev, const float* centers_dev, int N, int C, int H, int W,
                                const int32_t* keypoint_config, const OkpCamera* camera, const OkpDecodeParams* params,
                                const OkpDecodeTables* tables, const OkpRecordSink* sink, void* stream) {
-    return group_objects<float>(depth_dev, centers_dev, N, C, H, W, keypoint_config, camera, params, tables, sink, stream);
+    return group_objects<float>(depth_dev, centers_dev, N, C, H, W, keypoint_config, camera, nullptr, params, tables, sink, stream);
 }
 
 int okp_group_objects_emit_bf16(const void* depth_dev, const void* centers_dev, int N, int C, int H, int W,
                                 const int32_t* keypoint_config, const OkpCamera* camera, const OkpDecodeParams* params,
                                 const OkpDecodeTables* tables, const OkpRecordSink* sink, void* stream) {
     return group_objects<__nv_bfloat16>((const __nv_bfloat16*)depth_dev, (const __nv_bfloat16*)centers_dev, N, C, H, W,
-                                        keypoint_config, camera, params, tables, sink, stream);
+                                        keypoint_config, camera, nullptr, params, tables, sink, stream);
 }
 
 int okp_group_objects_emit_f16(const void* depth_dev, const void* centers_dev, int N, int C, int H, int W,
                                const int32_t* keypoint_config, const OkpCamera* camera, const OkpDecodeParams* params,
                                const OkpDecodeTables* tables, const OkpRecordSink* sink, void* stream) {
-    return group_objects<__half>((const __half*)depth_dev, (const __half*)centers_dev, N, C, H, W, keypoint_config, camera,
+    return group_objects<__half>((const __half*)depth_dev, (const __half*)centers_dev, N, C, H, W, keypoint_config, camera, nullptr,
                                  params, tables, sink, stream);
+}
+
+int okp_decode_cameras_f32(const float* heat_dev, const float* depth_dev, const float* centers_dev, int N, int C, int H, int W,
+                           const int32_t* keypoint_config, const OkpCamera* cameras_dev, const OkpDecodeParams* params,
+                           const OkpDecodeTables* tables, void* workspace_dev, size_t workspace_bytes,
+                           const OkpRecordSink* sink, void* stream) {
+    const int rc = check_cameras(N, depth_dev, cameras_dev, params);
+    if (rc != OKP_OK) return rc;
+    return decode<float>(heat_dev, depth_dev, centers_dev, N, C, H, W, keypoint_config, nullptr, cameras_dev, params, tables,
+                         workspace_dev, workspace_bytes, sink, stream);
+}
+
+int okp_decode_cameras_bf16(const void* heat_dev, const void* depth_dev, const void* centers_dev, int N, int C, int H, int W,
+                            const int32_t* keypoint_config, const OkpCamera* cameras_dev, const OkpDecodeParams* params,
+                            const OkpDecodeTables* tables, void* workspace_dev, size_t workspace_bytes,
+                            const OkpRecordSink* sink, void* stream) {
+    const int rc = check_cameras(N, depth_dev, cameras_dev, params);
+    if (rc != OKP_OK) return rc;
+    return decode<__nv_bfloat16>((const __nv_bfloat16*)heat_dev, (const __nv_bfloat16*)depth_dev, (const __nv_bfloat16*)centers_dev,
+                                 N, C, H, W, keypoint_config, nullptr, cameras_dev, params, tables, workspace_dev, workspace_bytes,
+                                 sink, stream);
+}
+
+int okp_decode_cameras_f16(const void* heat_dev, const void* depth_dev, const void* centers_dev, int N, int C, int H, int W,
+                           const int32_t* keypoint_config, const OkpCamera* cameras_dev, const OkpDecodeParams* params,
+                           const OkpDecodeTables* tables, void* workspace_dev, size_t workspace_bytes,
+                           const OkpRecordSink* sink, void* stream) {
+    const int rc = check_cameras(N, depth_dev, cameras_dev, params);
+    if (rc != OKP_OK) return rc;
+    return decode<__half>((const __half*)heat_dev, (const __half*)depth_dev, (const __half*)centers_dev, N, C, H, W,
+                          keypoint_config, nullptr, cameras_dev, params, tables, workspace_dev, workspace_bytes, sink, stream);
+}
+
+int okp_group_objects_cameras_f32(const float* depth_dev, const float* centers_dev, int N, int C, int H, int W,
+                                  const int32_t* keypoint_config, const OkpCamera* cameras_dev, const OkpDecodeParams* params,
+                                  const OkpDecodeTables* tables, const OkpRecordSink* sink, void* stream) {
+    const int rc = check_cameras(N, depth_dev, cameras_dev, params);
+    if (rc != OKP_OK) return rc;
+    return group_objects<float>(depth_dev, centers_dev, N, C, H, W, keypoint_config, nullptr, cameras_dev, params, tables, sink,
+                                stream);
+}
+
+int okp_group_objects_cameras_bf16(const void* depth_dev, const void* centers_dev, int N, int C, int H, int W,
+                                   const int32_t* keypoint_config, const OkpCamera* cameras_dev, const OkpDecodeParams* params,
+                                   const OkpDecodeTables* tables, const OkpRecordSink* sink, void* stream) {
+    const int rc = check_cameras(N, depth_dev, cameras_dev, params);
+    if (rc != OKP_OK) return rc;
+    return group_objects<__nv_bfloat16>((const __nv_bfloat16*)depth_dev, (const __nv_bfloat16*)centers_dev, N, C, H, W,
+                                        keypoint_config, nullptr, cameras_dev, params, tables, sink, stream);
+}
+
+int okp_group_objects_cameras_f16(const void* depth_dev, const void* centers_dev, int N, int C, int H, int W,
+                                  const int32_t* keypoint_config, const OkpCamera* cameras_dev, const OkpDecodeParams* params,
+                                  const OkpDecodeTables* tables, const OkpRecordSink* sink, void* stream) {
+    const int rc = check_cameras(N, depth_dev, cameras_dev, params);
+    if (rc != OKP_OK) return rc;
+    return group_objects<__half>((const __half*)depth_dev, (const __half*)centers_dev, N, C, H, W, keypoint_config, nullptr,
+                                 cameras_dev, params, tables, sink, stream);
 }
 
 int okp_fisheye_undistort_f64(const double* xy_dev, int n, const OkpCamera* camera, int round_to_f32,

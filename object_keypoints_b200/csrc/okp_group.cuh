@@ -10,7 +10,8 @@
 //     frame's sorted peak list in shared memory while the compute warps stream the next frames -- the normal path;
 //   * in okp_group_kernel below, which first pulls the frame's peak tables from HBM: the stand-alone entry
 //     (okp_group_objects_*), shapes the fused kernel does not cover, and the fix-up of frames one of whose maps
-//     took the overflow path (marked by n_objects = OKP_GROUP_PENDING).
+//     took the overflow path (marked by n_objects = OKP_GROUP_PENDING);
+//   * in okp_group_cameras_kernel, the same steps with one camera per frame (okp_*_cameras_*).
 #pragma once
 #include "okp_common.cuh"
 #include "okp_geometry.cuh"
@@ -103,13 +104,15 @@ struct OkpGroupArgs {
     int frame_smem_bytes;           // okp_group_smem_bytes()
 };
 
-// Shared-memory bytes ONE frame (= one warp) of the grouping needs.
-static inline size_t okp_group_smem_bytes(int C, int K, int O) {
+// Shared-memory bytes ONE frame (= one warp) of the grouping needs. The per-frame-camera form (okp_group_cameras_kernel)
+// keeps the frame's OkpCamera behind the scratch: the last sizeof(OkpCamera) bytes, 16-byte aligned.
+static_assert(sizeof(OkpCamera) % 16 == 0, "OkpCamera is copied as 16-byte words");
+static inline size_t okp_group_smem_bytes(int C, int K, int O, bool per_frame_camera = false) {
     size_t bytes = (size_t)O * 2 * sizeof(double);                                                  // centres
     bytes += (size_t)C * K * (2 * sizeof(double) + 2 * sizeof(float) + sizeof(float) + 2 * sizeof(int));
     bytes += (size_t)O * C * sizeof(int) + (size_t)O * sizeof(int);
     bytes += (2 * OKP_MAX_MAPS + 2) * sizeof(int);                                                  // counts, starts, flags
-    return (bytes + 15) / 16 * 16;
+    return (bytes + 15) / 16 * 16 + (per_frame_camera ? sizeof(OkpCamera) : 0);
 }
 
 // The frame's scratch, carved out of `mine` (okp_group_smem_bytes() bytes, 16-byte aligned).
@@ -167,10 +170,13 @@ __device__ __forceinline__ OkpGroupScratch okp_group_scratch(unsigned char* mine
 // the kernel is issue-bound with 12 active lanes per instruction: two frames per warp halve the warp instructions per
 // frame). `lane` is the thread's index inside its frame, FULL the mask of the frame's lanes in the warp; the two halves of
 // a warp run independently (every warp-level primitive below names the frame's own mask).
-template <typename E, int LANES = 32>
+// FRAME_CAMERA = false: the frame is lifted with the call's camera a.cam; true: with *frame_camera (the frame's row of the
+// caller's camera table, already in the frame's shared scratch).
+template <typename E, int LANES = 32, bool FRAME_CAMERA = false>
 __device__ __forceinline__ void okp_group_frame(const int n, const int lane, const OkpGroupScratch& g, const OkpGroupArgs& a,
-                                                const OkpDecodeTables& t) {
+                                                const OkpDecodeTables& t, const OkpCamera* frame_camera = nullptr) {
     constexpr int THREADS = LANES;
+    const OkpCamera& cam = FRAME_CAMERA ? *frame_camera : a.cam;
     const unsigned FULL = LANES == 32 ? 0xffffffffu : (0xffffu << (threadIdx.x & 16));
     const bool CLEAR = a.prm.lean_tables == 0;
     const int C = a.C, H = a.H, W = a.W, S = a.S;
@@ -338,7 +344,7 @@ __device__ __forceinline__ void okp_group_frame(const int n, const int lane, con
             reinterpret_cast<float2*>(t.kp_xy)[oc * S + s] = make_float2(pts[s][0], pts[s][1]);
             double p3[3] = {0.0, 0.0, 0.0};
             if (a.have_camera) {
-                okp_detection_to_point(pts[s][0], pts[s][1], depth + (m0 + c) * HW, H, W, a.cam, a.prm.compat_clip_bug, p3);
+                okp_detection_to_point(pts[s][0], pts[s][1], depth + (m0 + c) * HW, H, W, cam, a.prm.compat_clip_bug, p3);
                 double* out = t.kp_point + (oc * S + s) * 3;
                 out[0] = p3[0]; out[1] = p3[1]; out[2] = p3[2];
             }
@@ -368,7 +374,7 @@ __device__ __forceinline__ void okp_group_frame(const int n, const int lane, con
         reinterpret_cast<float2*>(t.kp_xy)[ocs] = make_float2(px, py);
         double p3[3] = {0.0, 0.0, 0.0};
         if (a.have_camera) {
-            okp_detection_to_point(px, py, depth + (m0 + c) * HW, H, W, a.cam, a.prm.compat_clip_bug, p3);
+            okp_detection_to_point(px, py, depth + (m0 + c) * HW, H, W, cam, a.prm.compat_clip_bug, p3);
             double* out = t.kp_point + ocs * 3;
             out[0] = p3[0]; out[1] = p3[1]; out[2] = p3[2];
         }
@@ -385,7 +391,8 @@ __device__ __forceinline__ void okp_group_frame(const int n, const int lane, con
 // Stand-alone form: one warp per frame, four frames per CTA (an SM holds 64 frames whose latency chains overlap).
 // The frame's peak records are pulled from the tables into shared memory with one round trip. only_pending != 0: only
 // frames marked OKP_GROUP_PENDING by the fused decode kernel are processed (the fix-up launch: with no overflowing map
-// it is one read of n_objects per frame).
+// it is one read of n_objects per frame). okp_group_cameras_kernel below repeats these first steps (flags, counts, the
+// pull of the peak records): a change to one of the two belongs in the other.
 template <typename E, int LANES>
 __global__ void __launch_bounds__(128)
 okp_group_kernel(const __grid_constant__ OkpGroupArgs a, const int only_pending, const OkpDecodeTables t) {
@@ -419,4 +426,50 @@ okp_group_kernel(const __grid_constant__ OkpGroupArgs a, const int only_pending,
     }
     __syncwarp(mask);
     okp_group_frame<E, LANES>(n, lane, g, a, t);
+}
+
+// Per-frame cameras (okp_decode_cameras_*, okp_group_objects_cameras_*): okp_group_kernel's steps, except that the frame's
+// lanes first copy cameras[n] (device memory, 16-byte aligned: 9 words of 16 bytes) into the last bytes of the frame's
+// scratch (okp_group_smem_bytes(..., true)) and the 3D lift reads that copy instead of a.cam, which is not read. Never a
+// fix-up launch: the fused single pass has no per-frame-camera form. A kernel of its own rather than a template flag of
+// okp_group_kernel: any rewrapping of that kernel's body changes its register allocation and scheduling.
+// Registers: under __launch_bounds__(128) alone ptxas settles on 64 (32 lanes) / 72 (16 lanes) and reloads loop invariants
+// from the stack in every iteration of pass 2, the per-peak lift loop. 72 registers keep pass 2 free of spills in both
+// forms (the remaining few spill bytes sit around the clustering call); a 128-thread CTA still fits 7 times per SM by
+// registers, and the 16-lane form (8 frames per CTA) is limited by shared memory first.
+template <typename E, int LANES>
+__global__ void __maxnreg__(72)
+okp_group_cameras_kernel(const __grid_constant__ OkpGroupArgs a, const OkpDecodeTables t, const OkpCamera* __restrict__ cameras) {
+    constexpr int SHIFT = LANES == 32 ? 5 : 4;
+    constexpr int WORDS = (int)(sizeof(OkpCamera) / sizeof(uint4));
+    const int lane = threadIdx.x & (LANES - 1);
+    const unsigned mask = LANES == 32 ? 0xffffffffu : (0xffffu << (threadIdx.x & 16));
+    const int n = blockIdx.x * (blockDim.x >> SHIFT) + (threadIdx.x >> SHIFT);
+    okp_wait_for_predecessor();
+    if (n >= a.N) return;
+    const int C = a.C, K = a.prm.max_peaks, O = a.prm.max_objects;
+    extern __shared__ __align__(16) unsigned char group_smem[];
+    unsigned char* const mine = group_smem + (size_t)(threadIdx.x >> SHIFT) * a.frame_smem_bytes;
+    const OkpGroupScratch g = okp_group_scratch(mine, C, K, O);
+    OkpCamera* const camera = reinterpret_cast<OkpCamera*>(mine + a.frame_smem_bytes - sizeof(OkpCamera));
+    if (lane < WORDS) reinterpret_cast<uint4*>(camera)[lane] = __ldg(reinterpret_cast<const uint4*>(cameras + n) + lane);
+    const size_t m0 = (size_t)n * C;
+    if (lane == 0) *g.flags = t.flags[n] & OKP_FLAG_GENERIC_PATH;
+    __syncwarp(mask);
+    if (lane < C) {
+        const int c = t.peak_count[m0 + lane];
+        g.counts[lane] = c < K ? c : K;
+        if (c > K) atomicOr(g.flags, OKP_FLAG_PEAK_OVERFLOW);
+    }
+    __syncwarp(mask);
+    for (int i = lane; i < C * K; i += LANES) {
+        const int c = i / K, k = i - c * K;
+        if (k >= g.counts[c]) continue;
+        const size_t s = (m0 + c) * K + k;
+        const float2 p = *reinterpret_cast<const float2*>(t.peak_xy + 2 * s);
+        g.xy[2 * i] = p.x; g.xy[2 * i + 1] = p.y;
+        g.conf[i] = t.peak_conf[s];
+    }
+    __syncwarp(mask);
+    okp_group_frame<E, LANES, true>(n, lane, g, a, t, camera);
 }

@@ -112,6 +112,38 @@ class DecodeTables:
                 for name, dtype, shape, start, nbytes in self._layout}
 
 
+class CameraTable:
+    """One camera per frame on the device (KeypointDecoder.camera_table): ``rows`` is a [N, 144] uint8 CUDA tensor of
+    OkpCamera records (include/okp.h), row n the camera frame n of a batch is lifted with. Built once per batch layout
+    and passed as ``cameras=`` to every decode of that layout, so no call uploads cameras."""
+    RECORD_BYTES = ctypes.sizeof(_abi.OkpCamera)
+
+    def __init__(self, rows):
+        if rows.dtype != torch.uint8 or rows.dim() != 2 or rows.shape[1] != self.RECORD_BYTES or not rows.is_cuda:
+            raise ValueError(f"rows must be a [N, {self.RECORD_BYTES}] uint8 CUDA tensor")
+        if rows.data_ptr() % 16 or not rows.is_contiguous():
+            raise ValueError("rows must be contiguous and 16-byte aligned")
+        self.rows = rows
+        self.N = int(rows.shape[0])
+
+    def data_ptr(self):
+        return self.rows.data_ptr()
+
+    def frames(self, start, stop):
+        """The rows of frames [start, stop): a view, i.e. a pointer offset into the same table."""
+        return CameraTable(self.rows[start:stop])
+
+    def check(self, N, device):
+        """The table must describe this batch and live on the decoder's device: the kernel reads it by raw pointer."""
+        if self.N != N:
+            raise ValueError(f"the camera table has {self.N} rows, the batch {N} frames")
+        if device.index is None:                             # 'cuda' = the current device
+            device = torch.device(device.type, torch.cuda.current_device())
+        if self.rows.device != device:
+            raise ValueError(f"the camera table is on {self.rows.device}, the decoder on {device}")
+        return self
+
+
 class KeypointDecoder:
     """Batched heatmap -> grouped 2D keypoints -> 3D points on the GPU.
 
@@ -142,6 +174,16 @@ class KeypointDecoder:
         """camera: object exposing K, D, Kinv, image_size (camera_utils.FisheyeCamera or the
         reference's own class), as DetectionToPoint.reset receives it (pipeline.py:159-162)."""
         self._camera = _abi.pack_camera(camera)
+
+    def camera_table(self, cameras, camera_index):
+        """Per-frame cameras for ``decode_batch`` / ``group_objects`` / ``decode_host_batch(cameras=...)``: a short
+        sequence of camera objects (as ``reset`` takes them) and camera_index [N], the index into ``cameras`` of every
+        frame -> CameraTable on this decoder's device. E.g. a stereo batch with the left views in even and the right views
+        in odd rows: ``camera_table((stereo.left_camera, stereo.right_camera), np.arange(N) % 2)``. The indices are
+        checked here (_abi.pack_camera_table); build the table once per batch layout and reuse it."""
+        packed = _abi.pack_camera_table(cameras, camera_index)
+        host = np.frombuffer(bytes(packed), dtype=np.uint8).reshape(len(packed), CameraTable.RECORD_BYTES)
+        return CameraTable(_aligned(torch.from_numpy(host.copy()).to(self.device)))
 
     def tables(self, N):
         if N not in self._tables:
@@ -177,7 +219,7 @@ class KeypointDecoder:
         """Bytes of one compact per-frame record (okp_decode_emit_*, include/okp.h)."""
         return int(self._lib.okp_record_bytes(self.params.max_objects, self.C, self._cfg_array))
 
-    def decode_batch(self, heat, depth, centers, tables=None, stream=None, records=None, peaks_done=None):
+    def decode_batch(self, heat, depth, centers, tables=None, stream=None, records=None, peaks_done=None, cameras=None):
         """heat [N,C,H,W], depth [N,C,H,W], centers [N,C-1,2,H,W] (float32, bfloat16 or float16; CUDA tensors
         are used in place, host arrays are copied, 16-bit tensors keep their type) -> DecodeTables on the device. No
         synchronisation. Heatmaps of one type with depth / centre maps of another take two C calls (peaks, then
@@ -187,7 +229,9 @@ class KeypointDecoder:
         peaks_done: a ``torch.cuda.Event`` recorded between the peak kernel (+ its overflow fix-up) and the grouping
         kernel -- the two halves are then enqueued by two C calls instead of one. A PAIR of timing events instead is
         recorded by the library right before and right after the peak kernel itself (okp_extract_peaks_events_f32:
-        bench.py's roofline figure is the time between them)."""
+        bench.py's roofline figure is the time between them).
+        cameras: a CameraTable with N rows (camera_table): frame n is lifted with its own camera instead of ``reset``'s
+        (okp_decode_cameras_* / okp_group_objects_cameras_*; not with ``single_pass``)."""
         heat, heat_kind = _as_device_map(heat, self.device)
         self._check(heat)
         depth, depth_kind = _as_device_map(depth, self.device)
@@ -201,13 +245,15 @@ class KeypointDecoder:
             raise ValueError(f"centers must be [N,{self.C - 1},2,{self.H},{self.W}], got {tuple(centers.shape)}")
         tables = self.tables(N) if tables is None else tables
         ws = self._workspace_for(N)
-        cam = ctypes.byref(self._camera) if self._camera is not None else None
+        # the _cameras entries take the DEVICE table where the _emit entries take the host camera
+        form, cam = ('cameras', ctypes.c_void_p(cameras.check(N, self.device).data_ptr())) if cameras is not None else \
+            ('emit', ctypes.byref(self._camera) if self._camera is not None else None)
         if heat_kind == depth_kind and peaks_done is None:
-            rc = getattr(self._lib, f'okp_decode_emit_{heat_kind}')(
+            rc = getattr(self._lib, f'okp_decode_{form}_{heat_kind}')(
                 heat.data_ptr(), depth.data_ptr(), centers.data_ptr(), N, self.C, self.H, self.W, self._cfg_array, cam,
                 ctypes.byref(self.params), ctypes.byref(tables.struct), ws.data_ptr(), ws.numel(),
                 ctypes.byref(records) if records is not None else None, _stream_handle(stream))
-            _lib.check(rc, f'okp_decode_emit_{heat_kind}')
+            _lib.check(rc, f'okp_decode_{form}_{heat_kind}')
         else:                                                # e.g. 16-bit heatmaps with float32 depth / centre maps
             pair = peaks_done if isinstance(peaks_done, (tuple, list)) else None
             if pair is not None and heat_kind == 'f32':
@@ -226,11 +272,11 @@ class KeypointDecoder:
                 _lib.check(rc, f'okp_extract_peaks_{heat_kind}')
                 for event in (pair if pair is not None else [peaks_done] if peaks_done is not None else []):
                     event.record(torch.cuda.current_stream(self.device) if stream is None else stream)
-            rc = getattr(self._lib, f'okp_group_objects_emit_{depth_kind}')(
+            rc = getattr(self._lib, f'okp_group_objects_{form}_{depth_kind}')(
                 depth.data_ptr(), centers.data_ptr(), N, self.C, self.H, self.W, self._cfg_array, cam,
                 ctypes.byref(self.params), ctypes.byref(tables.struct),
                 ctypes.byref(records) if records is not None else None, _stream_handle(stream))
-            _lib.check(rc, f'okp_group_objects_emit_{depth_kind}')
+            _lib.check(rc, f'okp_group_objects_{form}_{depth_kind}')
         return tables
 
     HOST_RESULT_TABLES = ('n_objects', 'flags', 'kp_count', 'kp_xy', 'kp_point')
@@ -290,7 +336,7 @@ class KeypointDecoder:
         return {name: torch.empty((N,) + tuple(like[name].shape[1:]), dtype=like[name].dtype).pin_memory()
                 for name in self.HOST_RESULT_TABLES}
 
-    def decode_host_batch(self, heat, depth, centers, chunk_frames=128, sparse='auto', out=None):
+    def decode_host_batch(self, heat, depth, centers, chunk_frames=128, sparse='auto', out=None, cameras=None):
         """End-to-end form for HOST inputs, the shape the reference's caller has (CPU tensors out of
         InferenceComponent, pipeline.py:24-28). The batch is cut into chunks that are pipelined: while chunk i is
         decoded, chunk i+1 crosses PCIe and chunk i+2 is prepared on the host. The three maps are float32, bfloat16
@@ -310,8 +356,11 @@ class KeypointDecoder:
         heatmaps. The host pass is float32-only: 16-bit heatmaps always take the dense copy. The object tables of
         every chunk are copied back into pinned host tensors.
         Returns a dict of CPU tensors (synchronised): freshly allocated for every call, or ``out`` (a dict from an earlier
-        call or from ``host_result``) filled in place."""
+        call or from ``host_result``) filled in place. cameras: a CameraTable with N rows, as in ``decode_batch``; each
+        chunk reads its own rows of it, wherever the chunk boundaries fall."""
         self._check_host_inputs(heat, depth, centers)
+        if cameras is not None:
+            cameras.check(int(heat.shape[0]), self.device)
         heat, depth, centers = heat.contiguous(), depth.contiguous(), centers.contiguous()
         N = int(heat.shape[0])
         chunk = max(1, min(chunk_frames, N))
@@ -415,7 +464,15 @@ class KeypointDecoder:
                 slot['ready'].record(copy_stream)
             compute.wait_event(slot['ready'])
             tables = slot['tables'] if n == chunk else self.tables(n)
-            if in_place:
+            chunk_cameras = cameras.frames(f0, f1) if cameras is not None else None
+            if in_place and chunk_cameras is not None:
+                ws = self._workspace_for(n)
+                rc = getattr(self._lib, f'okp_decode_cameras_{kind}')(
+                    slot['heat'].data_ptr(), depth_alias + f0 * depth_frame, centers_alias + f0 * centers_frame, n, self.C,
+                    self.H, self.W, self._cfg_array, ctypes.c_void_p(chunk_cameras.data_ptr()), ctypes.byref(self.params),
+                    ctypes.byref(tables.struct), ws.data_ptr(), ws.numel(), None, _stream_handle(compute))
+                _lib.check(rc, f'okp_decode_cameras_{kind}')
+            elif in_place:
                 ws = self._workspace_for(n)
                 rc = getattr(self._lib, f'okp_decode_{kind}')(
                     slot['heat'].data_ptr(), depth_alias + f0 * depth_frame, centers_alias + f0 * centers_frame, n, self.C,
@@ -423,7 +480,8 @@ class KeypointDecoder:
                     ws.data_ptr(), ws.numel(), _stream_handle(compute))
                 _lib.check(rc, f'okp_decode_{kind}')
             else:
-                self.decode_batch(slot['heat'][:n], slot['depth'][:n], slot['centers'][:n], tables=tables)
+                self.decode_batch(slot['heat'][:n], slot['depth'][:n], slot['centers'][:n], tables=tables,
+                                  cameras=chunk_cameras)
             for name in self.HOST_RESULT_TABLES:
                 result[name][f0:f1].copy_(tables[name][:n], non_blocking=True)
             slot['done'].record(compute)
@@ -482,10 +540,24 @@ class KeypointDecoder:
         self.host_marked_fraction = marked_tiles[0] / marked_tiles[1] if marked_tiles[1] else None
         return result
 
-    def group_objects(self, depth, centers, tables, stream=None):
-        """K3 + K4 on peak tables that are already filled (ObjectExtraction + DetectionToPoint)."""
+    def group_objects(self, depth, centers, tables, stream=None, cameras=None):
+        """K3 + K4 on peak tables that are already filled (ObjectExtraction + DetectionToPoint). cameras: a CameraTable
+        with tables.N rows, as in ``decode_batch`` (needs depth)."""
         N = tables.N
         centers, kind = _as_device_map(centers, self.device)
+        if cameras is not None:
+            if depth is None:
+                raise ValueError("the 3D lift with per-frame cameras needs the depth maps")
+            cameras.check(N, self.device)
+            depth, depth_kind = _as_device_map(depth, self.device)
+            if depth_kind != kind:
+                depth, centers, kind = depth.float(), centers.float(), 'f32'
+            rc = getattr(self._lib, f'okp_group_objects_cameras_{kind}')(
+                depth.data_ptr(), centers.data_ptr(), N, self.C, self.H, self.W, self._cfg_array,
+                ctypes.c_void_p(cameras.data_ptr()), ctypes.byref(self.params), ctypes.byref(tables.struct), None,
+                _stream_handle(stream))
+            _lib.check(rc, f'okp_group_objects_cameras_{kind}')
+            return tables
         depth_ptr = None
         cam = None
         if depth is not None and self._camera is not None:
@@ -664,9 +736,10 @@ class ObjectKeypointPipeline:
     def reset(self, camera):
         self.decoder.reset(camera)
 
-    def decode_batch(self, heatmap, p_depth, p_centers, stream=None):
-        """Any batch size, device tables out (no host round trip)."""
-        return self.decoder.decode_batch(heatmap, p_depth, p_centers, stream=stream)
+    def decode_batch(self, heatmap, p_depth, p_centers, stream=None, cameras=None):
+        """Any batch size, device tables out (no host round trip). cameras: a ``self.decoder.camera_table(...)`` with one
+        camera per frame, in place of ``reset``'s."""
+        return self.decoder.decode_batch(heatmap, p_depth, p_centers, stream=stream, cameras=cameras)
 
     def __call__(self, heatmap, p_depth, p_centers):
         assert heatmap.shape[0] == 1, "One at the time, please."
