@@ -379,6 +379,42 @@ int okp_associate_pairs_f64(const double* F_dev, const double* left_dev, const i
                             int max_right, double max_distance_px, int32_t* match_dev, double* cost_dev,
                             void* stream);
 
+/* Stereo objects: the decoded objects of P frame pairs of one stereo rig, matched across the two views and triangulated in
+ * the left camera's frame. O = max_objects, S = max(1, max(keypoint_config)) as in OkpDecodeTables; all arrays are device
+ * memory, dense row-major with the shapes given, and every entry is written. */
+#define OKP_STEREO_AMBIGUOUS 1u   /* a left object had two or more right objects within max_distance_px before the greedy
+                                     step: objects on one epipolar line, which epipolar matching cannot tell apart */
+#define OKP_STEREO_BAD_PAIR 2u    /* a frame index of the pair is outside [0, N): nothing was read or matched */
+typedef struct OkpStereoTables {
+    int32_t* object_match;  /* [P,O]       right object of left object o, -1 */
+    double*  object_cost;   /* [P,O]       epipolar cost of that match (pixels), 0 where there is none */
+    int32_t* slot_match;    /* [P,O,C,S]   right object's slot matched to left slot s, -1 */
+    double*  point;         /* [P,O,C,S,3] left camera frame, NaN where slot_match is -1 */
+    uint32_t* flags;        /* [P]         OKP_STEREO_* */
+} OkpStereoTables;
+
+/* For each pair p = (l, r) = (pairs_dev[2p], pairs_dev[2p+1]) of frames of `tables` (N frames decoded with C maps,
+ * keypoint_config and params; lean tables or cleared ones, only valid slots are read):
+ *   1. every valid keypoint kp_xy[f,o,c,s] (s < kp_count) of both frames is undistorted with its view's camera;
+ *   2. objects are matched by their centre keypoints with the cost and greedy one-to-one rule of okp_stereo_associate_f64
+ *      (mean point-to-epipolar-line distance, globally smallest first, ties to the smaller left then right index, while
+ *      cost <= max_distance_px);
+ *   3. for each matched object pair and each spoke type c >= 1 the two objects' slots of type c are matched the same way
+ *      (the centre slot is matched with its object);
+ *   4. every matched keypoint pair is triangulated like StereoCamera.triangulate (camera_utils.py:92-110): undistorted
+ *      points rounded to float32, with optimal_correction the Hartley-Sturm correction of okp_correct_matches_f64 rounded
+ *      to float32, then the two-view DLT with P_L, P_R, dehomogenised.
+ * F, P_L, P_R: 9, 12, 12 doubles row-major on the HOST (StereoCamera.F with x_R^T F x_L = 0, and
+ * StereoCamera.projection_matrices: K_L [I|0], K_R T_RL[:3]). pairs_dev: DEVICE int32 [P,2]; a pair with an index
+ * outside [0, N) gets OKP_STEREO_BAD_PAIR. P = 0 returns OKP_OK. Refused on the host, before any CUDA call: NULL pointers
+ * (OKP_E_NULL); N < 0, P < 0, C out of range, max_objects > 64 or 1 + sum(keypoint_config) > 64 (OKP_E_SHAPE: the greedy
+ * step keeps its used rows and columns in 64-bit masks). */
+int okp_triangulate_stereo_objects_f64(const OkpDecodeTables* tables, int N, int C, const int32_t* keypoint_config,
+                                       const OkpDecodeParams* params, const int32_t* pairs_dev, int P,
+                                       const OkpCamera* left_camera, const OkpCamera* right_camera, const double* F,
+                                       const double* P_L, const double* P_R, double max_distance_px, int optimal_correction,
+                                       const OkpStereoTables* out, void* stream);
+
 /* Evaluation bookkeeping (SURVEY section 8f rank 3). Replaces Results.add of the reference's
  * scripts/eval_model.py:141-187 for a batch of N frames, reading the decode tables in place:
  * kp_point_dev [N,O,C,S,3], kp_count_dev [N,O,C], n_objects_dev [N] (OkpDecodeTables fields), T_WC_dev

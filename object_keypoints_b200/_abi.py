@@ -22,6 +22,9 @@ FLAG_NO_CENTERS = 32
 FLAG_ARGMAX_RESOLVED = 64
 FLAG_GENERIC_PATH = 128      # property of the call, not of the data: the shape / mode ran on the exact generic kernels
 
+STEREO_AMBIGUOUS = 1         # OkpStereoTables.flags: a left object had two or more right objects within reach
+STEREO_BAD_PAIR = 2          # ... a frame index of the pair is outside the batch
+
 ERRORS = {0: 'OKP_OK', -1: 'OKP_E_NULL', -2: 'OKP_E_SHAPE', -3: 'OKP_E_CAPACITY',
           -4: 'OKP_E_UNSUPPORTED', -5: 'OKP_E_CUDA', -6: 'OKP_E_WORKSPACE'}
 
@@ -68,6 +71,34 @@ TABLE_LAYOUT = [
 
 class OkpDecodeTables(ctypes.Structure):
     _fields_ = [(name, ctypes.c_void_p) for name, _, _ in TABLE_LAYOUT]
+
+
+# OkpStereoTables: name, numpy dtype, shape as a function of (P, O, C, S) -- order = field order in okp.h
+STEREO_LAYOUT = [
+    ('object_match', np.int32, lambda P, O, C, S: (P, O)),
+    ('object_cost', np.float64, lambda P, O, C, S: (P, O)),
+    ('slot_match', np.int32, lambda P, O, C, S: (P, O, C, S)),
+    ('point', np.float64, lambda P, O, C, S: (P, O, C, S, 3)),
+    ('flags', np.uint32, lambda P, O, C, S: (P,)),
+]
+
+
+class OkpStereoTables(ctypes.Structure):
+    _fields_ = [(name, ctypes.c_void_p) for name, _, _ in STEREO_LAYOUT]
+
+
+def check_pairs(pairs, N):
+    """Frame pairs of okp_triangulate_stereo_objects_f64: [P, 2] integers (left frame, right frame) in [0, N) -> int32
+    array. The library reads the frames they name, so they are checked here, like pack_camera_table checks its indices:
+    ValueError for a shape other than [P, 2], non-integers and indices outside [0, N)."""
+    pairs = np.asarray(pairs)
+    if pairs.ndim != 2 or pairs.shape[1] != 2:
+        raise ValueError(f"pairs must be [P, 2] (left frame, right frame), got shape {pairs.shape}")
+    if pairs.size and pairs.dtype.kind not in 'iu':
+        raise ValueError(f"pairs must hold integers, got {pairs.dtype}")
+    if pairs.size and (pairs.min() < 0 or pairs.max() >= N):
+        raise ValueError(f"pairs out of range: values in [{pairs.min()}, {pairs.max()}] for {N} frames")
+    return np.ascontiguousarray(pairs, dtype=np.int32)
 
 
 def table_dims(N, C, keypoint_config, params):

@@ -684,6 +684,48 @@ int okp_associate_pairs_f64(const double* F_dev, const double* left_dev, const i
     return OKP_OK;
 }
 
+int okp_triangulate_stereo_objects_f64(const OkpDecodeTables* tables, int N, int C, const int32_t* keypoint_config,
+                                       const OkpDecodeParams* params, const int32_t* pairs_dev, int P,
+                                       const OkpCamera* left_camera, const OkpCamera* right_camera, const double* F,
+                                       const double* P_L, const double* P_R, double max_distance_px, int optimal_correction,
+                                       const OkpStereoTables* out, void* stream) {
+    if (N < 0 || P < 0 || C < 1 || C > OKP_MAX_MAPS) return OKP_E_SHAPE;
+    if (P == 0) return OKP_OK;
+    if (!tables || !params || (C > 1 && !keypoint_config) || !pairs_dev || !left_camera || !right_camera || !F || !P_L ||
+        !P_R || !out)
+        return OKP_E_NULL;
+    if (!tables->n_objects || !tables->kp_count || !tables->kp_xy || !out->object_match || !out->object_cost ||
+        !out->slot_match || !out->point || !out->flags)
+        return OKP_E_NULL;
+    OkpStereoShape d;
+    memset(&d, 0, sizeof(d));
+    d.N = N; d.C = C; d.O = params->max_objects;
+    if (d.O < 1 || d.O > 64) return OKP_E_SHAPE;                     // the greedy step's 64-bit masks
+    d.cfg[0] = 1;
+    d.S = 1; d.P = 1;
+    for (int c = 1; c < C; ++c) {
+        const int k = keypoint_config[c - 1];
+        if (k < 1 || k > OKP_MAX_SLOTS) return OKP_E_CAPACITY;
+        d.cfg[c] = k; d.off[c] = d.P;
+        d.P += k;
+        if (k > d.S) d.S = k;
+    }
+    if (d.P > 64) return OKP_E_SHAPE;
+    OkpStereoRig rig;
+    rig.cam[0] = *left_camera;
+    rig.cam[1] = *right_camera;
+    for (int i = 0; i < 9; ++i) rig.F.m[i] = F[i];
+    rig.ep = okp_epipoles(rig.F);                                     // as okp_correct_matches_f64 does
+    for (int i = 0; i < 12; ++i) { rig.proj[0][i] = P_L[i]; rig.proj[1][i] = P_R[i]; }
+    const size_t smem = okp_stereo_smem_bytes(d.O, d.C, d.P);
+    if (smem > 48 * 1024)
+        OKP_CUDA_CHECK(cudaFuncSetAttribute(okp_stereo_objects_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    okp_stereo_objects_kernel<<<P, 32, smem, (cudaStream_t)stream>>>(rig, d, tables->n_objects, tables->kp_count, tables->kp_xy,
+                                                                     pairs_dev, max_distance_px, optimal_correction, *out);
+    OKP_CUDA_CHECK(cudaGetLastError());
+    return OKP_OK;
+}
+
 int okp_eval_match_f64(const double* kp_point_dev, const int32_t* kp_count_dev, const int32_t* n_objects_dev,
                        const double* T_WC_dev, const double* scene_points_dev, int N, int O, int C, int S, int G, int Kp,
                        const OkpCamera* camera, double frame_limit_x, double frame_limit_y, double max_coordinate,

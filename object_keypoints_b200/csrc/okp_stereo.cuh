@@ -297,8 +297,51 @@ okp_correct_matches_kernel(OkpMat3 F, OkpEpipoles ep, const double* __restrict__
 // distances (pixels) of UNDISTORTED points, x_R^T F x_L = 0. Greedy one-to-one: repeatedly take
 // the globally smallest remaining cost (ties: smallest left index, then smallest right index)
 // until it exceeds max_distance. Statement of record: oracle/np_oracle.py::associate.
+// okp_associate_kernel and okp_stereo_objects_kernel share the cost and the greedy step below.
 // ---------------------------------------------------------------------------------------------
 #define OKP_ASSOC_MAX 64
+
+__device__ __forceinline__ double okp_epipolar_cost(const double* F, double x, double y, double xp, double yp) {
+    const double l0 = F[0] * x + F[1] * y + F[2], l1 = F[3] * x + F[4] * y + F[5], l2 = F[6] * x + F[7] * y + F[8];
+    const double m0 = F[0] * xp + F[3] * yp + F[6], m1 = F[1] * xp + F[4] * yp + F[7];
+    const double r = fabs(xp * l0 + yp * l1 + l2);
+    return 0.5 * (r / sqrt(l0 * l0 + l1 * l1) + r / sqrt(m0 * m0 + m1 * m1));
+}
+
+// The greedy one-to-one step on the costs s_cost[i * stride + j] (i < nl, j < nr <= 64), run by all 32 lanes of a warp.
+// The caller clears s_used_left / s_used_right and syncs the warp first. Lane 0 calls on_match(i, j, cost) for every
+// match, in the order the matches are taken.
+template <typename OnMatch>
+__device__ __forceinline__ void okp_greedy_match(const double* s_cost, int stride, int nl, int nr, double max_distance,
+                                                 unsigned long long& s_used_left, unsigned long long& s_used_right,
+                                                 int lane, OnMatch on_match) {
+    const int rounds = nl < nr ? nl : nr;
+    for (int round = 0; round < rounds; ++round) {
+        const unsigned long long ul = s_used_left, ur = s_used_right;
+        double best = INFINITY;
+        int arg = 0x7fffffff;
+        for (int e = lane; e < nl * nr; e += 32) {
+            const int i = e / nr, j = e - i * nr;
+            if (((ul >> i) & 1ull) || ((ur >> j) & 1ull)) continue;
+            const double c = s_cost[i * stride + j];
+            if (c < best || (c == best && e < arg)) { best = c; arg = e; }
+        }
+#pragma unroll
+        for (int off = 16; off > 0; off >>= 1) {
+            const double ob = __shfl_xor_sync(0xffffffffu, best, off);
+            const int oa = __shfl_xor_sync(0xffffffffu, arg, off);
+            if (ob < best || (ob == best && oa < arg)) { best = ob; arg = oa; }
+        }
+        if (!(best <= max_distance)) break;
+        const int i = arg / nr, j = arg - i * nr;
+        if (lane == 0) {
+            on_match(i, j, best);
+            s_used_left = ul | (1ull << i);
+            s_used_right = ur | (1ull << j);
+        }
+        __syncwarp();
+    }
+}
 
 __global__ void __launch_bounds__(32)
 okp_associate_kernel(OkpMat3 Fm, const double* __restrict__ F_pairs, const double* __restrict__ left,
@@ -315,11 +358,7 @@ okp_associate_kernel(OkpMat3 Fm, const double* __restrict__ F_pairs, const doubl
     const double* R = right + (size_t)b * MR * 2;
     for (int e = lane; e < nl * nr; e += 32) {
         const int i = e / nr, j = e - i * nr;
-        const double x = L[2 * i], y = L[2 * i + 1], xp = R[2 * j], yp = R[2 * j + 1];
-        const double l0 = F[0] * x + F[1] * y + F[2], l1 = F[3] * x + F[4] * y + F[5], l2 = F[6] * x + F[7] * y + F[8];
-        const double m0 = F[0] * xp + F[3] * yp + F[6], m1 = F[1] * xp + F[4] * yp + F[7];
-        const double r = fabs(xp * l0 + yp * l1 + l2);
-        s_cost[i * MR + j] = 0.5 * (r / sqrt(l0 * l0 + l1 * l1) + r / sqrt(m0 * m0 + m1 * m1));
+        s_cost[i * MR + j] = okp_epipolar_cost(F, L[2 * i], L[2 * i + 1], R[2 * j], R[2 * j + 1]);
     }
     for (int i = lane; i < ML; i += 32) {
         match[(size_t)b * ML + i] = -1;
@@ -327,31 +366,176 @@ okp_associate_kernel(OkpMat3 Fm, const double* __restrict__ F_pairs, const doubl
     }
     if (lane == 0) { s_used_left = 0ull; s_used_right = 0ull; }
     __syncwarp();
-    const int rounds = nl < nr ? nl : nr;
-    for (int round = 0; round < rounds; ++round) {
-        const unsigned long long ul = s_used_left, ur = s_used_right;
-        double best = INFINITY;
-        int arg = 0x7fffffff;
-        for (int e = lane; e < nl * nr; e += 32) {
-            const int i = e / nr, j = e - i * nr;
-            if (((ul >> i) & 1ull) || ((ur >> j) & 1ull)) continue;
-            const double c = s_cost[i * MR + j];
-            if (c < best || (c == best && e < arg)) { best = c; arg = e; }
-        }
-#pragma unroll
-        for (int off = 16; off > 0; off >>= 1) {
-            const double ob = __shfl_xor_sync(0xffffffffu, best, off);
-            const int oa = __shfl_xor_sync(0xffffffffu, arg, off);
-            if (ob < best || (ob == best && oa < arg)) { best = ob; arg = oa; }
-        }
-        if (!(best <= max_distance)) break;
-        const int i = arg / nr, j = arg - i * nr;
-        if (lane == 0) {
-            match[(size_t)b * ML + i] = j;
-            match_cost[(size_t)b * ML + i] = best;
-            s_used_left = ul | (1ull << i);
-            s_used_right = ur | (1ull << j);
-        }
-        __syncwarp();
+    okp_greedy_match(s_cost, MR, nl, nr, max_distance, s_used_left, s_used_right, lane, [&](int i, int j, double cost) {
+        match[(size_t)b * ML + i] = j;
+        match_cost[(size_t)b * ML + i] = cost;
+    });
+}
+
+// ---------------------------------------------------------------------------------------------
+// Stereo objects: triangulate the decoded objects of P frame pairs (left frame, right frame) of one
+// rig, one warp per pair. Statement of record: oracle/stereo_oracle.py::stereo_objects.
+//   1. undistort every valid keypoint of both frames with its view's camera (lanes own keypoints);
+//   2. match objects by their centre keypoints: okp_epipolar_cost + okp_greedy_match, as
+//      okp_associate_kernel does (lanes own (left, right) cost entries);
+//   3. for each matched object pair and spoke type, match the two objects' slots the same way;
+//   4. triangulate every matched keypoint pair (lanes own pairs) like StereoCamera.triangulate: the
+//      undistorted points rounded to float32, optionally okp_correct_pair (rounded to float32), then
+//      the two-view DLT with P_L = K_L [I|0], P_R = K_R T_RL[:3], dehomogenised.
+// Matching reads the unrounded undistorted points, as AssociationComponent does.
+// Keypoints of an object are kept in compact order k = off[c] + s (P = 1 + sum(keypoint_config) of them).
+// ---------------------------------------------------------------------------------------------
+#include "okp_geometry.cuh"
+#include "okp_dlt.cuh"
+
+struct OkpStereoRig {
+    OkpCamera cam[2];          // left, right
+    OkpMat3 F;                 // x_R^T F x_L = 0
+    OkpEpipoles ep;            // okp_epipoles(F), once per call on the host
+    double proj[2][12];        // P_L, P_R row-major 3x4
+};
+
+struct OkpStereoShape {
+    int N, C, O, S, P;         // P: keypoints per object (compact)
+    int32_t cfg[OKP_MAX_MAPS]; // cfg[0] = 1
+    int32_t off[OKP_MAX_MAPS]; // compact offset of map c
+};
+
+// Shared bytes per pair (one warp per CTA): undistorted points of both frames, centre costs, slot costs, matched-pair
+// list, right slot of every left keypoint, matched right object of every left object, keypoint counts of both frames.
+__host__ __device__ inline size_t okp_stereo_smem_bytes(int O, int C, int P) {
+    return sizeof(double) * 2 * 2 * (size_t)O * P + sizeof(double) * (size_t)O * O + sizeof(double) * OKP_MAX_SLOTS * OKP_MAX_SLOTS +
+           sizeof(uint32_t) * (size_t)O * P + (size_t)O * P + (size_t)O + 2 * (size_t)O * C;
+}
+
+__global__ void __launch_bounds__(32)
+okp_stereo_objects_kernel(OkpStereoRig rig, OkpStereoShape d, const int32_t* __restrict__ n_objects,
+                          const int32_t* __restrict__ kp_count, const float* __restrict__ kp_xy,
+                          const int32_t* __restrict__ pairs, double max_distance, int optimal_correction,
+                          OkpStereoTables out) {
+    extern __shared__ double s_xy[];                              // [2][O][P][2]
+    double* s_cost = s_xy + 4 * d.O * d.P;                        // [O][O] centre costs
+    double* s_slot_cost = s_cost + d.O * d.O;                     // [8][8] slot costs of one (object pair, type)
+    uint32_t* s_list = (uint32_t*)(s_slot_cost + OKP_MAX_SLOTS * OKP_MAX_SLOTS);   // matched keypoint pairs
+    int8_t* s_slot = (int8_t*)(s_list + d.O * d.P);               // [O][P] right slot of a left keypoint, -1
+    int8_t* s_object = s_slot + d.O * d.P;                        // [O] right object of a left object, -1
+    int8_t* s_count = s_object + d.O;                             // [2][O][C] keypoints kept
+    __shared__ unsigned long long s_used_left, s_used_right;
+    __shared__ int s_n_list;
+    const int p = blockIdx.x, lane = threadIdx.x;
+    const int O = d.O, C = d.C, S = d.S, P = d.P;
+    const int fl = pairs[2 * p], fr = pairs[2 * p + 1];
+    const bool bad = fl < 0 || fl >= d.N || fr < 0 || fr >= d.N;
+    const int nl = bad ? 0 : okp_clamp(n_objects[fl], 0, O), nr = bad ? 0 : okp_clamp(n_objects[fr], 0, O);
+    for (int e = lane; e < 2 * O * C; e += 32) {
+        const bool right = e >= O * C;
+        const int o = (e / C) % O, c = e % C;
+        s_count[e] = (int8_t)(o < (right ? nr : nl) ? okp_clamp(kp_count[((size_t)(right ? fr : fl) * O + o) * C + c], 0, d.cfg[c]) : 0);
     }
+    for (int e = lane; e < O * P; e += 32) s_slot[e] = -1;
+    for (int o = lane; o < O; o += 32) {
+        s_object[o] = -1;
+        out.object_match[(size_t)p * O + o] = -1;
+        out.object_cost[(size_t)p * O + o] = 0.0;
+    }
+    if (lane == 0) { s_used_left = 0ull; s_used_right = 0ull; s_n_list = 0; }
+    __syncwarp();
+    // 1. undistortion
+#pragma unroll
+    for (int v = 0; v < 2; ++v) {
+        const int f = v ? fr : fl;
+        for (int e = lane; e < (v ? nr : nl) * C * S; e += 32) {
+            const int o = e / (C * S), c = (e / S) % C, s = e % S;
+            if (s >= s_count[(v * O + o) * C + c]) continue;
+            const float* xy = kp_xy + ((((size_t)f * O + o) * C + c) * S + s) * 2;
+            double* u = s_xy + 2 * ((v * O + o) * P + d.off[c] + s);
+            okp_undistort_point((double)xy[0], (double)xy[1], rig.cam[v], u, u + 1);
+        }
+    }
+    __syncwarp();
+    // 2. objects by their centres
+    const double* L = s_xy;
+    const double* R = s_xy + 2 * O * P;
+    for (int e = lane; e < nl * nr; e += 32) {
+        const int i = e / nr, j = e - i * nr;
+        s_cost[i * O + j] = okp_epipolar_cost(rig.F.m, L[2 * i * P], L[2 * i * P + 1], R[2 * j * P], R[2 * j * P + 1]);
+    }
+    __syncwarp();
+    bool ambiguous = false;                                       // two or more right centres within reach of one left centre
+    for (int i = lane; i < nl; i += 32) {
+        int within = 0;
+        for (int j = 0; j < nr; ++j) within += s_cost[i * O + j] <= max_distance;
+        ambiguous |= within >= 2;
+    }
+    ambiguous = __any_sync(0xffffffffu, ambiguous);
+    okp_greedy_match(s_cost, O, nl, nr, max_distance, s_used_left, s_used_right, lane, [&](int i, int j, double cost) {
+        out.object_match[(size_t)p * O + i] = j;
+        out.object_cost[(size_t)p * O + i] = cost;
+        s_object[i] = (int8_t)j;
+        s_slot[i * P] = 0;
+        s_list[s_n_list++] = (uint32_t)i | (uint32_t)j << 8;      // left object, right object, map 0, slots 0
+    });
+    __syncwarp();
+    // 3. slots of every matched object pair, type by type
+    for (int i = 0; i < nl; ++i) {
+        const int j = s_object[i];
+        if (j < 0) continue;
+        for (int c = 1; c < C; ++c) {
+            const int nsl = s_count[i * C + c], nsr = s_count[(O + j) * C + c];
+            if (nsl == 0 || nsr == 0) continue;
+            const double* Ls = L + 2 * (i * P + d.off[c]);
+            const double* Rs = R + 2 * (j * P + d.off[c]);
+            for (int e = lane; e < nsl * nsr; e += 32) {
+                const int a = e / nsr, b = e - a * nsr;
+                s_slot_cost[a * OKP_MAX_SLOTS + b] = okp_epipolar_cost(rig.F.m, Ls[2 * a], Ls[2 * a + 1], Rs[2 * b], Rs[2 * b + 1]);
+            }
+            if (lane == 0) { s_used_left = 0ull; s_used_right = 0ull; }
+            __syncwarp();
+            okp_greedy_match(s_slot_cost, OKP_MAX_SLOTS, nsl, nsr, max_distance, s_used_left, s_used_right, lane,
+                             [&](int a, int b, double) {
+                s_slot[i * P + d.off[c] + a] = (int8_t)b;
+                s_list[s_n_list++] = (uint32_t)i | (uint32_t)j << 8 | (uint32_t)c << 16 | (uint32_t)a << 20 | (uint32_t)b << 24;
+            });
+            __syncwarp();
+        }
+    }
+    // slot_match for every slot; NaN points where nothing is matched
+    const double nan = __longlong_as_double(0x7ff8000000000000LL);
+    for (int e = lane; e < O * C * S; e += 32) {
+        const int o = e / (C * S), c = (e / S) % C, s = e % S;
+        const int m = s < d.cfg[c] ? s_slot[o * P + d.off[c] + s] : -1;
+        const size_t at = (size_t)p * O * C * S + e;
+        out.slot_match[at] = m;
+        if (m < 0) { out.point[3 * at] = nan; out.point[3 * at + 1] = nan; out.point[3 * at + 2] = nan; }
+    }
+    // 4. correction + DLT of every matched keypoint pair
+    for (int e = lane; e < s_n_list; e += 32) {
+        const uint32_t w = s_list[e];
+        const int i = w & 255, j = (w >> 8) & 255, c = (w >> 16) & 15, a = (w >> 20) & 15, b = w >> 24;
+        const double* l = L + 2 * (i * P + d.off[c] + a);
+        const double* r = R + 2 * (j * P + d.off[c] + b);
+        double x[2][2] = {{(double)(float)l[0], (double)(float)l[1]}, {(double)(float)r[0], (double)(float)r[1]}};
+        if (optimal_correction) {
+            okp_correct_pair(rig.F, rig.ep, x[0][0], x[0][1], x[1][0], x[1][1], x[0], x[1]);
+#pragma unroll
+            for (int v = 0; v < 2; ++v) { x[v][0] = (double)(float)x[v][0]; x[v][1] = (double)(float)x[v][1]; }
+        }
+        double A[4][4] = {};
+#pragma unroll
+        for (int v = 0; v < 2; ++v) {
+            const double* M = rig.proj[v];
+            double row[4];
+#pragma unroll
+            for (int k = 0; k < 4; ++k) row[k] = x[v][0] * M[8 + k] - M[k];
+            okp_givens_append(A, row);
+#pragma unroll
+            for (int k = 0; k < 4; ++k) row[k] = x[v][1] * M[8 + k] - M[4 + k];
+            okp_givens_append(A, row);
+        }
+        double h[4];
+        okp_smallest_right_singular_vector(A, h);
+        double* X = out.point + 3 * ((((size_t)p * O + i) * C + c) * S + a);
+        X[0] = h[0] / h[3]; X[1] = h[1] / h[3]; X[2] = h[2] / h[3];
+    }
+    if (lane == 0) out.flags[p] = (bad ? OKP_STEREO_BAD_PAIR : 0u) | (ambiguous ? OKP_STEREO_AMBIGUOUS : 0u);
 }

@@ -82,17 +82,16 @@ def _as_device_map(x, device):
     return _as_device_f32(x, device), 'f32'
 
 
-class DecodeTables:
-    """The OkpDecodeTables record as torch tensors on one device (layout: include/okp.h). All tables are views
-    into ONE allocation (each starting on a 256-byte boundary), so that the synchronising host copy of a decode --
-    what the reference-style per-frame ``__call__`` does after every frame -- is a single transfer."""
+class _TableSet:
+    """Tables as torch tensors on one device, all views into ONE allocation (each starting on a 256-byte boundary), so
+    that the synchronising host copy of a call is a single transfer. shapes: (name, numpy dtype, shape) in the field
+    order of `struct_type`, the matching ctypes struct of device pointers (include/okp.h)."""
     ALIGN = 256
 
-    def __init__(self, N, C, keypoint_config, params, device):
-        self.N, self.C = N, C
+    def __init__(self, shapes, struct_type, device):
         self._layout = []
         offset = 0
-        for name, dtype, shape in _abi.table_shapes(N, C, keypoint_config, params):
+        for name, dtype, shape in shapes:
             nbytes = int(np.prod(shape, dtype=np.int64)) * np.dtype(dtype).itemsize
             self._layout.append((name, np.dtype(dtype), tuple(shape), offset, nbytes))
             offset += (nbytes + self.ALIGN - 1) // self.ALIGN * self.ALIGN
@@ -100,7 +99,7 @@ class DecodeTables:
         self.tensors = {}
         for name, dtype, shape, start, nbytes in self._layout:
             self.tensors[name] = self.flat[start:start + nbytes].view(_TORCH_DTYPES[dtype]).reshape(shape)
-        self.struct = _abi.OkpDecodeTables(**{k: v.data_ptr() for k, v in self.tensors.items()})
+        self.struct = struct_type(**{k: v.data_ptr() for k, v in self.tensors.items()})
 
     def __getitem__(self, name):
         return self.tensors[name]
@@ -110,6 +109,28 @@ class DecodeTables:
         host = self.flat.cpu().numpy()
         return {name: host[start:start + nbytes].view(np.uint32 if name == 'flags' else dtype).reshape(shape)
                 for name, dtype, shape, start, nbytes in self._layout}
+
+
+class DecodeTables(_TableSet):
+    """The OkpDecodeTables record as torch tensors on one device (layout: include/okp.h), in one allocation: the
+    synchronising host copy of a decode -- what the reference-style per-frame ``__call__`` does after every frame -- is a
+    single transfer. keypoint_config and params are kept for the calls that read the tables (triangulate_stereo_objects)."""
+
+    def __init__(self, N, C, keypoint_config, params, device):
+        self.N, self.C = N, C
+        self.keypoint_config, self.params = list(keypoint_config), params
+        super().__init__(_abi.table_shapes(N, C, keypoint_config, params), _abi.OkpDecodeTables, device)
+
+
+class StereoTables(_TableSet):
+    """The OkpStereoTables record of triangulate_stereo_objects as torch tensors on one device, in one allocation:
+    object_match [P,O], object_cost [P,O], slot_match [P,O,C,S], point [P,O,C,S,3] (left camera frame, NaN where
+    slot_match is -1), flags [P] (_abi.STEREO_*)."""
+
+    def __init__(self, P, O, C, S, device):
+        self.P = P
+        super().__init__([(name, dtype, shape(P, O, C, S)) for name, dtype, shape in _abi.STEREO_LAYOUT],
+                         _abi.OkpStereoTables, device)
 
 
 class CameraTable:

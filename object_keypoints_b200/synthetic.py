@@ -313,3 +313,134 @@ def torch_grid_batch(n_frames, keypoint_config, size=(180, 320), seed=0, grid=(4
                     cys[disc] = vy[disc]
         heat[f0:f0 + n] = h.clamp_(0.0, 1.0)
     return heat, depth, centers, n_obj
+
+
+# --------------------------------------------------------------------------------------------
+# Stereo scenes: 3D objects in front of a rig, rasterised in both views (triangulate_stereo_objects).
+# --------------------------------------------------------------------------------------------
+def stereo_rig(prediction_size=(64, 64)):
+    """The config/calibration.yaml rig (cam0 left, cam1 right) with both cameras scaled and cut as default_camera does."""
+    import os
+    from . import camera_utils
+    p = camera_utils.load_calibration_params(os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))),
+                                                          'config', 'calibration.yaml'))
+    cameras = []
+    for K, D in ((p['K'], p['D']), (p['Kp'], p['Dp'])):
+        camera = camera_utils.FisheyeCamera(K, D, p['image_size'])
+        if tuple(prediction_size) == (64, 64):
+            scaled = camera.scale(511.0 / 720.0)
+            camera = scaled.cut(np.array([(scaled.image_size[1] - 511.0) / 2.0, 0.0])).scale(64.0 / 511.0)
+        else:
+            camera = camera.scale(prediction_size[0] / 720.0)
+        cameras.append(camera)
+    return camera_utils.StereoCamera(cameras[0], cameras[1], p['T_RL'])
+
+
+@dataclass
+class StereoBatch:
+    batch: Batch                 # 2P frames: the left view of pair p in row 2p, its right view in row 2p + 1
+    points: list                 # per pair: [n_obj, 1 + sum(cfg), 3] left camera frame; centre, then types and slots in order
+    right_of_left: list          # per pair: [n_obj], the right view's index of the left view's object i
+    pixels: list                 # per pair: ([n_obj, 1 + sum(cfg), 2] left, [...] right) distorted pixels
+
+
+def _epipolar_distance(F, left, right):
+    """Mean of the two point-to-epipolar-line distances, as oracle/np_oracle.associate scores a pair (undistorted px)."""
+    lx = F @ np.array([left[0], left[1], 1.0])
+    ly = F.T @ np.array([right[0], right[1], 1.0])
+    r = abs(right[0] * lx[0] + right[1] * lx[1] + lx[2])
+    return 0.5 * (r / np.hypot(lx[0], lx[1]) + r / np.hypot(ly[0], ly[1]))
+
+
+def stereo_batch(P, keypoint_config, size, stereo, seed, objects=(1, 4), depth_range=(0.5, 1.2), centre_margin=5.0, slot_margin=1.0,
+                 center_separation=22.0, spoke_radius=(5.0, 8.0), peak_separation=6.0, border=4.0, max_tries=5000):
+    """P stereo pairs of one rig. Per pair: objects (a centre and keypoint_config[t] keypoints of every type t) are placed
+    in front of the rig: pixels and depths are sampled in the left view under sample_scene's separations, lifted to 3D
+    and projected into the right view with FisheyeCamera.project; the right view must keep the centres' separation too.
+    Two different objects' centres stay farther than centre_margin from each other's epipolar line (no object is
+    ambiguous at max_distance_px < centre_margin), and two different keypoints of one object and type farther than
+    slot_margin (the construction's matching is the greedy one on noiseless keypoints). Each view is
+    rasterised with `rasterize`, z taken in that view's camera frame; the objects of a view are listed in raster order of
+    their centre pixel, the order in which the decode finds them."""
+    H, W = size
+    cams = (stereo.left_camera, stereo.right_camera)
+    T = (np.eye(4), stereo.T_RL)
+    n_kp = 1 + sum(keypoint_config)
+    heat = np.zeros((2 * P, len(keypoint_config) + 1, H, W), dtype=np.float32)
+    depth = np.zeros_like(heat)
+    centers = np.zeros((2 * P, len(keypoint_config), 2, H, W), dtype=np.float32)
+    scenes, points, right_of_left, pixels = [], [], [], []
+    lo, hi = np.array([border, border]), np.array([W - 1 - border, H - 1 - border])
+
+    def inside(px):
+        return bool((px >= lo).all() and (px <= hi).all())
+
+    for p, child in enumerate(np.random.SeedSequence(seed).spawn(P)):
+        rng = np.random.default_rng(child)
+        n_obj = int(rng.integers(objects[0], objects[1] + 1))
+        for _ in range(max_tries):
+            left = sample_scene(rng, keypoint_config, size, n_obj, center_separation, spoke_radius, peak_separation, border)
+            px_l = np.concatenate([left.centers[:, None]] + list(left.spokes), axis=1)        # [n_obj, n_kp, 2]
+            z = rng.uniform(*depth_range, size=n_obj)[:, None] + rng.uniform(-0.03, 0.03, size=(n_obj, n_kp))
+            und = cams[0].undistort(px_l.reshape(-1, 2))
+            X = (np.concatenate([und, np.ones((und.shape[0], 1))], axis=1) @ cams[0].Kinv.T) * z.reshape(-1, 1)
+            views = [c.project(X, t).reshape(n_obj, n_kp, 2) for c, t in zip(cams, T)]
+            if not all(inside(v) for v in views[1].reshape(-1, 2)):
+                continue
+            if not _far_enough_all(views[1][:, 0], center_separation):
+                continue
+            und_views = [c.undistort(v.reshape(-1, 2)).reshape(n_obj, n_kp, 2) for c, v in zip(cams, views)]
+            if not _epipolar_unique(stereo.F, und_views, keypoint_config, centre_margin, slot_margin):
+                continue
+            break
+        else:
+            raise RuntimeError("could not place the requested objects; relax the separations")
+        X = X.reshape(n_obj, n_kp, 3)
+        orders = [np.lexsort((np.rint(v[:, 0, 0]), np.rint(v[:, 0, 1]))) for v in views]      # raster order of the centres
+        for v, (camera_T, order) in enumerate(zip(T, orders)):
+            Xc = X[order] @ camera_T[:3, :3].T + camera_T[:3, 3]
+            px = views[v][order]
+            spokes, zs, k = [], [], 1
+            for count in keypoint_config:
+                spokes.append(px[:, k:k + count].copy())
+                zs.append(Xc[:, k:k + count, 2].copy())
+                k += count
+            scene = Scene(centers=px[:, 0].copy(), spokes=spokes,
+                          amplitude_center=rng.uniform(0.6, 1.0, size=n_obj),
+                          amplitude_spokes=[rng.uniform(0.6, 1.0, size=s.shape[:2]) for s in spokes],
+                          z_center=Xc[:, 0, 2].copy(), z_spokes=zs)
+            heat[2 * p + v], depth[2 * p + v], centers[2 * p + v] = rasterize(scene, keypoint_config, size, rng)
+            scenes.append(scene)
+        points.append(X[orders[0]])
+        rank_right = np.empty(n_obj, np.int64)
+        rank_right[orders[1]] = np.arange(n_obj)
+        right_of_left.append(rank_right[orders[0]])
+        pixels.append((views[0][orders[0]], views[1][orders[1]]))
+    batch = Batch(heat=heat, depth=depth, centers=centers, scenes=scenes, keypoint_config=list(keypoint_config))
+    return StereoBatch(batch=batch, points=points, right_of_left=right_of_left, pixels=pixels)
+
+
+def _far_enough_all(points, min_distance):
+    return all(_far_enough(points[i], points[:i], min_distance) for i in range(len(points)))
+
+
+def _epipolar_unique(F, und_views, keypoint_config, centre_margin, slot_margin):
+    """No centre of one object within centre_margin of the epipolar line of another object's centre, no keypoint of an
+    object within slot_margin of the line of another keypoint of the same object and type."""
+    left, right = und_views
+    n_obj = left.shape[0]
+    groups = [[0]]
+    k = 1
+    for count in keypoint_config:
+        groups.append(list(range(k, k + count)))
+        k += count
+    for i in range(n_obj):
+        for j in range(n_obj):
+            if i != j and _epipolar_distance(F, left[i, 0], right[j, 0]) <= centre_margin:
+                return False
+        for g in groups[1:]:
+            for a in g:
+                for b in g:
+                    if a != b and _epipolar_distance(F, left[i, a], right[i, b]) <= slot_margin:
+                        return False
+    return True

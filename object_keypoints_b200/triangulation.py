@@ -10,7 +10,9 @@
 * ``triangulate_multiview`` -- undistort, DLT over V views, reprojection-error gate, re-solve;
 * ``correct_matches`` -- cv2.correctMatches (Hartley-Sturm) as camera_utils.py:100-101 uses it;
 * ``AssociationComponent`` / ``associate`` -- stereo association by epipolar distance
-  (test/test_pipeline.py:208-261).
+  (test/test_pipeline.py:208-261);
+* ``triangulate_stereo_objects`` -- both halves on the decode tables of a stereo batch in one call: objects and
+  keypoints matched across the two views, corrected and triangulated in the left camera's frame.
 """
 import ctypes
 
@@ -18,7 +20,7 @@ import numpy as np
 import torch
 
 from . import _abi, _lib
-from .pipeline import _device, _stream_handle
+from .pipeline import StereoTables, _device, _stream_handle
 
 
 def _as_f64(x, device):
@@ -231,3 +233,39 @@ class TriangulationComponent:
     def __call__(self, left_keypoints, right_keypoints):
         return triangulate_stereo(self.stereo_camera, left_keypoints, right_keypoints,
                                   optimal_correction=self.optimal_correction)
+
+
+def triangulate_stereo_objects(tables, stereo, pairs=None, max_distance_px=2.5, optimal_correction=True, stream=None):
+    """The decoded objects of stereo frame pairs, matched across the two views and triangulated, on the device
+    (okp_triangulate_stereo_objects_f64). tables: the DecodeTables of a batch that holds both views of every pair (decode
+    it with ``camera_table((stereo.left_camera, stereo.right_camera), ...)`` so that each view is lifted with its own
+    camera). pairs: [P, 2] host integers (left frame, right frame), checked here (ValueError for a bad shape,
+    non-integers or frames outside the batch); None = (2p, 2p + 1), the interleaved layout, left views in even rows.
+    Per pair: objects are matched by the epipolar distance of their undistorted centres, greedily one to one while it is
+    <= max_distance_px (AssociationComponent's rule), then each matched object pair's slots type by type; every matched
+    keypoint pair is triangulated like StereoCamera.triangulate (optimal_correction: the Hartley-Sturm correction).
+    Returns StereoTables on the tables' device: object_match, object_cost, slot_match, point (left camera frame, NaN where
+    nothing is matched), flags (_abi.STEREO_AMBIGUOUS, _abi.STEREO_BAD_PAIR). Asynchronous: nothing synchronises."""
+    N = tables.N
+    device = tables.flat.device
+    if pairs is None:
+        if N % 2:
+            raise ValueError(f"the interleaved layout needs an even number of frames, the tables hold {N}")
+        pairs_dev = torch.arange(N, dtype=torch.int32, device=device).reshape(-1, 2)
+    else:
+        pairs_dev = torch.from_numpy(_abi.check_pairs(pairs, N)).to(device)
+    P = int(pairs_dev.shape[0])
+    O, C, S = (int(v) for v in tables['kp_xy'].shape[1:4])
+    out = StereoTables(P, O, C, S, device)
+    cfg = (ctypes.c_int32 * max(len(tables.keypoint_config), 1))(*tables.keypoint_config)
+    left, right = _abi.pack_camera(stereo.left_camera), _abi.pack_camera(stereo.right_camera)
+    F, P_L, P_R = (np.ascontiguousarray(m, dtype=np.float64) for m in (stereo.F, *stereo.projection_matrices()))
+    doubles = ctypes.POINTER(ctypes.c_double)
+    with torch.cuda.device(device):
+        rc = _lib.lib().okp_triangulate_stereo_objects_f64(
+            ctypes.byref(tables.struct), N, C, cfg, ctypes.byref(tables.params), pairs_dev.data_ptr(), P, ctypes.byref(left),
+            ctypes.byref(right), F.ctypes.data_as(doubles), P_L.ctypes.data_as(doubles), P_R.ctypes.data_as(doubles),
+            float(max_distance_px), int(bool(optimal_correction)), ctypes.byref(out.struct), _stream_handle(stream))
+    _lib.check(rc, 'okp_triangulate_stereo_objects_f64')
+    out.pairs = pairs_dev                                 # the launch reads it: kept alive with the result
+    return out
