@@ -385,6 +385,8 @@ int okp_associate_pairs_f64(const double* F_dev, const double* left_dev, const i
 #define OKP_STEREO_AMBIGUOUS 1u   /* a left object had two or more right objects within max_distance_px before the greedy
                                      step: objects on one epipolar line, which epipolar matching cannot tell apart */
 #define OKP_STEREO_BAD_PAIR 2u    /* a frame index of the pair is outside [0, N): nothing was read or matched */
+#define OKP_STEREO_NO_DEPTH 4u    /* depth association only: a candidate within max_distance_px had no valid lift in
+                                     either view, and was not matched */
 typedef struct OkpStereoTables {
     int32_t* object_match;  /* [P,O]       right object of left object o, -1 */
     double*  object_cost;   /* [P,O]       epipolar cost of that match (pixels), 0 where there is none */
@@ -414,6 +416,27 @@ int okp_triangulate_stereo_objects_f64(const OkpDecodeTables* tables, int N, int
                                        const OkpCamera* left_camera, const OkpCamera* right_camera, const double* F,
                                        const double* P_L, const double* P_R, double max_distance_px, int optimal_correction,
                                        const OkpStereoTables* out, void* stream);
+
+/* okp_triangulate_stereo_objects_f64 with depth association: objects on one epipolar line (side by side in the same
+ * image rows of this kind of rig) are told apart by each view's monocular lift, tables->kp_point (the frame's own camera
+ * frame: decode with a camera table). Per pair, the lift X of every valid keypoint is projected into the other view,
+ * q_R = pi(K_R (R_RL X_L + t_RL)) and q_L = pi(K_L (R_LR X_R + t_LR)) with T_LR = T_RL^-1 and K from fx, fy, cx, cy of
+ * the camera; a lift is valid when it is finite with z > 0. A candidate (i, j) is admissible when its epipolar cost (as
+ * above) is <= max_distance_px and d(i, j) <= max_depth_px, d = 0.5 (|q_R(i) - u_R(j)| + |q_L(j) - u_L(i)|) over the
+ * undistorted pixels u, or the one term whose lift is valid. The greedy one-to-one step of steps 2 and 3 runs on d over
+ * the admissible candidates (same tie rule); steps 1 and 4 are unchanged, and object_cost holds d. A candidate within
+ * max_distance_px without a valid lift on either side is never matched and sets OKP_STEREO_NO_DEPTH; OKP_STEREO_AMBIGUOUS
+ * marks a pair in which a left object had two or more admissible right objects.
+ * T_RL: 16 doubles row-major on the HOST (StereoCamera.T_RL, left camera frame -> right camera frame).
+ * P = 0 returns OKP_OK. Refused on the host, before any CUDA call: every refusal of okp_triangulate_stereo_objects_f64;
+ * NULL T_RL or NULL tables->kp_point (OKP_E_NULL); max_depth_px not finite or <= 0 (OKP_E_SHAPE); a shape whose shared
+ * memory, 8 (8 O P + O^2 + 64) + 5 O P + O + 2 O C bytes, exceeds sm_100's 227 KB per-block limit (OKP_E_SHAPE). */
+int okp_triangulate_stereo_objects_depth_f64(const OkpDecodeTables* tables, int N, int C, const int32_t* keypoint_config,
+                                             const OkpDecodeParams* params, const int32_t* pairs_dev, int P,
+                                             const OkpCamera* left_camera, const OkpCamera* right_camera, const double* F,
+                                             const double* P_L, const double* P_R, const double* T_RL,
+                                             double max_distance_px, double max_depth_px, int optimal_correction,
+                                             const OkpStereoTables* out, void* stream);
 
 /* Evaluation bookkeeping (SURVEY section 8f rank 3). Replaces Results.add of the reference's
  * scripts/eval_model.py:141-187 for a batch of N frames, reading the decode tables in place:

@@ -24,6 +24,7 @@ FLAG_GENERIC_PATH = 128      # property of the call, not of the data: the shape 
 
 STEREO_AMBIGUOUS = 1         # OkpStereoTables.flags: a left object had two or more right objects within reach
 STEREO_BAD_PAIR = 2          # ... a frame index of the pair is outside the batch
+STEREO_NO_DEPTH = 4          # ... association='depth': a candidate within reach had no valid lift in either view
 
 ERRORS = {0: 'OKP_OK', -1: 'OKP_E_NULL', -2: 'OKP_E_SHAPE', -3: 'OKP_E_CAPACITY',
           -4: 'OKP_E_UNSUPPORTED', -5: 'OKP_E_CUDA', -6: 'OKP_E_WORKSPACE'}

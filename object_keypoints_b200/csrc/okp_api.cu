@@ -684,20 +684,18 @@ int okp_associate_pairs_f64(const double* F_dev, const double* left_dev, const i
     return OKP_OK;
 }
 
-int okp_triangulate_stereo_objects_f64(const OkpDecodeTables* tables, int N, int C, const int32_t* keypoint_config,
-                                       const OkpDecodeParams* params, const int32_t* pairs_dev, int P,
-                                       const OkpCamera* left_camera, const OkpCamera* right_camera, const double* F,
-                                       const double* P_L, const double* P_R, double max_distance_px, int optimal_correction,
-                                       const OkpStereoTables* out, void* stream) {
-    if (N < 0 || P < 0 || C < 1 || C > OKP_MAX_MAPS) return OKP_E_SHAPE;
-    if (P == 0) return OKP_OK;
+// The host checks and set-up both stereo-objects entries share (after their P = 0 return): NULL pointers, the shape, the rig.
+static int okp_stereo_prepare(const OkpDecodeTables* tables, int N, int C, const int32_t* keypoint_config,
+                              const OkpDecodeParams* params, const int32_t* pairs_dev, const OkpCamera* left_camera,
+                              const OkpCamera* right_camera, const double* F, const double* P_L, const double* P_R,
+                              const OkpStereoTables* out, OkpStereoShape* shape, OkpStereoRig* rig_out) {
     if (!tables || !params || (C > 1 && !keypoint_config) || !pairs_dev || !left_camera || !right_camera || !F || !P_L ||
         !P_R || !out)
         return OKP_E_NULL;
     if (!tables->n_objects || !tables->kp_count || !tables->kp_xy || !out->object_match || !out->object_cost ||
         !out->slot_match || !out->point || !out->flags)
         return OKP_E_NULL;
-    OkpStereoShape d;
+    OkpStereoShape& d = *shape;
     memset(&d, 0, sizeof(d));
     d.N = N; d.C = C; d.O = params->max_objects;
     if (d.O < 1 || d.O > 64) return OKP_E_SHAPE;                     // the greedy step's 64-bit masks
@@ -711,17 +709,64 @@ int okp_triangulate_stereo_objects_f64(const OkpDecodeTables* tables, int N, int
         if (k > d.S) d.S = k;
     }
     if (d.P > 64) return OKP_E_SHAPE;
-    OkpStereoRig rig;
+    OkpStereoRig& rig = *rig_out;
     rig.cam[0] = *left_camera;
     rig.cam[1] = *right_camera;
     for (int i = 0; i < 9; ++i) rig.F.m[i] = F[i];
     rig.ep = okp_epipoles(rig.F);                                     // as okp_correct_matches_f64 does
     for (int i = 0; i < 12; ++i) { rig.proj[0][i] = P_L[i]; rig.proj[1][i] = P_R[i]; }
+    return OKP_OK;
+}
+
+int okp_triangulate_stereo_objects_f64(const OkpDecodeTables* tables, int N, int C, const int32_t* keypoint_config,
+                                       const OkpDecodeParams* params, const int32_t* pairs_dev, int P,
+                                       const OkpCamera* left_camera, const OkpCamera* right_camera, const double* F,
+                                       const double* P_L, const double* P_R, double max_distance_px, int optimal_correction,
+                                       const OkpStereoTables* out, void* stream) {
+    if (N < 0 || P < 0 || C < 1 || C > OKP_MAX_MAPS) return OKP_E_SHAPE;
+    if (P == 0) return OKP_OK;
+    OkpStereoShape d;
+    OkpStereoRig rig;
+    const int rc = okp_stereo_prepare(tables, N, C, keypoint_config, params, pairs_dev, left_camera, right_camera, F, P_L, P_R,
+                                      out, &d, &rig);
+    if (rc != OKP_OK) return rc;
     const size_t smem = okp_stereo_smem_bytes(d.O, d.C, d.P);
     if (smem > 48 * 1024)
         OKP_CUDA_CHECK(cudaFuncSetAttribute(okp_stereo_objects_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     okp_stereo_objects_kernel<<<P, 32, smem, (cudaStream_t)stream>>>(rig, d, tables->n_objects, tables->kp_count, tables->kp_xy,
                                                                      pairs_dev, max_distance_px, optimal_correction, *out);
+    OKP_CUDA_CHECK(cudaGetLastError());
+    return OKP_OK;
+}
+
+int okp_triangulate_stereo_objects_depth_f64(const OkpDecodeTables* tables, int N, int C, const int32_t* keypoint_config,
+                                             const OkpDecodeParams* params, const int32_t* pairs_dev, int P,
+                                             const OkpCamera* left_camera, const OkpCamera* right_camera, const double* F,
+                                             const double* P_L, const double* P_R, const double* T_RL,
+                                             double max_distance_px, double max_depth_px, int optimal_correction,
+                                             const OkpStereoTables* out, void* stream) {
+    if (N < 0 || P < 0 || C < 1 || C > OKP_MAX_MAPS) return OKP_E_SHAPE;
+    if (P == 0) return OKP_OK;
+    OkpStereoShape d;
+    OkpStereoRig rig;
+    const int rc = okp_stereo_prepare(tables, N, C, keypoint_config, params, pairs_dev, left_camera, right_camera, F, P_L, P_R,
+                                      out, &d, &rig);
+    if (rc != OKP_OK) return rc;
+    if (!T_RL || !tables->kp_point) return OKP_E_NULL;
+    if (!(max_depth_px > 0.0 && max_depth_px < INFINITY)) return OKP_E_SHAPE;          // NaN fails both
+    const size_t smem = okp_stereo_depth_smem_bytes(d.O, d.C, d.P);
+    if (smem > 227 * 1024) return OKP_E_SHAPE;                        // sm_100's per-block opt-in shared memory
+    OkpStereoLift lift;
+    for (int r = 0; r < 3; ++r) {                                     // [0] = T_RL, [1] = T_LR = T_RL^-1 (a rigid motion)
+        for (int c = 0; c < 3; ++c) { lift.R[0][3 * r + c] = T_RL[4 * r + c]; lift.R[1][3 * r + c] = T_RL[4 * c + r]; }
+        lift.t[0][r] = T_RL[4 * r + 3];
+        lift.t[1][r] = -(T_RL[r] * T_RL[3] + T_RL[4 + r] * T_RL[7] + T_RL[8 + r] * T_RL[11]);
+    }
+    if (smem > 48 * 1024)
+        OKP_CUDA_CHECK(cudaFuncSetAttribute(okp_stereo_depth_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    okp_stereo_depth_kernel<<<P, 32, smem, (cudaStream_t)stream>>>(rig, lift, d, tables->n_objects, tables->kp_count,
+                                                                   tables->kp_xy, tables->kp_point, pairs_dev, max_distance_px,
+                                                                   max_depth_px, optimal_correction, *out);
     OKP_CUDA_CHECK(cudaGetLastError());
     return OKP_OK;
 }

@@ -539,3 +539,197 @@ okp_stereo_objects_kernel(OkpStereoRig rig, OkpStereoShape d, const int32_t* __r
     }
     if (lane == 0) out.flags[p] = (bad ? OKP_STEREO_BAD_PAIR : 0u) | (ambiguous ? OKP_STEREO_AMBIGUOUS : 0u);
 }
+
+// ---------------------------------------------------------------------------------------------
+// Stereo objects, depth association (okp_triangulate_stereo_objects_depth_f64): the steps of okp_stereo_objects_kernel,
+// with every candidate scored by where each view's monocular lift (kp_point, in its own camera's frame) lands in the
+// other view. Statement of record: oracle/stereo_depth_oracle.py::stereo_objects_depth.
+//   1. every valid keypoint is undistorted (u) and its lift X projected into the other view, q = pi(K (R X + t)) with
+//      that view's fx, fy, cx, cy (NaN unless X is finite with z > 0): q_R of a left keypoint, q_L of a right one;
+//   2./3. candidate (i, j) is admissible when okp_epipolar_cost(u_L(i), u_R(j)) <= max_distance and
+//      d(i, j) <= max_depth, d = 0.5 (|q_R(i) - u_R(j)| + |q_L(j) - u_L(i)|), or the one term whose lift exists;
+//      okp_greedy_match runs on d (INFINITY where the epipolar gate fails), centres first, then slots type by type. A
+//      candidate inside the epipolar gate with no lift on either side is never matched and sets OKP_STEREO_NO_DEPTH;
+//      OKP_STEREO_AMBIGUOUS marks a left object with two or more admissible right objects;
+//   4. unchanged: correction + DLT of every matched keypoint pair, object_cost holds d.
+// This kernel repeats okp_stereo_objects_kernel's structure instead of sharing one inline body with it: that kernel's
+// body is left untouched, so its SASS stays what it was.
+// ---------------------------------------------------------------------------------------------
+struct OkpStereoLift {
+    double R[2][9];            // [0]: R_RL (a left lift into the right camera), [1]: R_LR = R_RL^T; row-major
+    double t[2][3];            // [0]: t_RL, [1]: t_LR = -R_RL^T t_RL
+};
+
+// okp_stereo_smem_bytes plus the projected lifts q of both frames, [2][O][P][2] doubles after the undistorted points
+__host__ __device__ inline size_t okp_stereo_depth_smem_bytes(int O, int C, int P) {
+    return okp_stereo_smem_bytes(O, C, P) + sizeof(double) * 2 * 2 * (size_t)O * P;
+}
+
+// q = pi(K (R X + t)) in the undistorted pixels of `cam`; NaN unless the lift is finite with z > 0
+__device__ __forceinline__ void okp_project_lift(const double* X, const double* R, const double* t, const OkpCamera& cam,
+                                                 double* q) {
+    const double x = X[0], y = X[1], z = X[2];
+    if (!(isfinite(x) && isfinite(y) && isfinite(z) && z > 0.0)) {
+        q[0] = q[1] = __longlong_as_double(0x7ff8000000000000LL);
+        return;
+    }
+    const double Y0 = R[0] * x + R[1] * y + R[2] * z + t[0];
+    const double Y1 = R[3] * x + R[4] * y + R[5] * z + t[1];
+    const double Y2 = R[6] * x + R[7] * y + R[8] * z + t[2];
+    q[0] = (cam.fx * Y0 + cam.cx * Y2) / Y2;
+    q[1] = (cam.fy * Y1 + cam.cy * Y2) / Y2;
+}
+
+// The cost of candidate (left keypoint: u_L, q_R; right keypoint: u_R, q_L): d when it passes the epipolar gate,
+// INFINITY otherwise; sets no_depth for a candidate inside the gate whose lifts are both missing.
+__device__ __forceinline__ double okp_depth_cost(const double* F, const double* uL, const double* qR, const double* uR,
+                                                 const double* qL, double max_distance, bool& no_depth) {
+    if (!(okp_epipolar_cost(F, uL[0], uL[1], uR[0], uR[1]) <= max_distance)) return INFINITY;
+    const bool has_r = qR[0] == qR[0], has_l = qL[0] == qL[0];
+    if (!has_r && !has_l) { no_depth = true; return INFINITY; }
+    double a = 0.0, b = 0.0;
+    if (has_r) { const double dx = qR[0] - uR[0], dy = qR[1] - uR[1]; a = sqrt(dx * dx + dy * dy); }
+    if (has_l) { const double dx = qL[0] - uL[0], dy = qL[1] - uL[1]; b = sqrt(dx * dx + dy * dy); }
+    return has_r && has_l ? 0.5 * (a + b) : (has_r ? a : b);
+}
+
+__global__ void __launch_bounds__(32)
+okp_stereo_depth_kernel(OkpStereoRig rig, OkpStereoLift lift, OkpStereoShape d, const int32_t* __restrict__ n_objects,
+                        const int32_t* __restrict__ kp_count, const float* __restrict__ kp_xy,
+                        const double* __restrict__ kp_point, const int32_t* __restrict__ pairs, double max_distance,
+                        double max_depth, int optimal_correction, OkpStereoTables out) {
+    extern __shared__ double s_xy[];                              // [2][O][P][2] undistorted points u
+    double* s_q = s_xy + 4 * d.O * d.P;                           // [2][O][P][2] lifts projected into the other view
+    double* s_cost = s_q + 4 * d.O * d.P;                         // [O][O] centre costs
+    double* s_slot_cost = s_cost + d.O * d.O;                     // [8][8] slot costs of one (object pair, type)
+    uint32_t* s_list = (uint32_t*)(s_slot_cost + OKP_MAX_SLOTS * OKP_MAX_SLOTS);   // matched keypoint pairs
+    int8_t* s_slot = (int8_t*)(s_list + d.O * d.P);               // [O][P] right slot of a left keypoint, -1
+    int8_t* s_object = s_slot + d.O * d.P;                        // [O] right object of a left object, -1
+    int8_t* s_count = s_object + d.O;                             // [2][O][C] keypoints kept
+    __shared__ unsigned long long s_used_left, s_used_right;
+    __shared__ int s_n_list;
+    const int p = blockIdx.x, lane = threadIdx.x;
+    const int O = d.O, C = d.C, S = d.S, P = d.P;
+    const int fl = pairs[2 * p], fr = pairs[2 * p + 1];
+    const bool bad = fl < 0 || fl >= d.N || fr < 0 || fr >= d.N;
+    const int nl = bad ? 0 : okp_clamp(n_objects[fl], 0, O), nr = bad ? 0 : okp_clamp(n_objects[fr], 0, O);
+    for (int e = lane; e < 2 * O * C; e += 32) {
+        const bool right = e >= O * C;
+        const int o = (e / C) % O, c = e % C;
+        s_count[e] = (int8_t)(o < (right ? nr : nl) ? okp_clamp(kp_count[((size_t)(right ? fr : fl) * O + o) * C + c], 0, d.cfg[c]) : 0);
+    }
+    for (int e = lane; e < O * P; e += 32) s_slot[e] = -1;
+    for (int o = lane; o < O; o += 32) {
+        s_object[o] = -1;
+        out.object_match[(size_t)p * O + o] = -1;
+        out.object_cost[(size_t)p * O + o] = 0.0;
+    }
+    if (lane == 0) { s_used_left = 0ull; s_used_right = 0ull; s_n_list = 0; }
+    __syncwarp();
+    // 1. undistortion, and every lift projected into the other view
+#pragma unroll
+    for (int v = 0; v < 2; ++v) {
+        const int f = v ? fr : fl;
+        for (int e = lane; e < (v ? nr : nl) * C * S; e += 32) {
+            const int o = e / (C * S), c = (e / S) % C, s = e % S;
+            if (s >= s_count[(v * O + o) * C + c]) continue;
+            const size_t at = (((size_t)f * O + o) * C + c) * S + s;
+            const int k = 2 * ((v * O + o) * P + d.off[c] + s);
+            okp_undistort_point((double)kp_xy[2 * at], (double)kp_xy[2 * at + 1], rig.cam[v], s_xy + k, s_xy + k + 1);
+            okp_project_lift(kp_point + 3 * at, lift.R[v], lift.t[v], rig.cam[1 - v], s_q + k);
+        }
+    }
+    __syncwarp();
+    // 2. objects by their centres
+    const double* L = s_xy;
+    const double* R = s_xy + 2 * O * P;
+    const double* QR = s_q;                                       // left keypoints' lifts in the right view
+    const double* QL = s_q + 2 * O * P;                           // right keypoints' lifts in the left view
+    bool no_depth = false;
+    for (int e = lane; e < nl * nr; e += 32) {
+        const int i = e / nr, j = e - i * nr;
+        s_cost[i * O + j] = okp_depth_cost(rig.F.m, L + 2 * i * P, QR + 2 * i * P, R + 2 * j * P, QL + 2 * j * P, max_distance,
+                                           no_depth);
+    }
+    __syncwarp();
+    bool ambiguous = false;                                       // two or more admissible right objects of one left object
+    for (int i = lane; i < nl; i += 32) {
+        int within = 0;
+        for (int j = 0; j < nr; ++j) within += s_cost[i * O + j] <= max_depth;
+        ambiguous |= within >= 2;
+    }
+    ambiguous = __any_sync(0xffffffffu, ambiguous);
+    okp_greedy_match(s_cost, O, nl, nr, max_depth, s_used_left, s_used_right, lane, [&](int i, int j, double cost) {
+        out.object_match[(size_t)p * O + i] = j;
+        out.object_cost[(size_t)p * O + i] = cost;
+        s_object[i] = (int8_t)j;
+        s_slot[i * P] = 0;
+        s_list[s_n_list++] = (uint32_t)i | (uint32_t)j << 8;      // left object, right object, map 0, slots 0
+    });
+    __syncwarp();
+    // 3. slots of every matched object pair, type by type
+    for (int i = 0; i < nl; ++i) {
+        const int j = s_object[i];
+        if (j < 0) continue;
+        for (int c = 1; c < C; ++c) {
+            const int nsl = s_count[i * C + c], nsr = s_count[(O + j) * C + c];
+            if (nsl == 0 || nsr == 0) continue;
+            const int kl = 2 * (i * P + d.off[c]), kr = 2 * (j * P + d.off[c]);
+            for (int e = lane; e < nsl * nsr; e += 32) {
+                const int a = e / nsr, b = e - a * nsr;
+                s_slot_cost[a * OKP_MAX_SLOTS + b] = okp_depth_cost(rig.F.m, L + kl + 2 * a, QR + kl + 2 * a, R + kr + 2 * b,
+                                                                    QL + kr + 2 * b, max_distance, no_depth);
+            }
+            if (lane == 0) { s_used_left = 0ull; s_used_right = 0ull; }
+            __syncwarp();
+            okp_greedy_match(s_slot_cost, OKP_MAX_SLOTS, nsl, nsr, max_depth, s_used_left, s_used_right, lane,
+                             [&](int a, int b, double) {
+                s_slot[i * P + d.off[c] + a] = (int8_t)b;
+                s_list[s_n_list++] = (uint32_t)i | (uint32_t)j << 8 | (uint32_t)c << 16 | (uint32_t)a << 20 | (uint32_t)b << 24;
+            });
+            __syncwarp();
+        }
+    }
+    no_depth = __any_sync(0xffffffffu, no_depth);
+    // slot_match for every slot; NaN points where nothing is matched
+    const double nan = __longlong_as_double(0x7ff8000000000000LL);
+    for (int e = lane; e < O * C * S; e += 32) {
+        const int o = e / (C * S), c = (e / S) % C, s = e % S;
+        const int m = s < d.cfg[c] ? s_slot[o * P + d.off[c] + s] : -1;
+        const size_t at = (size_t)p * O * C * S + e;
+        out.slot_match[at] = m;
+        if (m < 0) { out.point[3 * at] = nan; out.point[3 * at + 1] = nan; out.point[3 * at + 2] = nan; }
+    }
+    // 4. correction + DLT of every matched keypoint pair
+    for (int e = lane; e < s_n_list; e += 32) {
+        const uint32_t w = s_list[e];
+        const int i = w & 255, j = (w >> 8) & 255, c = (w >> 16) & 15, a = (w >> 20) & 15, b = w >> 24;
+        const double* l = L + 2 * (i * P + d.off[c] + a);
+        const double* r = R + 2 * (j * P + d.off[c] + b);
+        double x[2][2] = {{(double)(float)l[0], (double)(float)l[1]}, {(double)(float)r[0], (double)(float)r[1]}};
+        if (optimal_correction) {
+            okp_correct_pair(rig.F, rig.ep, x[0][0], x[0][1], x[1][0], x[1][1], x[0], x[1]);
+#pragma unroll
+            for (int v = 0; v < 2; ++v) { x[v][0] = (double)(float)x[v][0]; x[v][1] = (double)(float)x[v][1]; }
+        }
+        double A[4][4] = {};
+#pragma unroll
+        for (int v = 0; v < 2; ++v) {
+            const double* M = rig.proj[v];
+            double row[4];
+#pragma unroll
+            for (int k = 0; k < 4; ++k) row[k] = x[v][0] * M[8 + k] - M[k];
+            okp_givens_append(A, row);
+#pragma unroll
+            for (int k = 0; k < 4; ++k) row[k] = x[v][1] * M[8 + k] - M[4 + k];
+            okp_givens_append(A, row);
+        }
+        double h[4];
+        okp_smallest_right_singular_vector(A, h);
+        double* X = out.point + 3 * ((((size_t)p * O + i) * C + c) * S + a);
+        X[0] = h[0] / h[3]; X[1] = h[1] / h[3]; X[2] = h[2] / h[3];
+    }
+    if (lane == 0)
+        out.flags[p] = (bad ? OKP_STEREO_BAD_PAIR : 0u) | (ambiguous ? OKP_STEREO_AMBIGUOUS : 0u) |
+                       (no_depth ? OKP_STEREO_NO_DEPTH : 0u);
+}

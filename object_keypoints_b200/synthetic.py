@@ -353,7 +353,8 @@ def _epipolar_distance(F, left, right):
 
 
 def stereo_batch(P, keypoint_config, size, stereo, seed, objects=(1, 4), depth_range=(0.5, 1.2), centre_margin=5.0, slot_margin=1.0,
-                 center_separation=22.0, spoke_radius=(5.0, 8.0), peak_separation=6.0, border=4.0, max_tries=5000):
+                 center_separation=22.0, spoke_radius=(5.0, 8.0), peak_separation=6.0, border=4.0, max_tries=5000,
+                 same_row=False, row_jitter=0.0, depth_scale=0.0):
     """P stereo pairs of one rig. Per pair: objects (a centre and keypoint_config[t] keypoints of every type t) are placed
     in front of the rig: pixels and depths are sampled in the left view under sample_scene's separations, lifted to 3D
     and projected into the right view with FisheyeCamera.project; the right view must keep the centres' separation too.
@@ -361,7 +362,15 @@ def stereo_batch(P, keypoint_config, size, stereo, seed, objects=(1, 4), depth_r
     ambiguous at max_distance_px < centre_margin), and two different keypoints of one object and type farther than
     slot_margin (the construction's matching is the greedy one on noiseless keypoints). Each view is
     rasterised with `rasterize`, z taken in that view's camera frame; the objects of a view are listed in raster order of
-    their centre pixel, the order in which the decode finds them."""
+    their centre pixel, the order in which the decode finds them.
+    same_row: every object of a pair is moved vertically, with its keypoints, so that its centre lies in the row of the
+    first object's centre in the left view, give or take a uniform row_jitter (pixels): parts side by side on a table,
+    on one epipolar line of this rig. The centre_margin check is skipped then (slot_margin still applies), the left
+    view must keep sample_scene's separations, and every keypoint's depth must be readable where the decode lifts it:
+    DetectionToPoint reads the depth map at the undistorted pixel, which near the edges of a wide view lies off the disc
+    drawn around the distorted one. depth_scale: each (frame, map) depth map is multiplied by its own factor,
+    uniform in [1 - depth_scale, 1 + depth_scale] (a biased depth head); the ground truth is not. Both are off by
+    default and then draw nothing, so the batches of other arguments do not change."""
     H, W = size
     cams = (stereo.left_camera, stereo.right_camera)
     T = (np.eye(4), stereo.T_RL)
@@ -381,6 +390,12 @@ def stereo_batch(P, keypoint_config, size, stereo, seed, objects=(1, 4), depth_r
         for _ in range(max_tries):
             left = sample_scene(rng, keypoint_config, size, n_obj, center_separation, spoke_radius, peak_separation, border)
             px_l = np.concatenate([left.centers[:, None]] + list(left.spokes), axis=1)        # [n_obj, n_kp, 2]
+            if same_row:
+                row = px_l[0, 0, 1] + rng.uniform(-row_jitter, row_jitter, size=n_obj)
+                px_l[:, :, 1] += (row - px_l[:, 0, 1])[:, None]
+                if not (all(inside(v) for v in px_l.reshape(-1, 2)) and
+                        _separated(px_l, keypoint_config, center_separation, peak_separation)):
+                    continue
             z = rng.uniform(*depth_range, size=n_obj)[:, None] + rng.uniform(-0.03, 0.03, size=(n_obj, n_kp))
             und = cams[0].undistort(px_l.reshape(-1, 2))
             X = (np.concatenate([und, np.ones((und.shape[0], 1))], axis=1) @ cams[0].Kinv.T) * z.reshape(-1, 1)
@@ -390,7 +405,9 @@ def stereo_batch(P, keypoint_config, size, stereo, seed, objects=(1, 4), depth_r
             if not _far_enough_all(views[1][:, 0], center_separation):
                 continue
             und_views = [c.undistort(v.reshape(-1, 2)).reshape(n_obj, n_kp, 2) for c, v in zip(cams, views)]
-            if not _epipolar_unique(stereo.F, und_views, keypoint_config, centre_margin, slot_margin):
+            if not _epipolar_unique(stereo.F, und_views, keypoint_config, -1.0 if same_row else centre_margin, slot_margin):
+                continue
+            if same_row and not all(_lift_on_disc(u, v) for u, v in zip(und_views, views)):
                 continue
             break
         else:
@@ -416,8 +433,69 @@ def stereo_batch(P, keypoint_config, size, stereo, seed, objects=(1, 4), depth_r
         rank_right[orders[1]] = np.arange(n_obj)
         right_of_left.append(rank_right[orders[0]])
         pixels.append((views[0][orders[0]], views[1][orders[1]]))
+    if depth_scale:
+        scale = np.random.default_rng([seed, 1]).uniform(1.0 - depth_scale, 1.0 + depth_scale, size=depth.shape[:2])
+        depth *= scale[:, :, None, None].astype(np.float32)
     batch = Batch(heat=heat, depth=depth, centers=centers, scenes=scenes, keypoint_config=list(keypoint_config))
     return StereoBatch(batch=batch, points=points, right_of_left=right_of_left, pixels=pixels)
+
+
+def stereo_match_errors(sb, tables, result):
+    """A stereo-objects result scored against the construction -> (wrong object matches, wrong slot matches, largest
+    relative error of a correctly matched point). tables: the decode tables of sb.batch (n_objects, kp_count, kp_xy;
+    NumPy), result: the StereoTables of the interleaved pairs (NumPy). Decoded objects and slots are identified with the
+    construction's by their nearest pixel in each view: the decode lists objects in raster order of their peak pixel,
+    which for objects in one row need not be the construction's order."""
+    cfg = sb.batch.keypoint_config
+    wrong_objects = wrong_slots = 0
+    worst = 0.0
+    groups = np.cumsum([0, 1] + list(cfg))
+
+    def nearest(xy, pixels):
+        return int(np.linalg.norm(pixels - xy[None], axis=-1).argmin())
+    for p, (perm, X) in enumerate(zip(sb.right_of_left, sb.points)):
+        px_l, px_r = sb.pixels[p]
+        for i in range(int(tables['n_objects'][2 * p])):
+            a = nearest(tables['kp_xy'][2 * p, i, 0, 0], px_l[:, 0])
+            j = int(result['object_match'][p, i])
+            if j < 0 or nearest(tables['kp_xy'][2 * p + 1, j, 0, 0], px_r[:, 0]) != perm[a]:
+                wrong_objects += 1
+                continue
+            for c in range(len(cfg) + 1):
+                k0, k1 = groups[c], groups[c + 1]
+                for s in range(int(tables['kp_count'][2 * p, i, c])):
+                    k = k0 + nearest(tables['kp_xy'][2 * p, i, c, s], px_l[a, k0:k1])
+                    m = int(result['slot_match'][p, i, c, s])
+                    if m < 0 or k0 + nearest(tables['kp_xy'][2 * p + 1, j, c, m], px_r[perm[a], k0:k1]) != k:
+                        wrong_slots += 1
+                        continue
+                    error = np.linalg.norm(result['point'][p, i, c, s] - X[a, k]) / np.linalg.norm(X[a, k])
+                    worst = max(worst, float(error))
+    return wrong_objects, wrong_slots, worst
+
+
+def _lift_on_disc(undistorted, distorted, radius=DISC_RADIUS - 0.5):
+    """The pixel DetectionToPoint reads for every keypoint (the rounded undistorted position) lies inside the keypoint's
+    depth disc (drawn around the distorted position, pixel centres at +0.5), with half a pixel to spare."""
+    read = np.rint(undistorted.reshape(-1, 2)) + 0.5
+    return bool((np.linalg.norm(read - distorted.reshape(-1, 2), axis=1) < radius).all())
+
+
+def _separated(px, keypoint_config, center_separation, peak_separation):
+    """sample_scene's separations on keypoints [n_obj, 1 + sum(cfg), 2]: centres, same-map peaks, and every spoke nearer
+    to its own centre than to any other."""
+    if not _far_enough_all(px[:, 0], center_separation):
+        return False
+    k = 1
+    for count in keypoint_config:
+        spokes = px[:, k:k + count]
+        if not _far_enough_all(spokes.reshape(-1, 2), peak_separation):
+            return False
+        own = np.linalg.norm(spokes[:, :, None] - px[None, None, :, 0], axis=-1).argmin(axis=-1)     # [n_obj, count]
+        if not (own == np.arange(len(px))[:, None]).all():
+            return False
+        k += count
+    return True
 
 
 def _far_enough_all(points, min_distance):

@@ -235,7 +235,12 @@ class TriangulationComponent:
                                   optimal_correction=self.optimal_correction)
 
 
-def triangulate_stereo_objects(tables, stereo, pairs=None, max_distance_px=2.5, optimal_correction=True, stream=None):
+STEREO_ASSOCIATIONS = ('epipolar', 'depth')
+DEFAULT_MAX_DEPTH_PX = 8.0      # DESIGN.md section 3: admits a +-25 % depth error at z >= 0.5 m on the ZED Mini rig
+
+
+def triangulate_stereo_objects(tables, stereo, pairs=None, max_distance_px=2.5, optimal_correction=True, stream=None,
+                               association='epipolar', max_depth_px=DEFAULT_MAX_DEPTH_PX):
     """The decoded objects of stereo frame pairs, matched across the two views and triangulated, on the device
     (okp_triangulate_stereo_objects_f64). tables: the DecodeTables of a batch that holds both views of every pair (decode
     it with ``camera_table((stereo.left_camera, stereo.right_camera), ...)`` so that each view is lifted with its own
@@ -244,8 +249,21 @@ def triangulate_stereo_objects(tables, stereo, pairs=None, max_distance_px=2.5, 
     Per pair: objects are matched by the epipolar distance of their undistorted centres, greedily one to one while it is
     <= max_distance_px (AssociationComponent's rule), then each matched object pair's slots type by type; every matched
     keypoint pair is triangulated like StereoCamera.triangulate (optimal_correction: the Hartley-Sturm correction).
-    Returns StereoTables on the tables' device: object_match, object_cost, slot_match, point (left camera frame, NaN where
-    nothing is matched), flags (_abi.STEREO_AMBIGUOUS, _abi.STEREO_BAD_PAIR). Asynchronous: nothing synchronises."""
+    association='depth' (okp_triangulate_stereo_objects_depth_f64) tells apart objects on one epipolar line, such as
+    parts side by side in the same image rows: each keypoint's lift (kp_point) is projected into the other view, and the
+    greedy step runs on the mean distance d between those predictions and the other view's keypoints, over the
+    candidates within max_distance_px of the epipolar line and with d <= max_depth_px. It needs lifts taken at the right
+    pixel: ValueError when the tables were decoded with compat_clip_bug and a camera's image is not square.
+    Returns StereoTables on the tables' device: object_match, object_cost (d with association='depth'), slot_match,
+    point (left camera frame, NaN where nothing is matched), flags (_abi.STEREO_AMBIGUOUS, _abi.STEREO_BAD_PAIR,
+    _abi.STEREO_NO_DEPTH). Asynchronous: nothing synchronises."""
+    if association not in STEREO_ASSOCIATIONS:
+        raise ValueError(f"association must be one of {STEREO_ASSOCIATIONS}, got {association!r}")
+    if association == 'depth':
+        sizes = [np.asarray(c.image_size).reshape(-1)[:2] for c in (stereo.left_camera, stereo.right_camera)]
+        if tables.params.compat_clip_bug and any(s[0] != s[1] for s in sizes):
+            raise ValueError("association='depth' reads kp_point, and with compat_clip_bug a non-square image is lifted with "
+                             "the depth of a clipped column: decode with compat_clip_bug=False")
     N = tables.N
     device = tables.flat.device
     if pairs is None:
@@ -261,11 +279,19 @@ def triangulate_stereo_objects(tables, stereo, pairs=None, max_distance_px=2.5, 
     left, right = _abi.pack_camera(stereo.left_camera), _abi.pack_camera(stereo.right_camera)
     F, P_L, P_R = (np.ascontiguousarray(m, dtype=np.float64) for m in (stereo.F, *stereo.projection_matrices()))
     doubles = ctypes.POINTER(ctypes.c_double)
+    head = (ctypes.byref(tables.struct), N, C, cfg, ctypes.byref(tables.params), pairs_dev.data_ptr(), P, ctypes.byref(left),
+            ctypes.byref(right), F.ctypes.data_as(doubles), P_L.ctypes.data_as(doubles), P_R.ctypes.data_as(doubles))
     with torch.cuda.device(device):
-        rc = _lib.lib().okp_triangulate_stereo_objects_f64(
-            ctypes.byref(tables.struct), N, C, cfg, ctypes.byref(tables.params), pairs_dev.data_ptr(), P, ctypes.byref(left),
-            ctypes.byref(right), F.ctypes.data_as(doubles), P_L.ctypes.data_as(doubles), P_R.ctypes.data_as(doubles),
-            float(max_distance_px), int(bool(optimal_correction)), ctypes.byref(out.struct), _stream_handle(stream))
-    _lib.check(rc, 'okp_triangulate_stereo_objects_f64')
+        if association == 'depth':
+            name = 'okp_triangulate_stereo_objects_depth_f64'
+            T_RL = np.ascontiguousarray(stereo.T_RL, dtype=np.float64).reshape(16)
+            rc = _lib.lib().okp_triangulate_stereo_objects_depth_f64(
+                *head, T_RL.ctypes.data_as(doubles), float(max_distance_px), float(max_depth_px),
+                int(bool(optimal_correction)), ctypes.byref(out.struct), _stream_handle(stream))
+        else:
+            name = 'okp_triangulate_stereo_objects_f64'
+            rc = _lib.lib().okp_triangulate_stereo_objects_f64(
+                *head, float(max_distance_px), int(bool(optimal_correction)), ctypes.byref(out.struct), _stream_handle(stream))
+    _lib.check(rc, name)
     out.pairs = pairs_dev                                 # the launch reads it: kept alive with the result
     return out
