@@ -438,6 +438,50 @@ int okp_triangulate_stereo_objects_depth_f64(const OkpDecodeTables* tables, int 
                                              double max_distance_px, double max_depth_px, int optimal_correction,
                                              const OkpStereoTables* out, void* stream);
 
+/* Sequence objects: the decoded objects of a sequence filmed by one moving camera with known poses (BASELINE config 3),
+ * each anchor frame's objects matched into its V - 1 view frames and every anchor keypoint triangulated over the views
+ * in the world frame. A anchors, O = max_objects, S = max(1, max(keypoint_config)); all arrays are device memory, dense
+ * row-major with the shapes given, and every entry is written. */
+typedef struct OkpSequenceObjectTables {
+    int32_t* object_match;  /* [A,V-1,O]       object of view frame v + 1 matched to anchor object o, -1 */
+    double*  object_cost;   /* [A,V-1,O]       cost of that match (epipolar cost, or d with depth association), 0 where none */
+    int32_t* slot_match;    /* [A,V-1,O,C,S]   matched object's slot for anchor slot s, -1 */
+    uint32_t* flags;        /* [A,V-1]         OKP_STEREO_* of the pair (anchor, view v + 1) */
+    double*  observations;  /* [A,O,C,S,V,2]   track of every anchor slot: view 0 the anchor's keypoint, view v its match in
+                               view frame v; kp_xy (distorted pixels), 0 where there is none */
+    uint8_t* valid;         /* [A,O,C,S,V]     observed, after the reprojection filter */
+    uint8_t* observed;      /* [A,O,C,S,V]     1 where the track has an observation */
+    double*  point;         /* [A,O,C,S,3]     world frame, NaN where fewer than two views are valid */
+    double*  error;         /* [A,O,C,S,V]     reprojection error (pixels) against the final point; NaN for a track with
+                               fewer than two observations */
+    int32_t* dropped;       /* [A,O,C,S]       views dropped by the reprojection filter */
+} OkpSequenceObjectTables;
+
+/* For every anchor a and view v in [1, V): the pair (anchor frame frames_dev[a,0], view frame frames_dev[a,v]) of `tables`
+ * (N frames decoded with C maps, keypoint_config and params, all with `camera`; lean tables or cleared ones, only valid
+ * slots are read) is matched like a stereo pair of okp_triangulate_stereo_objects_f64 (association 0: epipolar cost under
+ * F_dev[a,v-1], <= max_distance_px) or of okp_triangulate_stereo_objects_depth_f64 (association 1: kp_point lifts projected
+ * with the pair's rigid motion, epipolar gate, then d <= max_depth_px), anchor frame as the left view: objects by their
+ * centres, then each matched object pair's slots type by type; same costs, tie rule and flags. Every anchor slot's matches
+ * form a track of V views, which okp_triangulate_tracks_f64 solves with G = A groups of O*C*S tracks: undistortion, V-view
+ * DLT with the poses poses_dev[a], reprojection filter with max_error_px and max_rounds, world-frame points.
+ * frames_dev: DEVICE int32 [A,V]. F_dev: DEVICE [A,V-1,3,3] row-major, x_view^T F x_anchor = 0 for undistorted pixels.
+ * motion_dev: DEVICE [A,V-1,2,12]: (R row-major, t) of T = T_CW[view] T_CW[anchor]^-1 (anchor camera -> view camera), then
+ * (R^T, -R^T t); read with association 1 only (may be NULL otherwise). poses_dev: DEVICE [A,V,4,4] world -> camera of the
+ * frames. A pair with a frame index outside [0, N) gets OKP_STEREO_BAD_PAIR and matches nothing (column 0 still holds the
+ * anchor's keypoints when the anchor frame is in range). A = 0 returns OKP_OK. Refused on the host, before any CUDA call:
+ * NULL pointers (OKP_E_NULL; with association 1 also NULL motion_dev or tables->kp_point); association not 0 or 1
+ * (OKP_E_UNSUPPORTED); N < 0, A < 0, C out of range, max_objects > 64, 1 + sum(keypoint_config) > 64, V < 2, V > 64,
+ * A > 65535, A * O * C * S > 2^31 - 1, max_rounds < 0, a max_depth_px (association 1) not finite or <= 0, or a shape whose
+ * shared memory, 8 (8 O P + O^2 + 64) + O P + O + 2 O C bytes with P = 1 + sum(keypoint_config), exceeds sm_100's 227 KB
+ * per-block limit (OKP_E_SHAPE). */
+int okp_triangulate_sequence_objects_f64(const OkpDecodeTables* tables, int N, int C, const int32_t* keypoint_config,
+                                         const OkpDecodeParams* params, const int32_t* frames_dev, int A, int V,
+                                         const double* F_dev, const double* motion_dev, const double* poses_dev,
+                                         const OkpCamera* camera, int association, double max_distance_px,
+                                         double max_depth_px, double max_error_px, int max_rounds,
+                                         const OkpSequenceObjectTables* out, void* stream);
+
 /* Evaluation bookkeeping (SURVEY section 8f rank 3). Replaces Results.add of the reference's
  * scripts/eval_model.py:141-187 for a batch of N frames, reading the decode tables in place:
  * kp_point_dev [N,O,C,S,3], kp_count_dev [N,O,C], n_objects_dev [N] (OkpDecodeTables fields), T_WC_dev

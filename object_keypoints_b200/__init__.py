@@ -10,7 +10,7 @@ ethz-asl/object_keypoints, behind the reference's pipeline API.
 Importing the package does not need a GPU; constructing a pipeline does (no CPU fallback).
 """
 from . import camera_utils, linalg                                   # noqa: F401
-from .pipeline import (CameraTable, DecodeTables, StereoTables, KeypointDecoder, InferenceComponent, KeypointExtractionComponent,   # noqa: F401
+from .pipeline import (CameraTable, DecodeTables, StereoTables, SequenceObjectTables, KeypointDecoder, InferenceComponent, KeypointExtractionComponent,   # noqa: F401
                        ObjectExtraction, DetectionToPoint, ObjectKeypointPipeline,
                        LearnedKeypointTrackingPipeline, tables_to_objects, tables_to_keypoints)
 from .triangulation import (TriangulationComponent, triangulate, triangulate_multiview, triangulate_stereo,   # noqa: F401

@@ -88,6 +88,25 @@ class OkpStereoTables(ctypes.Structure):
     _fields_ = [(name, ctypes.c_void_p) for name, _, _ in STEREO_LAYOUT]
 
 
+# OkpSequenceObjectTables: name, numpy dtype, shape as a function of (A, V, O, C, S) -- order = field order in okp.h
+SEQUENCE_LAYOUT = [
+    ('object_match', np.int32, lambda A, V, O, C, S: (A, V - 1, O)),
+    ('object_cost', np.float64, lambda A, V, O, C, S: (A, V - 1, O)),
+    ('slot_match', np.int32, lambda A, V, O, C, S: (A, V - 1, O, C, S)),
+    ('flags', np.uint32, lambda A, V, O, C, S: (A, V - 1)),
+    ('observations', np.float64, lambda A, V, O, C, S: (A, O, C, S, V, 2)),
+    ('valid', np.uint8, lambda A, V, O, C, S: (A, O, C, S, V)),
+    ('observed', np.uint8, lambda A, V, O, C, S: (A, O, C, S, V)),
+    ('point', np.float64, lambda A, V, O, C, S: (A, O, C, S, 3)),
+    ('error', np.float64, lambda A, V, O, C, S: (A, O, C, S, V)),
+    ('dropped', np.int32, lambda A, V, O, C, S: (A, O, C, S)),
+]
+
+
+class OkpSequenceObjectTables(ctypes.Structure):
+    _fields_ = [(name, ctypes.c_void_p) for name, _, _ in SEQUENCE_LAYOUT]
+
+
 def check_pairs(pairs, N):
     """Frame pairs of okp_triangulate_stereo_objects_f64: [P, 2] integers (left frame, right frame) in [0, N) -> int32
     array. The library reads the frames they name, so they are checked here, like pack_camera_table checks its indices:

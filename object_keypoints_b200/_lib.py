@@ -25,7 +25,7 @@ EXPORTS = [
     'okp_extract_peaks_f16', 'okp_group_objects_f16', 'okp_decode_f16', 'okp_decode_emit_f16', 'okp_group_objects_emit_f16',
     'okp_decode_cameras_f32', 'okp_decode_cameras_bf16', 'okp_decode_cameras_f16',
     'okp_group_objects_cameras_f32', 'okp_group_objects_cameras_bf16', 'okp_group_objects_cameras_f16',
-    'okp_triangulate_stereo_objects_f64', 'okp_triangulate_stereo_objects_depth_f64',
+    'okp_triangulate_stereo_objects_f64', 'okp_triangulate_stereo_objects_depth_f64', 'okp_triangulate_sequence_objects_f64',
 ]
 
 
@@ -168,6 +168,10 @@ def lib():
                                                            P(_abi.OkpDecodeParams), vp, i32, P(_abi.OkpCamera),
                                                            P(_abi.OkpCamera), P(dbl), P(dbl), P(dbl), P(dbl), dbl, dbl, i32,
                                                            P(_abi.OkpStereoTables), vp]
+    L.okp_triangulate_sequence_objects_f64.restype = i32
+    L.okp_triangulate_sequence_objects_f64.argtypes = [P(_abi.OkpDecodeTables), i32, i32, P(ctypes.c_int32),
+                                                       P(_abi.OkpDecodeParams), vp, i32, i32, vp, vp, vp, P(_abi.OkpCamera),
+                                                       i32, dbl, dbl, dbl, i32, P(_abi.OkpSequenceObjectTables), vp]
     L.okp_eval_match_f64.restype = i32
     L.okp_eval_match_f64.argtypes = [vp, vp, vp, vp, vp, i32, i32, i32, i32, i32, i32, P(_abi.OkpCamera), dbl, dbl, dbl, dbl,
                                      vp, vp, vp, vp, vp, vp, vp]

@@ -12,6 +12,7 @@
 #include "okp_group.cuh"
 #include "okp_dlt.cuh"
 #include "okp_stereo.cuh"
+#include "okp_sequence.cuh"
 #include "okp_eval.cuh"
 #include "okp_records.cuh"
 #include "okp_targets.cuh"
@@ -684,17 +685,9 @@ int okp_associate_pairs_f64(const double* F_dev, const double* left_dev, const i
     return OKP_OK;
 }
 
-// The host checks and set-up both stereo-objects entries share (after their P = 0 return): NULL pointers, the shape, the rig.
-static int okp_stereo_prepare(const OkpDecodeTables* tables, int N, int C, const int32_t* keypoint_config,
-                              const OkpDecodeParams* params, const int32_t* pairs_dev, const OkpCamera* left_camera,
-                              const OkpCamera* right_camera, const double* F, const double* P_L, const double* P_R,
-                              const OkpStereoTables* out, OkpStereoShape* shape, OkpStereoRig* rig_out) {
-    if (!tables || !params || (C > 1 && !keypoint_config) || !pairs_dev || !left_camera || !right_camera || !F || !P_L ||
-        !P_R || !out)
-        return OKP_E_NULL;
-    if (!tables->n_objects || !tables->kp_count || !tables->kp_xy || !out->object_match || !out->object_cost ||
-        !out->slot_match || !out->point || !out->flags)
-        return OKP_E_NULL;
+// The object shape the stereo and sequence entries share (params and, for C > 1, keypoint_config checked for NULL):
+// O = max_objects and P = 1 + sum(keypoint_config) up to 64, for the greedy step's 64-bit masks.
+static int okp_objects_shape(int N, int C, const int32_t* keypoint_config, const OkpDecodeParams* params, OkpStereoShape* shape) {
     OkpStereoShape& d = *shape;
     memset(&d, 0, sizeof(d));
     d.N = N; d.C = C; d.O = params->max_objects;
@@ -709,6 +702,22 @@ static int okp_stereo_prepare(const OkpDecodeTables* tables, int N, int C, const
         if (k > d.S) d.S = k;
     }
     if (d.P > 64) return OKP_E_SHAPE;
+    return OKP_OK;
+}
+
+// The host checks and set-up both stereo-objects entries share (after their P = 0 return): NULL pointers, the shape, the rig.
+static int okp_stereo_prepare(const OkpDecodeTables* tables, int N, int C, const int32_t* keypoint_config,
+                              const OkpDecodeParams* params, const int32_t* pairs_dev, const OkpCamera* left_camera,
+                              const OkpCamera* right_camera, const double* F, const double* P_L, const double* P_R,
+                              const OkpStereoTables* out, OkpStereoShape* shape, OkpStereoRig* rig_out) {
+    if (!tables || !params || (C > 1 && !keypoint_config) || !pairs_dev || !left_camera || !right_camera || !F || !P_L ||
+        !P_R || !out)
+        return OKP_E_NULL;
+    if (!tables->n_objects || !tables->kp_count || !tables->kp_xy || !out->object_match || !out->object_cost ||
+        !out->slot_match || !out->point || !out->flags)
+        return OKP_E_NULL;
+    const int rc = okp_objects_shape(N, C, keypoint_config, params, shape);
+    if (rc != OKP_OK) return rc;
     OkpStereoRig& rig = *rig_out;
     rig.cam[0] = *left_camera;
     rig.cam[1] = *right_camera;
@@ -769,6 +778,41 @@ int okp_triangulate_stereo_objects_depth_f64(const OkpDecodeTables* tables, int 
                                                                    max_depth_px, optimal_correction, *out);
     OKP_CUDA_CHECK(cudaGetLastError());
     return OKP_OK;
+}
+
+int okp_triangulate_sequence_objects_f64(const OkpDecodeTables* tables, int N, int C, const int32_t* keypoint_config,
+                                         const OkpDecodeParams* params, const int32_t* frames_dev, int A, int V,
+                                         const double* F_dev, const double* motion_dev, const double* poses_dev,
+                                         const OkpCamera* camera, int association, double max_distance_px,
+                                         double max_depth_px, double max_error_px, int max_rounds,
+                                         const OkpSequenceObjectTables* out, void* stream) {
+    if (N < 0 || A < 0 || C < 1 || C > OKP_MAX_MAPS) return OKP_E_SHAPE;
+    if (A == 0) return OKP_OK;
+    if (!tables || !params || (C > 1 && !keypoint_config) || !frames_dev || !F_dev || !poses_dev || !camera || !out)
+        return OKP_E_NULL;
+    if (!tables->n_objects || !tables->kp_count || !tables->kp_xy || !out->object_match || !out->object_cost ||
+        !out->slot_match || !out->flags || !out->observations || !out->valid || !out->observed || !out->point ||
+        !out->error || !out->dropped)
+        return OKP_E_NULL;
+    if (association != 0 && association != 1) return OKP_E_UNSUPPORTED;
+    if (association == 1 && (!motion_dev || !tables->kp_point)) return OKP_E_NULL;
+    OkpStereoShape d;
+    const int rc = okp_objects_shape(N, C, keypoint_config, params, &d);
+    if (rc != OKP_OK) return rc;
+    // the track kernel's limits (okp_triangulate_tracks_f64), checked here so that nothing is launched before a refusal
+    const int Pg = d.O * d.C * d.S;
+    if (V < 2 || V > OKP_MAX_VIEWS || max_rounds < 0 || A > 65535 || (long long)A * Pg > 0x7fffffffLL) return OKP_E_SHAPE;
+    if (association == 1 && !(max_depth_px > 0.0 && max_depth_px < INFINITY)) return OKP_E_SHAPE;     // NaN fails both
+    const size_t smem = okp_sequence_smem_bytes(d.O, d.C, d.P);
+    if (smem > 227 * 1024) return OKP_E_SHAPE;                        // sm_100's per-block opt-in shared memory
+    if (smem > 48 * 1024)
+        OKP_CUDA_CHECK(cudaFuncSetAttribute(okp_sequence_match_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    okp_sequence_match_kernel<<<A * (V - 1), 32, smem, (cudaStream_t)stream>>>(
+        *camera, d, V, tables->n_objects, tables->kp_count, tables->kp_xy, tables->kp_point, frames_dev, F_dev,
+        association == 1 ? motion_dev : nullptr, association, max_distance_px, max_depth_px, *out);
+    OKP_CUDA_CHECK(cudaGetLastError());
+    return okp_triangulate_tracks_f64(out->observations, out->valid, poses_dev, camera, A, Pg, V, max_error_px, max_rounds,
+                                      out->point, out->error, out->dropped, stream);
 }
 
 int okp_eval_match_f64(const double* kp_point_dev, const int32_t* kp_count_dev, const int32_t* n_objects_dev,

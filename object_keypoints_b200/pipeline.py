@@ -21,7 +21,7 @@ import torch
 from . import _abi, _lib
 
 _TORCH_DTYPES = {np.dtype(np.int32): torch.int32, np.dtype(np.uint32): torch.int32,
-                 np.dtype(np.float32): torch.float32, np.dtype(np.float64): torch.float64}
+                 np.dtype(np.float32): torch.float32, np.dtype(np.float64): torch.float64, np.dtype(np.uint8): torch.uint8}
 
 
 def _device(device=None):
@@ -131,6 +131,19 @@ class StereoTables(_TableSet):
         self.P = P
         super().__init__([(name, dtype, shape(P, O, C, S)) for name, dtype, shape in _abi.STEREO_LAYOUT],
                          _abi.OkpStereoTables, device)
+
+
+class SequenceObjectTables(_TableSet):
+    """The OkpSequenceObjectTables record of SequenceTriangulator.objects as torch tensors on one device, in one
+    allocation: per (anchor, view) pair object_match / object_cost [A,V-1,O], slot_match [A,V-1,O,C,S], flags [A,V-1]
+    (_abi.STEREO_*); per anchor slot a track of V views, observations [A,O,C,S,V,2] (distorted pixels; view 0 is the
+    anchor's own keypoint), observed / valid [A,O,C,S,V] (before / after the reprojection filter), error [A,O,C,S,V],
+    dropped [A,O,C,S], and point [A,O,C,S,3] in the world frame (NaN where fewer than two views are valid)."""
+
+    def __init__(self, A, V, O, C, S, device):
+        self.A, self.V = A, V
+        super().__init__([(name, dtype, shape(A, V, O, C, S)) for name, dtype, shape in _abi.SEQUENCE_LAYOUT],
+                         _abi.OkpSequenceObjectTables, device)
 
 
 class CameraTable:

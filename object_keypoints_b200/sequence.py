@@ -13,6 +13,12 @@ This module is the chain for a whole decoded sequence, everything on the device:
       -> tracks [A, C*K, V]                                                   observation of anchor peak k in every view
       -> okp_triangulate_tracks_f64                                           V-view DLT + reprojection filter + re-solve
 
+``SequenceTriangulator.objects`` is the same chain on the decode tables' objects instead of raw peaks: each anchor frame's
+objects are matched into its view frames (by epipolar distance, or by where each frame's depth lift lands in the other
+frame), slot by slot, and every anchor keypoint becomes a track of V views, all in one matching kernel
+(okp_triangulate_sequence_objects_f64) followed by the same robust track kernel. Its result says which object and slot
+each world point belongs to.
+
 Frames are taken in ``views`` strides: anchor a in [0, N // views) is seen again in frames a + v * (N // views).
 The synthetic sequence (``synthetic_sequence``) follows SURVEY.md section 8d #3: 900 frames of 180x320, 8 valves on a
 4 x 2 grid, camera on a spherical cap r in [0.6, 1.0] m looking at the workspace.
@@ -23,7 +29,7 @@ import numpy as np
 import torch
 
 from . import _abi, _lib, camera_utils, linalg
-from .pipeline import _device, _stream_handle
+from .pipeline import SequenceObjectTables, _device, _stream_handle
 
 
 def synthetic_sequence(n_frames=900, keypoint_config=(1, 3), grid=(4, 2), spacing=0.22, seed=1003):
@@ -104,6 +110,47 @@ def pair_fundamentals(camera, T_CW, frames):
     return F
 
 
+def pair_motions(T_CW, frames):
+    """motion [A, V-1, 2, 12]: for each (anchor, view) pair the rigid motion T = T_CW[view] inv(T_CW[anchor]) (anchor camera ->
+    view camera; the T_RL of pair_fundamentals) as (R row-major, t), then its inverse as (R^T, -R^T t), the inverse formed
+    in the operation order okp_triangulate_stereo_objects_depth_f64 uses for T_RL."""
+    A, V = frames.shape
+    motion = np.zeros((A, V - 1, 2, 12))
+    for a in range(A):
+        T_anchor_inv = linalg.inv_transform(T_CW[frames[a, 0]])
+        for v in range(1, V):
+            T = T_CW[frames[a, v]] @ T_anchor_inv
+            R, t = T[:3, :3], T[:3, 3]
+            motion[a, v - 1, 0, :9], motion[a, v - 1, 0, 9:] = R.reshape(9), t
+            motion[a, v - 1, 1, :9] = R.T.reshape(9)
+            motion[a, v - 1, 1, 9:] = [-(R[0, r] * t[0] + R[1, r] * t[1] + R[2, r] * t[2]) for r in range(3)]
+    return motion
+
+
+SEQUENCE_ASSOCIATIONS = ('epipolar', 'depth')
+# DESIGN.md section 3 (sequence objects): the worst true-pair depth cost of this sequence's pairs at a +-10 % depth error
+DEFAULT_SEQUENCE_MAX_DEPTH_PX = 16.0
+
+
+def anchor_objects(result, a):
+    """One anchor's objects from the host copy (``SequenceObjectTables.numpy()``) of SequenceTriangulator.objects, in the
+    structure tables_to_objects gives a frame: a list (one entry per anchor object) of dicts with 'keypoints' (per map, the
+    anchor's distorted pixels [k, 2], an empty array where the object has none) and 'p_W' (per map, the world points
+    [k, 3], NaN where a track had fewer than two valid views; None where the object has no keypoint of that map)."""
+    observed = result['observed'][a, ..., 0].astype(bool)                  # [O, C, S]: the anchor's own keypoints
+    objects = []
+    for o in range(observed.shape[0]):
+        if not observed[o, 0, 0]:
+            continue
+        keypoints, points = [], []
+        for c in range(observed.shape[1]):
+            k = int(observed[o, c].sum())
+            keypoints.append(result['observations'][a, o, c, :k, 0].copy() if k else np.array([]))
+            points.append(result['point'][a, o, c, :k].copy() if k else None)
+        objects.append({'keypoints': keypoints, 'p_W': points})
+    return objects
+
+
 class SequenceTriangulator:
     """decode tables of a sequence + its camera poses -> one 3D point per anchor peak (world frame)."""
 
@@ -118,13 +165,17 @@ class SequenceTriangulator:
         self._lib = _lib.lib()
 
     def prepare(self, T_CW):
-        """Host-side, once per sequence: the view schedule, the poses of every track group and the pair geometry."""
+        """Host-side, once per sequence: the view schedule, the poses of every track group and the pair geometry
+        (F for both calls; for ``objects`` also the schedule as int32, the pairs' rigid motions and the frame count)."""
         T_CW = np.asarray(T_CW, dtype=np.float64)
         frames = view_schedule(T_CW.shape[0], self.views)
         F = pair_fundamentals(self.camera, T_CW, frames)
         return {'frames': torch.from_numpy(frames).to(self.device),
                 'poses': torch.from_numpy(np.ascontiguousarray(T_CW[frames])).to(self.device),           # [A, V, 4, 4]
-                'F': torch.from_numpy(F).to(self.device)}
+                'F': torch.from_numpy(F).to(self.device),
+                'frames_i32': torch.from_numpy(frames.astype(np.int32)).to(self.device),
+                'motion': torch.from_numpy(pair_motions(T_CW, frames)).to(self.device),                   # [A, V-1, 2, 12]
+                'n_frames': int(T_CW.shape[0])}
 
     def __call__(self, tables, prepared, stream=None):
         """tables: DecodeTables (or a dict of CUDA tensors) of the N frames. -> dict of CUDA tensors:
@@ -176,3 +227,41 @@ class SequenceTriangulator:
         _lib.check(rc, 'okp_triangulate_tracks_f64')
         return {'points': points, 'valid': valid, 'error': error, 'dropped': dropped, 'observed': observed, 'match': match,
                 'observations': obs}
+
+    def objects(self, tables, prepared, association='epipolar', max_depth_px=DEFAULT_SEQUENCE_MAX_DEPTH_PX, stream=None):
+        """The decoded objects of the sequence, per anchor and slot, triangulated in the world frame
+        (okp_triangulate_sequence_objects_f64). tables: the DecodeTables of the N frames ``prepare`` was given, decoded with
+        this camera. Each anchor frame's objects are matched into its V - 1 view frames by their centres, then each matched
+        object's slots type by type, greedily one to one: association='epipolar' by the epipolar distance under the pair's
+        F while it is <= max_distance_px (triangulate_stereo_objects' rule); association='depth' by where each keypoint's
+        lift (kp_point) lands in the other frame, over the candidates within max_distance_px of the epipolar line and with
+        d <= max_depth_px (the stereo depth rule), which tells apart objects that lie on one epipolar line of a view. The
+        matches of every anchor slot form a track of V views, solved like ``__call__`` solves peak tracks (V-view DLT,
+        reprojection filter with max_error_px, re-solve). ValueError for an unknown mode, tables of another frame count
+        than the prepared poses, and association='depth' on tables decoded with compat_clip_bug when the camera's image is
+        not square (such lifts read the depth of a clipped column). Returns SequenceObjectTables on the tables' device;
+        asynchronous: nothing synchronises. anchor_objects(result.numpy(), a) gives anchor a's objects as dicts."""
+        if association not in SEQUENCE_ASSOCIATIONS:
+            raise ValueError(f"association must be one of {SEQUENCE_ASSOCIATIONS}, got {association!r}")
+        if tables.N != prepared['n_frames']:
+            raise ValueError(f"the tables hold {tables.N} frames, the prepared poses {prepared['n_frames']}")
+        if association == 'depth':
+            size = np.asarray(self.camera.image_size).reshape(-1)[:2]
+            if tables.params.compat_clip_bug and size[0] != size[1]:
+                raise ValueError("association='depth' reads kp_point, and with compat_clip_bug a non-square image is lifted "
+                                 "with the depth of a clipped column: decode with compat_clip_bug=False")
+        frames = prepared['frames_i32']
+        A, V = (int(v) for v in frames.shape)
+        O, C, S = (int(v) for v in tables['kp_xy'].shape[1:4])
+        device = tables.flat.device
+        out = SequenceObjectTables(A, V, O, C, S, device)
+        cfg = (ctypes.c_int32 * max(len(tables.keypoint_config), 1))(*tables.keypoint_config)
+        with torch.cuda.device(device):
+            rc = self._lib.okp_triangulate_sequence_objects_f64(
+                ctypes.byref(tables.struct), tables.N, C, cfg, ctypes.byref(tables.params), frames.data_ptr(), A, V,
+                prepared['F'].data_ptr(), prepared['motion'].data_ptr(), prepared['poses'].data_ptr(), ctypes.byref(self._cam),
+                SEQUENCE_ASSOCIATIONS.index(association), self.max_distance_px, float(max_depth_px), self.max_error_px,
+                self.max_rounds, ctypes.byref(out.struct), _stream_handle(stream))
+        _lib.check(rc, 'okp_triangulate_sequence_objects_f64')
+        out.prepared = prepared                              # the launch reads its arrays: kept alive with the result
+        return out
