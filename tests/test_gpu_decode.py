@@ -230,6 +230,16 @@ def test_component_level_api():
     assert np.abs(got - want).max() <= TOL_METRES_REL * np.abs(want).max()
 
 
+def assert_peaks_match_oracle(got, want):
+    """Peak tables of extract_peaks against the oracle's decode of the same maps: counts and pixels identical, float32
+    columns bitwise, and no assignment (extract_peaks groups nothing)."""
+    np.testing.assert_array_equal(got['peak_count'], want['peak_count'])
+    np.testing.assert_array_equal(got['peak_yx'], want['peak_yx'])
+    for key in ['peak_score', 'peak_xy', 'peak_conf']:
+        np.testing.assert_array_equal(got[key].view(np.uint32), want[key].view(np.uint32), err_msg=key)
+    assert (got['peak_object'] == -1).all()
+
+
 @pytest.mark.parametrize('H,W,N,C,K', [
     (64, 64, 37, 3, 32),       # maps not a multiple of the maps-per-CTA group
     (3, 4, 5, 2, 8),           # tiny map: every window is clipped
@@ -256,11 +266,7 @@ def test_peak_extraction_shapes_noise_and_overflow(H, W, N, C, K):
     got = decoder.extract_peaks(heat).numpy()
     want = c_oracle.decode(heat, np.zeros_like(heat), np.zeros((N, C - 1, 2, H, W), np.float32), cfg, None,
                            max_peaks=K, max_objects=16)
-    np.testing.assert_array_equal(got['peak_count'], want['peak_count'])
-    np.testing.assert_array_equal(got['peak_yx'], want['peak_yx'])
-    for key in ['peak_score', 'peak_xy', 'peak_conf']:
-        np.testing.assert_array_equal(got[key].view(np.uint32), want[key].view(np.uint32), err_msg=key)
-    assert (got['peak_object'] == -1).all()
+    assert_peaks_match_oracle(got, want)
     if (H, W) == (33, 320):                                       # both the overflow path and the fast path
         assert (want['peak_count'] > K).any() and (want['peak_count'] <= K).any()
 
