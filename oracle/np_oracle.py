@@ -493,7 +493,9 @@ def associate(F, left, right, max_distance_px=2.5):
     match_cost = np.zeros(nl)
     free = np.ones((nl, nr), bool)
     for _ in range(min(nl, nr)):
-        masked = np.where(free, cost, np.inf)
+        # a NaN cost (a left point at the epipole: l = F x = 0) is never admissible, like any cost above the gate; the
+        # step goes on with the other candidates (np.argmin would return the first NaN and end the matching)
+        masked = np.where(free & ~np.isnan(cost), cost, np.inf)
         e = int(np.argmin(masked))                 # first minimum in (left, right) raster order
         i, j = divmod(e, nr)
         if not (masked[i, j] <= max_distance_px):

@@ -22,7 +22,7 @@ def _greedy(cost, max_cost):
     match_cost = np.zeros(nl)
     free = np.ones((nl, nr), bool)
     for _ in range(min(nl, nr)):
-        masked = np.where(free, cost, np.inf)
+        masked = np.where(free & ~np.isnan(cost), cost, np.inf)        # NaN: not admissible, as in associate
         e = int(np.argmin(masked))                 # first minimum in (left, right) raster order
         i, j = divmod(e, nr)
         if not (masked[i, j] <= max_cost):
